@@ -269,6 +269,31 @@ def actor_flops(N, P=1, H=200):
     return 2 * (gemm + adj)
 
 
+DUMP_LIMIT_BYTES = 64 * 10 ** 6
+
+
+def last_step_outputs(env, actions):
+    """what a caller of the timed path holds after its last step: the actor's actions (when the actor drives the step;
+    the env-step clips them in place) and every output of the env-step, as float32 / float64 numpy arrays.  A batch whose
+    arrays exceed DUMP_LIMIT_BYTES is cut to a fixed sample of environments (seed 0, sorted), the same for every run with
+    the same --batch."""
+    import torch
+    names = ("x_n", "A_s", "A_n_ts", "A_n_cs", "nN_x_n", "nN_x_e", "move_range", "point", "status") + \
+        (("y", "y_weak") + env.FP64_FIELDS if env.fp64_outputs else ())
+    tensors = dict(zip(("a_geo", "a_topo"), actions or ()))
+    tensors.update((k, getattr(env, k)) for k in names)
+    per_env = sum(t[0].numel() * (8 if t.dtype == torch.float64 else 4) for t in tensors.values())
+    keep = min(env.B, (DUMP_LIMIT_BYTES - 4096 * len(tensors)) // per_env)
+    rows = None
+    if keep < env.B:
+        rows = torch.from_numpy(np.sort(np.random.RandomState(0).choice(env.B, keep, replace=False))).to(env.device)
+    out = {}
+    for k, t in tensors.items():
+        t = t if rows is None else t.index_select(0, rows)
+        out[k] = t.to(torch.float64 if t.dtype == torch.float64 else torch.float32).cpu().numpy()
+    return out
+
+
 def _max_over_ranks(ms, dev, world):
     if world > 1:
         import torch
@@ -511,7 +536,14 @@ def main():
     ap.add_argument("--train", action="store_true", help="only the training loop of BASELINE config 5 (large roof, MADDPG update with gradient all-reduce)")
     ap.add_argument("--train-steps", type=int, default=0, help="timed steps of the training leg (default: 10, or --steps with --train)")
     ap.add_argument("--train-eager", action="store_true", help="training leg: run the learner update eagerly instead of as a captured CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned (actions, state tensors, point, status, "
+                         "float64 FEM fields) as DIR/<name>.npy, float32 or float64, at most 64 MB in all (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.train or args.impl != "b200"):
+        ap.error("--dump-outputs writes the outputs of the B200 env-step path; it does not apply to --train or --impl reference")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -610,6 +642,10 @@ def main():
         one_step(i, timed=True)
         ends[i].record()
     torch.cuda.synchronize()
+    if args.dump_outputs and rank == 0:                 # before the e2e legs below step `env` again
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in last_step_outputs(env, (a_geo_buf, a_topo_buf) if use_actor else None).items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     launches = env.launch_count() + (pol.launch_count() if use_actor else 0) - launches0
     step_ms = [s.elapsed_time(e) for s, e in zip(starts, ends)]
     total_ms = float(sum(step_ms))

@@ -78,6 +78,70 @@ def test_training_leg_line():
     assert set(d["stages_ms"]) >= {"rollout_3x_act_3x_env_step", "replay_push", "learner_train_update"}
 
 
+@pytest.mark.gpu
+def test_dump_outputs_repeat(tmp_path):
+    """--dump-outputs: the last timed step's outputs as float32 / float64 .npy files, identical for identical arguments;
+    one more timed step (--steps 5) is the oracle's env-step of the --steps 4 state under the dumped actions"""
+    import numpy as np
+    from oracle.truss_oracle import TrussOracle
+    args = ("--warmup", "3", "--cpu-seconds", "0.2", "--batch", "300", "--no-extras")
+    dumps = []
+    for k, steps in enumerate(("4", "4", "5")):
+        run_bench("--steps", steps, *args, "--dump-outputs", str(tmp_path / str(k)))
+        dumps.append({f[:-4]: np.load(tmp_path / str(k) / f) for f in sorted(os.listdir(tmp_path / str(k)))})
+    a, b, c = dumps
+    assert {"a_geo", "a_topo", "x_n", "nN_x_e", "point", "status", "d"} <= set(a) and set(a) == set(b) == set(c)
+    for name in a:
+        assert a[name].dtype in (np.float32, np.float64) and a[name].shape[0] == 300, name
+        assert np.array_equal(a[name], b[name]), name
+    assert (a["status"] == 0).all() and (c["status"] == 0).all() and np.isfinite(a["d"]).all()
+    assert not np.array_equal(a["nN_x_n"], c["nN_x_n"])
+    o = TrussOracle("small_bridge")
+    for i in range(0, 300, 37):
+        # the coin of a step is not dumped: one of the two must give the dumped state
+        outs = [o.step(a["nN_x_n"][i], a["nN_x_e"][i], a["move_range"][i, :, 0], a["move_range"][i, :, 1],
+                       c["a_geo"][i].copy(), c["a_topo"][i].copy(), coin) for coin in (False, True)]
+        assert any(np.array_equal(out["y"].astype(np.float32), c["nN_x_n"][i, :, 1]) and
+                   np.array_equal(out["section"], c["nN_x_e"][i, :, 0].astype(np.int32)) and
+                   np.array_equal(out["max_up"], c["move_range"][i, :, 0]) and
+                   np.array_equal(out["max_down"], c["move_range"][i, :, 1]) for out in outs), i
+
+
+def test_dump_outputs_sample():
+    """a batch larger than the dump budget is cut to the same sorted sample of environments for every output"""
+    import numpy as np
+    import torch
+    import bench
+
+    class Env:
+        FP64_FIELDS = ("d",)
+        fp64_outputs, device = True, torch.device("cpu")
+
+        def __init__(self, B):
+            self.B = B
+            rows = torch.arange(B)
+            for k, shape in (("x_n", (13,)), ("A_s", (3, 3)), ("A_n_ts", (3, 3)), ("A_n_cs", (3, 3)), ("nN_x_n", (12,)),
+                             ("nN_x_e", (5, 21)), ("move_range", (3, 2)), ("point", (4,)), ("y", (3,))):
+                setattr(self, k, rows.reshape(B, *[1] * len(shape)).expand(B, *shape).to(torch.float32).contiguous())
+            self.d = rows.to(torch.float64)[:, None].repeat(1, 6)
+            self.status = torch.zeros(B, dtype=torch.int32)
+            self.y_weak = torch.ones(B, 3, dtype=torch.uint8)
+
+    small = bench.last_step_outputs(Env(50), (torch.rand(50, 3, 2), torch.rand(50, 3, 3)))
+    assert all(a.shape[0] == 50 for a in small.values()) and small["d"].dtype == np.float64
+    assert small["status"].dtype == np.float32 and small["y_weak"].dtype == np.float32
+    B = 200000
+    out = bench.last_step_outputs(Env(B), None)
+    assert "a_geo" not in out
+    rows = out["x_n"][:, 0].astype(np.int64)
+    assert 0 < len(rows) < B and (np.diff(rows) > 0).all()
+    for name, a in out.items():
+        if name not in ("status", "y_weak"):                  # every other fake output carries its row index
+            assert np.array_equal(a.reshape(len(rows), -1)[:, 0], rows), name
+    assert sum(a.nbytes for a in out.values()) <= bench.DUMP_LIMIT_BYTES
+    assert np.array_equal(bench.last_step_outputs(Env(B), None)["d"], out["d"])
+
+
 def test_e2e_piece_schedule_argument():
     """--e2e-pieces: 'auto' (HostRollout decides), a count of equal pieces, explicit sizes, or fractions of the batch"""
     import bench
