@@ -9,8 +9,9 @@
  *     error (text via tfem_last_error()); per-environment numerical trouble is reported in status[].
  *   - all buffers are caller-owned, contiguous, 16-byte aligned; "device" pointers are CUDA device
  *     pointers valid on the handle's device, "host" pointers are (preferably pinned) host memory.
- *   - one handle per (GPU, geometry family); re-entrant per handle; the only hidden state is the
- *     family's constant tables.  stream is a cudaStream_t passed as void*.
+ *   - one handle per (GPU, geometry family), or per (GPU, set of families of one topology) for the mixed
+ *     entry points; re-entrant per handle; the only hidden state is the families' constant tables.
+ *     stream is a cudaStream_t passed as void*.
  *   - B = number of independent environments in the call.  N = 2*num_x nodes, E = 5*num_x-4 elements,
  *     ndof = free DOFs in the reference numbering (FEM_2Dtruss.py:227-261).
  */
@@ -26,6 +27,7 @@ extern "C" {
 
 #define TFEM_MAX_NX 16
 #define TFEM_NSEC 5
+#define TFEM_MAX_FAMILIES 16
 
 enum { TFEM_BRIDGE = 0, TFEM_ROOF = 1 };
 /* symmetry convention of truss2D_ENV.py: none = train/code, small = test/00,01 (:460-553),
@@ -33,7 +35,7 @@ enum { TFEM_BRIDGE = 0, TFEM_ROOF = 1 };
 enum { TFEM_SYM_NONE = 0, TFEM_SYM_SMALL = 1, TFEM_SYM_LARGE = 2 };
 
 /* status[] bits */
-enum { TFEM_STATUS_OK = 0, TFEM_STATUS_NOT_SPD = 1, TFEM_STATUS_NONFINITE = 2 };
+enum { TFEM_STATUS_OK = 0, TFEM_STATUS_NOT_SPD = 1, TFEM_STATUS_NONFINITE = 2, TFEM_STATUS_BAD_FAMILY = 4 };
 
 /* error codes */
 enum {
@@ -196,6 +198,30 @@ int tfem_read_genes(tfem_handle_t h, int B, const double* genes, double max_heig
  * and synchronises the stream before returning.  Scratch device memory is owned by the handle. */
 int tfem_step_host(tfem_handle_t h, int B, const tfem_step_in* in_host, const tfem_step_out* out_host,
                    void* stream);
+
+/* Mixed-family batches: the reference's training driver draws one of the five 6 x 2 shapes and a truss type for
+ * every episode (train/code/master_DDPG_truss2D_MO.py:787-815), so B episodes run in parallel form a batch of mixed
+ * families.  tfem_create_mixed builds one handle from n_families (1..TFEM_MAX_FAMILIES) descriptions that share the
+ * topology: num_x (mesh, element order, output maps) and the DOF map that support_case fixes (TNSC, RES tables).  A
+ * mismatch returns TFEM_ERR_UNSUPPORTED with the name of the differing table.  Everything else (spans, span_y, tar_y,
+ * d_min, load_y, truss type, symmetry convention, sections, young, allow_stress) may differ.  The large meshes fit
+ * fewer families per launch than the small ones: a count that would lower the kernel's CTAs per SM is refused with
+ * TFEM_ERR_UNSUPPORTED and the limit in the error text.  device < 0 gives a tables-only handle, as for tfem_create.
+ *
+ * family [B] (device, uint8) holds one index into descs per environment; it is an input of every call and is not
+ * kept by the handle.  Environment b is tfem_reset / tfem_step of family family[b]: the same outputs, the same
+ * point normalisation by that family's int_obj, the same status bits.  An index >= n_families sets
+ * status[b] = TFEM_STATUS_BAD_FAMILY and writes nothing else for that environment.
+ *
+ * With n_families == 1 the handle also serves every single-family entry point, exactly like tfem_create.  With more
+ * families those (tfem_reset, tfem_step, tfem_solve_only, tfem_read_genes, tfem_step_host, tfem_solve_dense_dmma)
+ * return TFEM_ERR_ARG, and tfem_get_table serves only the topology tables (CONN, TNSC, RES, TOP, PAIR, A_N, MASK,
+ * NC_E); a tables-only handle of one family serves the others. */
+int tfem_create_mixed(const tfem_family_desc* descs, int n_families, int device, tfem_handle_t* out);
+int tfem_reset_mixed(tfem_handle_t h, int B, const uint8_t* family, float* move_range_out, const tfem_step_out* out,
+                     void* stream);
+int tfem_step_mixed(tfem_handle_t h, int B, const uint8_t* family, const tfem_step_in* in, const tfem_step_out* out,
+                    void* stream);
 
 /* number of kernels this library launched on behalf of the handle since creation; tfem_book_launches adds kernel
  * launches that were replayed from a CUDA graph captured around tfem_step (trollout_step_host) */

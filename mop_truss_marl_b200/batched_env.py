@@ -40,7 +40,7 @@ class BatchedTrussEnv:
             raise capi.TfemError("CUDA is not available: libtfem has no CPU path")
         index = self.device.index if self.device.index is not None else torch.cuda.current_device()
         self.device = torch.device("cuda", index)
-        self.handle = capi.Handle(family_desc(self.spec), index)
+        self.handle = self._open_handle(index)
         d = self.handle.dims
         self.B, self.N, self.E, self.ndof, self.nres = int(batch), d.N, d.E, d.ndof, d.nres
         self.fp64_outputs = fp64_outputs
@@ -48,9 +48,15 @@ class BatchedTrussEnv:
         self.A_n = torch.from_numpy(self.handle.table("A_n")).to(self.device)
         self.mask = torch.from_numpy(self.handle.table("mask")).to(self.device)
         self.nC_e = torch.from_numpy(self.handle.table("nC_e")).to(self.device)
-        self.int_obj = self.handle.table("int_obj")
+        self.int_obj = self._int_obj()
         self.game_step = 1                     # Game_research04.game_step (:242)
         self._alloc(self.B)
+
+    def _open_handle(self, index):
+        return capi.Handle(family_desc(self.spec), index)
+
+    def _int_obj(self):
+        return self.handle.table("int_obj")
 
     # ------------------------------------------------------------------------------------------------
     def _alloc(self, B):
@@ -120,9 +126,7 @@ class BatchedTrussEnv:
                 raise ValueError("coin must be a contiguous uint8 [B] tensor on the env device")
         src = self
         if parent is not None:
-            if parent.B != self.B or parent.N != self.N or parent.E != self.E or parent.device != self.device:
-                raise ValueError("parent must be a batch of the same family, size and device")
-            self.move_range[lo:hi].copy_(parent.move_range[lo:hi])
+            self._inherit(parent, lo, hi)
             src = parent
         sin = capi.StepIn()
         sin.set_node = _ptr(src.nN_x_n[lo:hi])
@@ -132,10 +136,19 @@ class BatchedTrussEnv:
         sin.coin = _ptr(coin)
         sin.move_range = _ptr(self.move_range[lo:hi])
         out = self._out if rows is None else self._make_out(lo, hi)
-        capi.check(capi.lib.tfem_step(self.handle.ptr, nb, C.byref(sin), C.byref(out), self._stream()))
+        self._launch_step(lo, hi, sin, out)
         if rows is None or hi == self.B:
             self.game_step += 1
         return self.point if rows is None else self.point[lo:hi]
+
+    def _inherit(self, parent, lo, hi):
+        """the per-environment state a child batch takes from its parent besides the raw tables"""
+        if parent.B != self.B or parent.N != self.N or parent.E != self.E or parent.device != self.device:
+            raise ValueError("parent must be a batch of the same family, size and device")
+        self.move_range[lo:hi].copy_(parent.move_range[lo:hi])
+
+    def _launch_step(self, lo, hi, sin, out):
+        capi.check(capi.lib.tfem_step(self.handle.ptr, hi - lo, C.byref(sin), C.byref(out), self._stream()))
 
     def _check(self, t, shape):
         if not (isinstance(t, torch.Tensor) and t.dtype == torch.float32 and tuple(t.shape) == shape
@@ -181,6 +194,52 @@ class BatchedTrussEnv:
 
     def launch_count(self) -> int:
         return self.handle.launch_count()
+
+
+class MixedTrussEnv(BatchedTrussEnv):
+    """``batch`` environments on ``device``, each of its own family among ``families`` (names or FamilySpecs that share
+    num_x and support_case, at most ``capi.MAX_FAMILIES``; the large meshes fit fewer, see ``tfem_create_mixed``).  This is
+    the reference's training batch: ``train/code/master_DDPG_truss2D_MO.py:787-815`` draws a shape and a truss type for
+    every episode (``families.TRAIN_FAMILIES``).  One ``tfem_step_mixed`` launch steps the whole batch; environment b is
+    bit for bit what a ``BatchedTrussEnv`` of family ``families[family_ids[b]]`` computes from the same inputs.
+
+    ``reset(family_ids)`` takes a uint8 CUDA tensor [B] of indices into ``families`` and keeps a copy as
+    ``self.family_ids``; ``step`` has the signature of ``BatchedTrussEnv.step`` (``parent=`` children copy the parent's
+    family ids).  ``int_obj`` is [F, 2].  The single-family calls (``solve_only``, ``solve_dense_dmma``) and
+    ``host_pipeline.HostRollout`` refuse a batch of more than one family."""
+
+    def __init__(self, families, batch: int, device="cuda:0", fp64_outputs: bool = True):
+        self.specs = tuple(FAMILIES[f] if isinstance(f, str) else f for f in families)
+        if not self.specs:
+            raise ValueError("at least one family is needed")
+        super().__init__(self.specs[0], batch, device, fp64_outputs)
+        self.family_ids = torch.full((self.B,), 255, dtype=torch.uint8, device=self.device)   # no family until reset
+
+    def _open_handle(self, index):
+        return capi.MixedHandle([family_desc(s) for s in self.specs], index)
+
+    def _int_obj(self):
+        return np.stack([capi.Handle(family_desc(s), -1).table("int_obj") for s in self.specs])
+
+    def reset(self, family_ids: torch.Tensor):
+        if not (isinstance(family_ids, torch.Tensor) and family_ids.dtype == torch.uint8 and tuple(family_ids.shape) == (self.B,)
+                and family_ids.device == self.device and family_ids.is_contiguous()):
+            raise ValueError("family_ids must be a contiguous uint8 [B] tensor on the env device")
+        self.family_ids.copy_(family_ids)
+        capi.check(capi.lib.tfem_reset_mixed(self.handle.ptr, self.B, _ptr(self.family_ids), _ptr(self.move_range),
+                                             C.byref(self._out), self._stream()))
+        self.game_step = 1
+        return self.state()
+
+    def _inherit(self, parent, lo, hi):
+        if not isinstance(parent, MixedTrussEnv) or parent.specs != self.specs:
+            raise ValueError("parent must be a mixed batch over the same families")
+        super()._inherit(parent, lo, hi)
+        self.family_ids[lo:hi].copy_(parent.family_ids[lo:hi])
+
+    def _launch_step(self, lo, hi, sin, out):
+        capi.check(capi.lib.tfem_step_mixed(self.handle.ptr, hi - lo, _ptr(self.family_ids[lo:hi]), C.byref(sin),
+                                            C.byref(out), self._stream()))
 
 
 def step_host(handle: capi.Handle, set_node, set_element, move_range, a_geo, a_topo, coin=None,

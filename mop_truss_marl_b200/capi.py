@@ -15,8 +15,9 @@ LIB_PATH = os.environ.get("TFEM_LIB", os.path.join(_HERE, "lib", "libtfem.so"))
 
 MAX_NX = 16
 NSEC = 5
+MAX_FAMILIES = 16
 
-STATUS_OK, STATUS_NOT_SPD, STATUS_NONFINITE = 0, 1, 2
+STATUS_OK, STATUS_NOT_SPD, STATUS_NONFINITE, STATUS_BAD_FAMILY = 0, 1, 2, 4
 
 
 class FamilyDesc(C.Structure):
@@ -72,7 +73,8 @@ class GenesOut(C.Structure):
 
 
 EXPORTS = ("tfem_version", "tfem_last_error", "tfem_create", "tfem_destroy", "tfem_get_dims", "tfem_get_table",
-           "tfem_reset", "tfem_step", "tfem_solve_only", "tfem_read_genes", "tfem_solve_dense_dmma", "tfem_step_host", "tfem_launch_count", "tfem_book_launches")
+           "tfem_reset", "tfem_step", "tfem_solve_only", "tfem_read_genes", "tfem_solve_dense_dmma", "tfem_step_host", "tfem_launch_count", "tfem_book_launches",
+           "tfem_create_mixed", "tfem_reset_mixed", "tfem_step_mixed")
 
 
 class TfemError(RuntimeError):
@@ -98,6 +100,9 @@ def _load():
                                     C.POINTER(GenesOut), C.c_void_p]
     lib.tfem_solve_dense_dmma.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 5
     lib.tfem_step_host.argtypes = [C.c_void_p, C.c_int, C.POINTER(StepIn), C.POINTER(StepOut), C.c_void_p]
+    lib.tfem_create_mixed.argtypes = [C.POINTER(FamilyDesc), C.c_int, C.c_int, C.POINTER(C.c_void_p)]
+    lib.tfem_reset_mixed.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.POINTER(StepOut), C.c_void_p]
+    lib.tfem_step_mixed.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.POINTER(StepIn), C.POINTER(StepOut), C.c_void_p]
     lib.tfem_launch_count.argtypes = [C.c_void_p]
     lib.tfem_launch_count.restype = C.c_int64
     for name in EXPORTS:
@@ -146,3 +151,17 @@ class Handle:
 
     def launch_count(self) -> int:
         return int(lib.tfem_launch_count(self._h))
+
+
+class MixedHandle(Handle):
+    """One handle over several families of one topology: ``tfem_create_mixed``.  With more than one family only the
+    topology tables can be read (``table``)."""
+
+    def __init__(self, descs, device: int = 0):
+        self._h = C.c_void_p()
+        arr = (FamilyDesc * len(descs))(*descs)
+        check(lib.tfem_create_mixed(arr, len(descs), int(device), C.byref(self._h)))
+        self.n_families = len(descs)
+        self.device = int(device)
+        self.dims = Dims()
+        check(lib.tfem_get_dims(self._h, C.byref(self.dims)))

@@ -19,7 +19,8 @@ bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) ==
 }  // namespace
 
 struct tfem_handle_s {
-  tfem::Family fam;
+  tfem::Family fam;                  // the only family, or the first of a mixed handle
+  int n_families = 1;                // tfem_create_mixed: tables of all families follow each other in d_tables
   int device = 0;
   tfem::FamilyTables* d_tables = nullptr;
   uint16_t* d_maps = nullptr;
@@ -41,6 +42,37 @@ struct DeviceGuard {
   }
   ~DeviceGuard() { if (prev >= 0) cudaSetDevice(prev); }
 };
+
+// entry points that serve one family refuse a handle of several
+int single_family(tfem_handle_t h, const char* call, const char* instead) {
+  if (h->n_families == 1) return 0;
+  return fail(TFEM_ERR_ARG, std::string(call) + ": the handle holds " + std::to_string(h->n_families) +
+                                " families; use " + instead + " (or a handle of one family)");
+}
+
+// the mixed entry points need the mixed kernel configured (tfem_create_mixed); a tables-only handle fails at launch
+int mixed_family(tfem_handle_t h, const char* call) {
+  if (h->device < 0 || h->launch.smem_mixed > 0) return 0;
+  return fail(TFEM_ERR_ARG, std::string(call) + ": the handle was made by tfem_create; use tfem_create_mixed");
+}
+
+// first topology table in which family b differs from family a, or nullptr.  These are what the kernel reads once per
+// launch (or once before its environment loop) and what the output maps are built from.
+const char* topology_mismatch(const tfem::Family& a, const tfem::Family& b) {
+  const tfem::FamilyTables &s = a.t, &t = b.t;
+  if (s.nx != t.nx) return "num_x";
+  if (memcmp(s.conn, t.conn, sizeof(s.conn))) return "CONN";
+  if (memcmp(s.top, t.top, sizeof(s.top))) return "TOP";
+  if (memcmp(s.pair, t.pair, sizeof(s.pair))) return "PAIR";
+  if (memcmp(s.adj, t.adj, sizeof(s.adj))) return "adjacency";
+  if (a.maps != b.maps || s.map_xn != t.map_xn || s.map_as != t.map_as || s.map_ts != t.map_ts || s.map_cs != t.map_cs ||
+      s.map_rawn != t.map_rawn || s.map_rawe != t.map_rawe || s.map_total != t.map_total)
+    return "output maps";
+  if (memcmp(s.res, t.res, sizeof(s.res))) return "RES";
+  if (memcmp(s.dof, t.dof, sizeof(s.dof)) || s.ndof != t.ndof || s.nres != t.nres) return "TNSC";
+  if (memcmp(s.react_slot, t.react_slot, sizeof(s.react_slot))) return "reaction slots";
+  return nullptr;
+}
 
 int check_out_alignment(const tfem_step_out* o) {
   const void* ps[] = {o->x_n, o->A_s, o->A_n_ts, o->A_n_cs, o->nN_x_n, o->nN_x_e, o->point, o->point64,
@@ -93,6 +125,57 @@ int tfem_create(const tfem_family_desc* desc, int device, tfem_handle_t* out) {
   return TFEM_OK;
 }
 
+int tfem_create_mixed(const tfem_family_desc* descs, int n_families, int device, tfem_handle_t* out) {
+  if (!descs || !out) return fail(TFEM_ERR_ARG, "null argument");
+  *out = nullptr;
+  if (n_families < 1 || n_families > TFEM_MAX_FAMILIES)
+    return fail(TFEM_ERR_ARG, "n_families must be 1.." + std::to_string(TFEM_MAX_FAMILIES) + ", got " + std::to_string(n_families));
+  std::vector<tfem::Family> fams(n_families);
+  for (int i = 0; i < n_families; ++i) {
+    if (!tfem::build_family(descs[i], fams[i])) return fail(TFEM_ERR_UNSUPPORTED, "family " + std::to_string(i) + ": " + fams[i].error);
+    if (i == 0) continue;
+    if (const char* tab = topology_mismatch(fams[0], fams[i]))
+      return fail(TFEM_ERR_UNSUPPORTED, "family " + std::to_string(i) + " differs from family 0 in the " + tab +
+                                            " table: the families of one handle must share num_x and support_case");
+  }
+  tfem_handle_s* h = new (std::nothrow) tfem_handle_s();
+  if (!h) return fail(TFEM_ERR_ARG, "out of host memory");
+  h->fam = fams[0];
+  h->n_families = n_families;
+  if (device < 0) {
+    h->device = -1;
+    *out = h;
+    return TFEM_OK;
+  }
+  int ndev = 0;
+  cudaError_t e = cudaGetDeviceCount(&ndev);
+  if (e != cudaSuccess || ndev == 0) { delete h; return fail(TFEM_ERR_CUDA, "no CUDA device: libtfem has no CPU path"); }
+  if (device >= ndev) { delete h; return fail(TFEM_ERR_ARG, "bad device index"); }
+  h->device = device;
+  DeviceGuard guard(device);
+  if (!guard.ok) { delete h; return fail(TFEM_ERR_CUDA, "cudaSetDevice failed"); }
+  const size_t tab_bytes = sizeof(tfem::FamilyTables);
+  e = cudaMalloc(&h->d_tables, n_families * tab_bytes);
+  if (e == cudaSuccess) e = cudaMalloc(&h->d_maps, h->fam.maps.size() * sizeof(uint16_t));
+  for (int i = 0; i < n_families && e == cudaSuccess; ++i)
+    e = cudaMemcpy(h->d_tables + i, &fams[i].t, tab_bytes, cudaMemcpyHostToDevice);
+  if (e == cudaSuccess) e = cudaMemcpy(h->d_maps, h->fam.maps.data(), h->fam.maps.size() * sizeof(uint16_t), cudaMemcpyHostToDevice);
+  if (e != cudaSuccess) { tfem_destroy(h); return cuda_fail(e, "table upload"); }
+  int rc = tfem::step_kernel_configure(h->fam.t.nx, device, h->fam.t.map_total, &h->launch);
+  int max_families = 0;
+  if (rc == 0) rc = tfem::step_kernel_configure_mixed(h->fam.t.nx, (int)h->fam.maps.size(), n_families, &h->launch, &max_families);
+  if (rc != 0) { tfem_destroy(h); return cuda_fail((cudaError_t)rc, "kernel configure"); }
+  if (n_families > max_families) {
+    const int nx = h->fam.t.nx, ctas = h->launch.ctas_per_sm;
+    tfem_destroy(h);
+    return fail(TFEM_ERR_UNSUPPORTED, "num_x = " + std::to_string(nx) + ": at most " + std::to_string(max_families) +
+                                          " families fit the shared memory of one CTA at the env-step kernel's " +
+                                          std::to_string(ctas) + " CTAs per SM; got " + std::to_string(n_families));
+  }
+  *out = h;
+  return TFEM_OK;
+}
+
 int tfem_destroy(tfem_handle_t h) {
   if (!h) return TFEM_OK;
   if (h->device < 0) { delete h; return TFEM_OK; }
@@ -117,6 +200,16 @@ int tfem_get_table(tfem_handle_t h, int which, void* dst, size_t bytes) {
   const tfem::Family& f = h->fam;
   const void* src = nullptr;
   size_t n = 0;
+  if (h->n_families > 1) {
+    switch (which) {
+      case TFEM_TAB_CONN: case TFEM_TAB_TNSC: case TFEM_TAB_RES: case TFEM_TAB_TOP: case TFEM_TAB_PAIR:
+      case TFEM_TAB_A_N: case TFEM_TAB_MASK: case TFEM_TAB_NC_E: break;
+      default:
+        if (which < TFEM_TAB_CONN || which > TFEM_TAB_SCALARS) return fail(TFEM_ERR_ARG, "unknown table id");
+        return fail(TFEM_ERR_ARG, "table " + std::to_string(which) + " differs between the " + std::to_string(h->n_families) +
+                                      " families of this handle: read it from a tables-only handle of one family");
+    }
+  }
   float int_obj[2] = {f.t.int_obj1, f.t.int_obj2};
   double scal[8] = {f.t.y_max, f.t.y_min, f.t.d_min, f.t.max_def, f.t.young, f.t.allow, f.t.load_y, 0.0};
   switch (which) {
@@ -159,6 +252,7 @@ static int launch(tfem_handle_t h, tfem::StepArgs& a, void* stream) {
 
 int tfem_reset(tfem_handle_t h, int B, float* move_range_out, const tfem_step_out* out, void* stream) {
   if (!h || !out) return fail(TFEM_ERR_ARG, "null argument");
+  if (int rc = single_family(h, "tfem_reset", "tfem_reset_mixed")) return rc;
   if (B < 0) return fail(TFEM_ERR_ARG, "negative batch");
   if (int rc = check_out_alignment(out)) return rc;
   if (move_range_out && !aligned16(move_range_out)) return fail(TFEM_ERR_ALIGN, "move_range must be 16-byte aligned");
@@ -167,25 +261,59 @@ int tfem_reset(tfem_handle_t h, int B, float* move_range_out, const tfem_step_ou
   return launch(h, a, stream);
 }
 
-int tfem_step(tfem_handle_t h, int B, const tfem_step_in* in, const tfem_step_out* out, void* stream) {
-  if (!h || !in || !out) return fail(TFEM_ERR_ARG, "null argument");
-  if (B < 0) return fail(TFEM_ERR_ARG, "negative batch");
-  if (B == 0) return TFEM_OK;
+static int check_step_in(const tfem_step_in* in) {
   if ((!in->set_node && !in->set_node_y) || (!in->set_element && !in->set_element_section) || !in->a_geo || !in->a_topo ||
       !in->move_range)
     return fail(TFEM_ERR_ARG, "set_node (or set_node_y), set_element (or set_element_section), a_geo, a_topo and move_range are required");
   if ((in->set_node && !aligned16(in->set_node)) || (in->set_element && !aligned16(in->set_element)) || !aligned16(in->a_geo) ||
       !aligned16(in->a_topo) || !aligned16(in->move_range))
     return fail(TFEM_ERR_ALIGN, "input buffers must be 16-byte aligned");
+  return 0;
+}
+
+int tfem_step(tfem_handle_t h, int B, const tfem_step_in* in, const tfem_step_out* out, void* stream) {
+  if (!h || !in || !out) return fail(TFEM_ERR_ARG, "null argument");
+  if (int rc = single_family(h, "tfem_step", "tfem_step_mixed")) return rc;
+  if (B < 0) return fail(TFEM_ERR_ARG, "negative batch");
+  if (B == 0) return TFEM_OK;
+  if (int rc = check_step_in(in)) return rc;
   if (int rc = check_out_alignment(out)) return rc;
   tfem::StepArgs a{};
   a.B = B; a.mode = tfem::MODE_STEP; a.in = *in; a.out = *out;
   return launch(h, a, stream);
 }
 
+int tfem_reset_mixed(tfem_handle_t h, int B, const uint8_t* family, float* move_range_out, const tfem_step_out* out,
+                     void* stream) {
+  if (!h || !family || !out) return fail(TFEM_ERR_ARG, "null argument");
+  if (int rc = mixed_family(h, "tfem_reset_mixed")) return rc;
+  if (B < 0) return fail(TFEM_ERR_ARG, "negative batch");
+  if (int rc = check_out_alignment(out)) return rc;
+  if (move_range_out && !aligned16(move_range_out)) return fail(TFEM_ERR_ALIGN, "move_range must be 16-byte aligned");
+  tfem::StepArgs a{};
+  a.B = B; a.mode = tfem::MODE_RESET; a.out = *out; a.reset_move_range = move_range_out;
+  a.family = family; a.n_families = h->n_families;
+  return launch(h, a, stream);
+}
+
+int tfem_step_mixed(tfem_handle_t h, int B, const uint8_t* family, const tfem_step_in* in, const tfem_step_out* out,
+                    void* stream) {
+  if (!h || !family || !in || !out) return fail(TFEM_ERR_ARG, "null argument");
+  if (int rc = mixed_family(h, "tfem_step_mixed")) return rc;
+  if (B < 0) return fail(TFEM_ERR_ARG, "negative batch");
+  if (B == 0) return TFEM_OK;
+  if (int rc = check_step_in(in)) return rc;
+  if (int rc = check_out_alignment(out)) return rc;
+  tfem::StepArgs a{};
+  a.B = B; a.mode = tfem::MODE_STEP; a.in = *in; a.out = *out;
+  a.family = family; a.n_families = h->n_families;
+  return launch(h, a, stream);
+}
+
 int tfem_solve_only(tfem_handle_t h, int B, const double* y, const int32_t* section, double* d, double* axial,
                     double* ratio, double* U, double* reactions, int32_t* status, void* stream) {
   if (!h || !y || !section) return fail(TFEM_ERR_ARG, "null argument");
+  if (int rc = single_family(h, "tfem_solve_only", "a handle of one family")) return rc;
   if (B < 0) return fail(TFEM_ERR_ARG, "negative batch");
   tfem::StepArgs a{};
   a.B = B; a.mode = tfem::MODE_SOLVE_ONLY; a.so_y = y; a.so_sec = section;
@@ -196,6 +324,7 @@ int tfem_solve_only(tfem_handle_t h, int B, const double* y, const int32_t* sect
 int tfem_read_genes(tfem_handle_t h, int B, const double* genes, double max_height, float int_obj1, float int_obj2,
                     const tfem_genes_out* out, void* stream) {
   if (!h || !genes || !out) return fail(TFEM_ERR_ARG, "null argument");
+  if (int rc = single_family(h, "tfem_read_genes", "a handle of one family")) return rc;
   if (B < 0) return fail(TFEM_ERR_ARG, "negative batch");
   if (!(max_height > 0.0)) return fail(TFEM_ERR_ARG, "max_height must be positive");
   if (out->point && !aligned16(out->point)) return fail(TFEM_ERR_ALIGN, "point must be 16-byte aligned");
@@ -211,6 +340,7 @@ int tfem_read_genes(tfem_handle_t h, int B, const double* genes, double max_heig
 int tfem_solve_dense_dmma(tfem_handle_t h, int B, const double* y, const int32_t* section, double* d,
                           int32_t* status, void* stream) {
   if (!h || !y || !section || !d) return fail(TFEM_ERR_ARG, "null argument");
+  if (int rc = single_family(h, "tfem_solve_dense_dmma", "a handle of one family")) return rc;
   if (B < 0) return fail(TFEM_ERR_ARG, "negative batch");
   if (h->device < 0) return fail(TFEM_ERR_CUDA, "tables-only handle (device < 0): libtfem has no CPU path");
   if (B == 0) return TFEM_OK;
@@ -224,6 +354,7 @@ int tfem_solve_dense_dmma(tfem_handle_t h, int B, const double* y, const int32_t
 
 int tfem_step_host(tfem_handle_t h, int B, const tfem_step_in* in, const tfem_step_out* out, void* stream_) {
   if (!h || !in || !out) return fail(TFEM_ERR_ARG, "null argument");
+  if (int rc = single_family(h, "tfem_step_host", "tfem_step_mixed on device buffers")) return rc;
   if (B <= 0) return B == 0 ? TFEM_OK : fail(TFEM_ERR_ARG, "negative batch");
   if (!in->set_node || !in->set_element || !in->a_geo || !in->a_topo || !in->move_range)
     return fail(TFEM_ERR_ARG, "set_node, set_element, a_geo, a_topo and move_range are required");
@@ -308,3 +439,5 @@ int64_t tfem_launch_count(tfem_handle_t h) { return h ? h->launches.load() : 0; 
 void tfem_book_launches(tfem_handle_t h, int64_t n) { if (h) h->launches.fetch_add(n); }
 
 }  // extern "C"
+
+int tfem::handle_family_count(tfem_handle_t h) { return h ? h->n_families : 0; }

@@ -167,15 +167,21 @@ __host__ __device__ constexpr int align16(int v) { return (v + 15) & ~15; }
 #define TFEM_MINB_LARGE 2
 #endif
 // GM = false: env-step / reset / solve-only (args.mode); GM = true: the gene-vector objective (MODE_GENES) -- a separate
-// instantiation so that the env-step keeps its register allocation
-template <int NX, bool GM>
+// instantiation so that the env-step keeps its register allocation.
+// MF = true: mixed-family env-step / reset (tfem_step_mixed, tfem_reset_mixed).  The CTA stages args.n_families tables of
+// one topology and ONE copy of the output maps (they depend on N, E and conn only); each environment reads its tables
+// through fam = staged + family[b].  Values read before the environment loop are topology and come from table 0.
+template <int NX, bool GM, bool MF>
 __global__ void __launch_bounds__(WARPS_PER_CTA * 32, (NX <= 8) ? TFEM_MINB_SMALL : TFEM_MINB_LARGE)
 tfem_step_kernel(const StepArgs args) {
+  static_assert(!(GM && MF), "the gene-vector objective has no mixed-family form");
   using D = Dims<NX>;
   constexpr int N = D::N, E = D::E, NI = D::NI, EPL = D::EPL;
   extern __shared__ __align__(16) unsigned char smem_raw[];
-  FamilyTables* fam = reinterpret_cast<FamilyTables*>(smem_raw);
-  uint16_t* maps = reinterpret_cast<uint16_t*>(smem_raw + align16((int)sizeof(FamilyTables)));
+  FamilyTables* const fams = reinterpret_cast<FamilyTables*>(smem_raw);
+  FamilyTables* fam = fams;
+  const int tab_bytes = MF ? args.n_families * (int)sizeof(FamilyTables) : (int)sizeof(FamilyTables);
+  uint16_t* maps = reinterpret_cast<uint16_t*>(smem_raw + align16(tab_bytes));
 
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int mode = GM ? (int)MODE_GENES : args.mode;
@@ -184,12 +190,15 @@ tfem_step_kernel(const StepArgs args) {
   // ---- per-env inputs are fetched one environment ahead (the first batch overlaps the table staging) ----
   float in_y = 0.f, in_at0 = 0.f, in_at1 = 0.f, in_at2 = 0.f, in_sec[EPL];
   float2 in_mr = make_float2(0.f, 0.f), in_ag = make_float2(0.f, 0.f);
-  int in_coin = 0;
+  int in_coin = 0, in_fam = 0;
   // the two live columns of the parent tables: compact arrays when the caller has them, else column 1 / column 0
   const float* const col_y = args.in.set_node_y ? args.in.set_node_y : args.in.set_node + 1;
   const float* const col_sec = args.in.set_element_section ? args.in.set_element_section : args.in.set_element;
   const int col_y_stride = args.in.set_node_y ? 1 : 12, col_sec_stride = args.in.set_element_section ? 1 : 21;
   auto fetch_inputs = [&](int b) {
+    if constexpr (MF) {
+      if (b < args.B) in_fam = args.family[b];
+    }
     if (mode != MODE_STEP || b >= args.B) return;
     in_y = col_y[((size_t)b * N + node) * col_y_stride];
     in_mr = reinterpret_cast<const float2*>(args.in.move_range)[(size_t)b * N + node];
@@ -206,7 +215,7 @@ tfem_step_kernel(const StepArgs args) {
   {  // stage the family tables and output maps once per CTA (L2-resident, 8..15 KB)
     const uint4* src = reinterpret_cast<const uint4*>(args.fam);
     uint4* dst = reinterpret_cast<uint4*>(fam);
-    for (int i = tid; i < (int)(sizeof(FamilyTables) / 16); i += blockDim.x) dst[i] = src[i];
+    for (int i = tid; i < tab_bytes / 16; i += blockDim.x) dst[i] = src[i];
     const uint4* msrc = reinterpret_cast<const uint4*>(args.maps);
     uint4* mdst = reinterpret_cast<uint4*>(maps);
     for (int i = tid; i < args.map_entries / 8; i += blockDim.x) mdst[i] = msrc[i];
@@ -216,7 +225,7 @@ tfem_step_kernel(const StepArgs args) {
   asm volatile("griddepcontrol.wait;" ::: "memory");
   fetch_inputs(blockIdx.x * WARPS_PER_CTA + warp);
   __syncthreads();
-  unsigned char* wbase = smem_raw + align16((int)sizeof(FamilyTables)) + align16(args.map_entries * 2) + warp * D::WARP_BYTES;
+  unsigned char* wbase = smem_raw + align16(tab_bytes) + align16(args.map_entries * 2) + warp * D::WARP_BYTES;
   double* Kb = reinterpret_cast<double*>(wbase);            // [NI][BAND]: Kb[j*8+k] = K[j+k][j]
   double* z = Kb + (NI + PADC) * BAND;                      // [NI + PADC] rhs -> solution
   double* dinv = z + NI + PADC;                             // [NI] 1 / pivot
@@ -227,8 +236,10 @@ tfem_step_kernel(const StepArgs args) {
   double* g = reinterpret_cast<double*>(dyn);               // [E][3] element stiffness terms (needs 16B align)
   float* at_s = dyn;                                        // [N][3] clipped a_topo (before g is written)
   int* sec_s = reinterpret_cast<int*>(dyn + 3 * N);         // [E] sections after the action
-  for (int i = lane; i < pl.dyn_base(); i += 32) pool[i] = fam->pool_const[i];
+  if constexpr (!MF)                        // mixed launches copy it per family, in the environment loop
+    for (int i = lane; i < pl.dyn_base(); i += 32) pool[i] = fam->pool_const[i];
   __syncwarp();
+  int pool_fam = -1;                         // MF: the family whose constant columns the pool holds
 
   // trailing-update role of this lane: (a, b), 1 <= b <= a <= 7, for lanes 0..27
   int ta = 0, tb = 0;
@@ -244,6 +255,20 @@ tfem_step_kernel(const StepArgs args) {
   const bool is_top = fam->top[node] != 0;
 
   for (int b = blockIdx.x * WARPS_PER_CTA + warp; b < args.B; b += warps_total) {
+    if constexpr (MF) {
+      const int f = in_fam;
+      if (f >= args.n_families) {            // no table is read and nothing but the status is written
+        fetch_inputs(b + warps_total);
+        if (lane == 0 && args.out.status) args.out.status[b] = TFEM_STATUS_BAD_FAMILY;
+        continue;
+      }
+      fam = fams + f;
+      if (f != pool_fam) {                   // normalised x / support / load columns differ between families
+        for (int i = lane; i < pl.dyn_base(); i += 32) pool[i] = fam->pool_const[i];
+        __syncwarp();
+        pool_fam = f;
+      }
+    }
     int status = 0;
     TS y, yp;                                // this node's height and its vertical pair's
     int sec[EPL];
@@ -357,7 +382,8 @@ tfem_step_kernel(const StepArgs args) {
         if (e < E) sec[p] = min(sec[p], sec_s[fam->sym_elem[e]]);
       }
       __syncwarp();
-    } else if (mode == MODE_RESET) {
+    } else if (MF || mode == MODE_RESET) {
+      if constexpr (MF) fetch_inputs(b + warps_total);
       y = W(fam->y0[node]);
       yp = W(fam->y0[fam->pair[node]]);
 #pragma unroll
@@ -677,20 +703,46 @@ tfem_step_kernel(const StepArgs args) {
 }
 
 template <int NX>
-int smem_bytes_for(int map_entries) {
-  return align16((int)sizeof(FamilyTables)) + align16(((map_entries + 7) & ~7) * 2) + WARPS_PER_CTA * Dims<NX>::WARP_BYTES;
+int smem_bytes_for(int map_entries, int n_tables = 1) {
+  return align16(n_tables * (int)sizeof(FamilyTables)) + align16(((map_entries + 7) & ~7) * 2) + WARPS_PER_CTA * Dims<NX>::WARP_BYTES;
 }
 
 }  // namespace
 
 namespace {
-template <int NX, bool GM>
+template <int NX, bool GM, bool MF>
 cudaError_t configure_one(int smem, int* ctas) {
-  cudaError_t err = cudaFuncSetAttribute(tfem_step_kernel<NX, GM>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+  cudaError_t err = cudaFuncSetAttribute(tfem_step_kernel<NX, GM, MF>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
   if (err != cudaSuccess) return err;
-  err = cudaFuncSetAttribute(tfem_step_kernel<NX, GM>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+  err = cudaFuncSetAttribute(tfem_step_kernel<NX, GM, MF>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
   if (err != cudaSuccess) return err;
-  return cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas, tfem_step_kernel<NX, GM>, WARPS_PER_CTA * 32, smem);
+  return cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas, tfem_step_kernel<NX, GM, MF>, WARPS_PER_CTA * 32, smem);
+}
+
+// The opt-in size is an attribute of the function, shared by every live handle of this NX.  It is set to what the
+// largest family count needs (capped by the device's per-block limit), never to what one handle needs, so creating a
+// handle of few families cannot break a live handle of more.
+template <int NX>
+cudaError_t configure_mixed_nx(int map_entries, int single_ctas, int n_families, int* smem, int* max_families) {
+  int dev = 0, optin = 0;
+  cudaError_t err = cudaGetDevice(&dev);
+  if (err == cudaSuccess) err = cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
+  if (err != cudaSuccess) return err;
+  int top = TFEM_MAX_FAMILIES;
+  while (top > 1 && smem_bytes_for<NX>(map_entries, top) > optin) --top;
+  int ctas = 0;
+  err = configure_one<NX, false, true>(smem_bytes_for<NX>(map_entries, top), &ctas);
+  if (err != cudaSuccess) return err;
+  *max_families = 0;
+  for (int f = 1; f <= top; ++f) {
+    err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas, tfem_step_kernel<NX, false, true>, WARPS_PER_CTA * 32,
+                                                        smem_bytes_for<NX>(map_entries, f));
+    if (err != cudaSuccess) return err;
+    if (ctas < single_ctas) break;
+    *max_families = f;
+  }
+  *smem = (n_families <= *max_families) ? smem_bytes_for<NX>(map_entries, n_families) : 0;
+  return cudaSuccess;
 }
 }  // namespace
 
@@ -699,16 +751,16 @@ int step_kernel_configure(int nx, int device, int map_entries, LaunchInfo* info)
   int smem = 0, ctas = 0, ctas_g = 0, sms = 0;
   if (nx == 6) {                   // the 6 x 2 shapes of train/code/master_DDPG_truss2D_MO.py:787-795
     smem = smem_bytes_for<6>(map_entries);
-    err = configure_one<6, false>(smem, &ctas);
-    if (err == cudaSuccess) err = configure_one<6, true>(smem, &ctas_g);
+    err = configure_one<6, false, false>(smem, &ctas);
+    if (err == cudaSuccess) err = configure_one<6, true, false>(smem, &ctas_g);
   } else if (nx == 8) {
     smem = smem_bytes_for<8>(map_entries);
-    err = configure_one<8, false>(smem, &ctas);
-    if (err == cudaSuccess) err = configure_one<8, true>(smem, &ctas_g);
+    err = configure_one<8, false, false>(smem, &ctas);
+    if (err == cudaSuccess) err = configure_one<8, true, false>(smem, &ctas_g);
   } else if (nx == 16) {
     smem = smem_bytes_for<16>(map_entries);
-    err = configure_one<16, false>(smem, &ctas);
-    if (err == cudaSuccess) err = configure_one<16, true>(smem, &ctas_g);
+    err = configure_one<16, false, false>(smem, &ctas);
+    if (err == cudaSuccess) err = configure_one<16, true, false>(smem, &ctas_g);
   } else {
     return (int)cudaErrorInvalidValue;
   }
@@ -722,29 +774,43 @@ int step_kernel_configure(int nx, int device, int map_entries, LaunchInfo* info)
   info->ctas_per_sm = ctas;
   info->grid = sms * ctas;          // persistent: a multiple of the SM count, warps stride over envs
   info->grid_genes = sms * ctas_g;
+  info->smem_mixed = 0;
   return 0;
+}
+
+int step_kernel_configure_mixed(int nx, int map_entries, int n_families, LaunchInfo* info, int* max_families) {
+  cudaError_t err;
+  if (nx == 6) err = configure_mixed_nx<6>(map_entries, info->ctas_per_sm, n_families, &info->smem_mixed, max_families);
+  else if (nx == 8) err = configure_mixed_nx<8>(map_entries, info->ctas_per_sm, n_families, &info->smem_mixed, max_families);
+  else if (nx == 16) err = configure_mixed_nx<16>(map_entries, info->ctas_per_sm, n_families, &info->smem_mixed, max_families);
+  else return (int)cudaErrorInvalidValue;
+  return (int)err;
 }
 
 int step_kernel_launch(int nx, const StepArgs& args, const LaunchInfo& info, cudaStream_t stream) {
   if (args.B <= 0) return 0;
-  const bool gm = args.mode == MODE_GENES;
+  const bool gm = args.mode == MODE_GENES, mf = args.family != nullptr;
+  if (mf && (gm || info.smem_mixed <= 0)) return (int)cudaErrorInvalidValue;
   const int needed = (args.B + WARPS_PER_CTA - 1) / WARPS_PER_CTA;
   const int full = gm ? info.grid_genes : info.grid;
   const int grid = needed < full ? needed : full;
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3((unsigned)info.block);
-  cfg.dynamicSmemBytes = (size_t)info.smem_bytes; cfg.stream = stream;
+  cfg.dynamicSmemBytes = (size_t)(mf ? info.smem_mixed : info.smem_bytes); cfg.stream = stream;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;     // see griddepcontrol.wait in the kernel
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr; cfg.numAttrs = 1;
   cudaError_t e;
-  if (nx == 6 && !gm) e = cudaLaunchKernelEx(&cfg, tfem_step_kernel<6, false>, args);
-  else if (nx == 6) e = cudaLaunchKernelEx(&cfg, tfem_step_kernel<6, true>, args);
-  else if (nx == 8 && !gm) e = cudaLaunchKernelEx(&cfg, tfem_step_kernel<8, false>, args);
-  else if (nx == 8) e = cudaLaunchKernelEx(&cfg, tfem_step_kernel<8, true>, args);
-  else if (nx == 16 && !gm) e = cudaLaunchKernelEx(&cfg, tfem_step_kernel<16, false>, args);
-  else if (nx == 16) e = cudaLaunchKernelEx(&cfg, tfem_step_kernel<16, true>, args);
+  if (nx == 6 && mf) e = cudaLaunchKernelEx(&cfg, tfem_step_kernel<6, false, true>, args);
+  else if (nx == 6 && !gm) e = cudaLaunchKernelEx(&cfg, tfem_step_kernel<6, false, false>, args);
+  else if (nx == 6) e = cudaLaunchKernelEx(&cfg, tfem_step_kernel<6, true, false>, args);
+  else if (nx == 8 && mf) e = cudaLaunchKernelEx(&cfg, tfem_step_kernel<8, false, true>, args);
+  else if (nx == 8 && !gm) e = cudaLaunchKernelEx(&cfg, tfem_step_kernel<8, false, false>, args);
+  else if (nx == 8) e = cudaLaunchKernelEx(&cfg, tfem_step_kernel<8, true, false>, args);
+  else if (nx == 16 && mf) e = cudaLaunchKernelEx(&cfg, tfem_step_kernel<16, false, true>, args);
+  else if (nx == 16 && !gm) e = cudaLaunchKernelEx(&cfg, tfem_step_kernel<16, false, false>, args);
+  else if (nx == 16) e = cudaLaunchKernelEx(&cfg, tfem_step_kernel<16, true, false>, args);
   else return (int)cudaErrorInvalidValue;
   return (int)(e != cudaSuccess ? e : cudaGetLastError());
 }

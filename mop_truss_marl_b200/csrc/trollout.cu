@@ -11,6 +11,7 @@
 #include <vector>
 
 #include "../../include/trollout.h"
+#include "tfem_kernels.cuh"
 
 namespace {
 struct Dev {
@@ -143,6 +144,10 @@ int trollout_create(tfem_handle_t env, tactor_handle_t actor, int max_batch, int
   if (!h) return rfail(TFEM_ERR_ARG, "out of host memory");
   h->env = env; h->actor = actor; h->max_batch = max_batch;
   if (tfem_get_dims(env, &h->dims) != TFEM_OK) { delete h; return rfail(TFEM_ERR_ARG, "bad env handle"); }
+  if (tfem::handle_family_count(env) > 1) {       // the captured pipeline carries no per-environment family ids
+    delete h;
+    return rfail(TFEM_ERR_UNSUPPORTED, "the env handle holds several families (tfem_create_mixed): the rollout steps one family");
+  }
   int piece = (max_batch + pieces - 1) / pieces;
   piece = (piece + 31) / 32 * 32;                  // piece boundaries on 32 environments: every sub-array stays 16-byte aligned
   for (int lo = 0; lo < max_batch; lo += piece) h->piece_len.push_back(piece);

@@ -65,6 +65,10 @@ for _i, _tar in enumerate(_TRAIN_TAR):
         FAMILIES["train%d_%s" % (_i, _tt)] = FamilySpec("train%d_%s" % (_i, _tt), 6, (4.0, 3.0, 5.0, 3.0, 5.0), (5,), _tar, 0.2, 0,
                                                         -100000, _tt, 1, SYM_NONE)
 
+# the ten training families (five shapes x two truss types) in a fixed order: the index of a name here is the family id
+# of a mixed-family batch built over TRAIN_FAMILIES (batched_env.MixedTrussEnv)
+TRAIN_FAMILIES = tuple("train%d_%s" % (_i, _tt) for _i in range(len(_TRAIN_TAR)) for _tt in ("roof", "bridge"))
+
 
 def family_desc(spec: FamilySpec):
     """FamilySpec -> ctypes ``tfem_family_desc``"""
