@@ -335,7 +335,6 @@ struct PackArgs {
   uint32_t* w1frag;
   float* wscale_inv;                   // [NGEMM + 3]
   float* wmax;                         // [TACTOR_NLAYERS] scratch: max(|W|, |b|) per layer
-  int ncta;
 };
 __constant__ int kInDev[TACTOR_NLAYERS] = {13, 13, 13, 4, 200, 200, 200, 200, 200, 200, 200, 200, 200};
 __constant__ int kOutDev[TACTOR_NLAYERS] = {200, 200, 200, 200, 200, 200, 200, 200, 200, 200, 200, 2, 3};
@@ -377,23 +376,22 @@ __global__ void __launch_bounds__(256) pack_plain_kernel(PackArgs a) {
   if (blockIdx.x == 0 && threadIdx.x < LD) a.d_b[l][threadIdx.x] = threadIdx.x < kout ? a.bias[l][threadIdx.x] : 0.f;
 }
 
-// tcgen05 operand images of the seven [200,200] layers (grid: layer 4..10 x blocks): per 16-wide K chunk, per CTA of the pair
-// (its half of the 208 columns), [hi | lo][kb][n][8 halfs]; row k = 200 holds the bias
+// tcgen05 operand images of the seven [200,200] layers (grid: layer 4..10 x blocks): per 16-wide K chunk
+// [hi | lo][kb][n][8 halfs]; row k = 200 holds the bias
 __global__ void __launch_bounds__(256) pack_img_kernel(PackArgs a) {
   const int l = 4 + blockIdx.y, K = kInDev[l], kout = kOutDev[l];
-  const int bn = tc::TCN / a.ncta, kpc = tc::KPC, nkb = tc::KCH / kpc;
+  const int bn = tc::TCN, kpc = tc::KPC, nkb = tc::KCH / kpc;
   const int nch = (K + 1 + tc::KCH - 1) / tc::KCH;
-  const int total = nch * a.ncta * 2 * nkb * bn * kpc;
+  const int total = nch * 2 * nkb * bn * kpc;
   const float scale = pow2_scale_dev(a.wmax[l]);
   for (int idx = blockIdx.x * 256 + threadIdx.x; idx < total; idx += gridDim.x * 256) {
     int r = idx;
     const int t = r % kpc; r /= kpc;
-    const int nl = r % bn; r /= bn;
+    const int n = r % bn; r /= bn;
     const int kb = r % nkb; r /= nkb;
     const int part = r % 2; r /= 2;
-    const int half = r % a.ncta; r /= a.ncta;
     const int c = r;
-    const int n = half * bn + nl, k = c * tc::KCH + kpc * kb + t;
+    const int k = c * tc::KCH + kpc * kb + t;
     float v = 0.f;
     if (n < kout && k < K) v = a.kernel[l][(size_t)k * kout + n] * scale;
     else if (n < kout && k == K) v = a.bias[l][n] * scale;
@@ -476,10 +474,7 @@ struct tactor_handle_s {
   uint32_t* d_w1frag = nullptr;        // mma.sync A-fragment image of the three layer-1 kernels (tactor_pipe.cuh)
   float* d_wmax = nullptr;             // [13] scratch of tactor_set_weights_device
   float* d_wscale_inv = nullptr;       // [NGEMM + 3] 1 / power-of-two scale of d_wimg[4 + g] and of the three layer-1 images
-  int dev_flags = 0;                   // TACTOR_FLAGS (development switches of the actor kernel)
-  int variant = 0;                     // generator phases / epilogue warps of actor_pipe_kernel (TACTOR_VARIANT, A/B timing)
   int* d_error = nullptr;              // set by a kernel whose mbarrier wait timed out
-  int ncta = 1;                        // CTAs per tcgen05 group (2 = CTA pair, cta_group::2)
   int sms = 0;                         // SM count of the device (persistent grid, tile splitting of the last wave); TACTOR_NO_SPLIT=1:
                                        // one CTA per unsplit tile
   std::atomic<int64_t> launches{0};
@@ -497,71 +492,41 @@ struct Guard {
   ~Guard() { if (prev >= 0) cudaSetDevice(prev); }
 };
 
-template <int NODES, int NCTA, int NPH, int NEPIW, int NREAL = NODES>
+template <int NODES, int NREAL = NODES>
 cudaError_t launch_pipe(tactor::tc::fused::Params& p, int M, int sms, cudaStream_t st) {
   using namespace tactor;
   const int tiles = (M + tc::TCM - 1) / tc::TCM;
   // wave quantisation: one CTA per SM, so `tiles % sms` tiles would run as a last wave that leaves most SMs idle.
   // Cut those tiles into 2 or 4 row pieces (one CTA each) when the pieces still fit one wave.
-  int grid = (tiles + NCTA - 1) / NCTA * NCTA;
+  int grid = tiles;
   p.split_from = grid; p.split_f = 1;
-  if (NCTA == 1 && sms > 0) {
+  if (sms > 0) {
     const int rem = tiles % sms, full = tiles - rem;
     const int f = (rem > 0 && 4 * rem <= sms) ? 4 : (rem > 0 && 2 * rem <= sms) ? 2 : 1;
     if (f > 1) { p.split_from = full; p.split_f = f; grid = full + f * rem; }
   }
   p.n_items = grid;
-  if (NCTA == 1 && sms > 0 && grid > sms) grid = sms;      // persistent: one CTA per SM walks the items
+  if (sms > 0 && grid > sms) grid = sms;                   // persistent: one CTA per SM walks the items
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3((unsigned)grid);
-  cfg.blockDim = dim3((unsigned)tc::pipe::pipe_threads<NPH, NEPIW>());
-  cfg.dynamicSmemBytes = tc::pipe::pipe_smem_bytes<NODES, NCTA>();
+  cfg.blockDim = dim3((unsigned)tc::pipe::PTHREADS);
+  cfg.dynamicSmemBytes = tc::pipe::pipe_smem_bytes<NODES>();
   cfg.stream = st;
   cudaLaunchAttribute attr[2];
   attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = NCTA; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
+  attr[0].val.clusterDim.x = 1; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
   // programmatic dependent launch: the kernel's set-up (TMEM, barriers, weights) runs beside the Pareto-branch kernel that
   // precedes it; the generators wait (griddepcontrol.wait) before they touch its output or the state tensors
   attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr; cfg.numAttrs = (NCTA == 1) ? 2 : 1;
-  return cudaLaunchKernelEx(&cfg, tc::pipe::actor_pipe_kernel<NODES, NCTA, NPH, NEPIW, NREAL>, p);
+  cfg.attrs = attr; cfg.numAttrs = 2;
+  return cudaLaunchKernelEx(&cfg, tc::pipe::actor_pipe_kernel<NODES, NREAL>, p);
 }
 
-template <int NODES, int NCTA, int NPH, int NEPIW, int NREAL = NODES>
+template <int NODES, int NREAL = NODES>
 cudaError_t set_pipe_smem() {
-  return cudaFuncSetAttribute(tactor::tc::pipe::actor_pipe_kernel<NODES, NCTA, NPH, NEPIW, NREAL>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                              tactor::tc::pipe::pipe_smem_bytes<NODES, NCTA>());
-}
-
-// Build variants of actor_pipe_kernel: (generator phases, epilogue warps).  0 = (2, 4) is the production choice (measured
-// fastest for both node counts on the final build: 0.181 ms small bridge 4096, 0.706 ms large bridge 8192; (3, 4) 0.186 / 0.787,
-// (2, 8) 0.186 / 0.870, (3, 8) 0.192 / 0.807, (4, 4) 0.188 / 0.780, 5 = (1, 4) 0.208 / 0.853 -- half the generator warps, 15 % slower:
-// the two phases of a row group share a scheduler and mostly run in lock-step); the others are kept for A/B timing (TACTOR_VARIANT).
-// The CTA-pair build exists for variant 0 only.
-template <int NODES>
-cudaError_t set_pipe_smem_variant(int ncta, int variant) {
-  if (ncta == 2) return set_pipe_smem<NODES, 2, 2, 8>();
-  switch (variant) {
-    case 1: return set_pipe_smem<NODES, 1, 3, 4>();
-    case 2: return set_pipe_smem<NODES, 1, 2, 8>();
-    case 3: return set_pipe_smem<NODES, 1, 3, 8>();
-    case 4: return set_pipe_smem<NODES, 1, 4, 4>();
-    case 5: return set_pipe_smem<NODES, 1, 1, 4>();
-    default: return set_pipe_smem<NODES, 1, 2, 4>();
-  }
-}
-template <int NODES>
-cudaError_t launch_pipe_variant(int ncta, int variant, tactor::tc::fused::Params& p, int M, int sms, cudaStream_t st) {
-  if (ncta == 2) return launch_pipe<NODES, 2, 2, 8>(p, M, sms, st);
-  switch (variant) {
-    case 1: return launch_pipe<NODES, 1, 3, 4>(p, M, sms, st);
-    case 2: return launch_pipe<NODES, 1, 2, 8>(p, M, sms, st);
-    case 3: return launch_pipe<NODES, 1, 3, 8>(p, M, sms, st);
-    case 4: return launch_pipe<NODES, 1, 4, 4>(p, M, sms, st);
-    case 5: return launch_pipe<NODES, 1, 1, 4>(p, M, sms, st);
-    default: return launch_pipe<NODES, 1, 2, 4>(p, M, sms, st);
-  }
+  return cudaFuncSetAttribute(tactor::tc::pipe::actor_pipe_kernel<NODES, NREAL>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                              tactor::tc::pipe::pipe_smem_bytes<NODES>());
 }
 
 // (re)builds the device copies of the weights: packed [Kpad,208] kernels / [208] biases and the tcgen05 operand
@@ -580,12 +545,10 @@ cudaError_t upload_weights(tactor_handle_s* h, const tactor_weights* w) {
     if (e == cudaSuccess) e = cudaMemcpy(h->d_w[l], wp.data(), wp.size() * 4, cudaMemcpyHostToDevice);
     if (e == cudaSuccess) e = cudaMemcpy(h->d_b[l], bp.data(), bp.size() * 4, cudaMemcpyHostToDevice);
   }
-  // tcgen05 operand images of the [200,200] layers: per 16-wide K chunk, per CTA of the pair (its half of the 208
-  // columns), [hi|lo][kb][n][8 halfs].  W is scaled by S = 2^s (largest s with max(|W|, |b|) S < 2^14, so that hi and lo stay
+  // tcgen05 operand images of the [200,200] layers: per 16-wide K chunk, [hi|lo][kb][n][8 halfs].  W is scaled by S = 2^s (largest s with max(|W|, |b|) S < 2^14, so that hi and lo stay
   // normal fp16 numbers), hi = fp16(W S), lo = fp16(W S - hi); the kernel's epilogue multiplies the accumulator by 1/S
   // (exact).  Row k = 200 of the image (inside the zero-padded tail chunk) holds the bias: the generators feed a constant
   // 1 in column 200 of A.
-  const int bn = tactor::tc::TCN / h->ncta;
   float wscale_inv[tactor::tc::fused::NGEMM + 3];
   auto pow2_scale = [](float wmax, float& scale, float& inv) {     // largest 2^s with wmax 2^s < 2^14
     int ex = 0;
@@ -605,19 +568,17 @@ cudaError_t upload_weights(tactor_handle_s* h, const tactor_weights* w) {
     std::vector<__half> img;
     const int kpc = tactor::tc::KPC, nkb = tactor::tc::KCH / kpc;
     for (int c = 0; c * tactor::tc::KCH < K + 1; ++c)
-      for (int half = 0; half < h->ncta; ++half)
-        for (int part = 0; part < 2; ++part)
-          for (int kb = 0; kb < nkb; ++kb)
-            for (int nl = 0; nl < bn; ++nl)
-              for (int t = 0; t < kpc; ++t) {
-                const int n = half * bn + nl;
-                const int k = c * tactor::tc::KCH + kpc * kb + t;
-                float v = 0.f;
-                if (n < kout && k < K) v = w->kernel[l][(size_t)k * kout + n] * scale;
-                else if (n < kout && k == K) v = w->bias[l][n] * scale;       // A's column K is the constant 1
-                const __half hi = __float2half_rn(v);
-                img.push_back(part == 0 ? hi : __float2half_rn(v - __half2float(hi)));
-              }
+      for (int part = 0; part < 2; ++part)
+        for (int kb = 0; kb < nkb; ++kb)
+          for (int n = 0; n < tactor::tc::TCN; ++n)
+            for (int t = 0; t < kpc; ++t) {
+              const int k = c * tactor::tc::KCH + kpc * kb + t;
+              float v = 0.f;
+              if (n < kout && k < K) v = w->kernel[l][(size_t)k * kout + n] * scale;
+              else if (n < kout && k == K) v = w->bias[l][n] * scale;         // A's column K is the constant 1
+              const __half hi = __float2half_rn(v);
+              img.push_back(part == 0 ? hi : __float2half_rn(v - __half2float(hi)));
+            }
     if (!h->d_wimg[l]) e = cudaMalloc(&h->d_wimg[l], img.size() * sizeof(__half));
     if (e == cudaSuccess) e = cudaMemcpy(h->d_wimg[l], img.data(), img.size() * sizeof(__half), cudaMemcpyHostToDevice);
   }
@@ -711,10 +672,10 @@ cudaError_t run_forward(tactor_handle_s* h, int B, const tactor_inputs* in, floa
   for (int g = 0; g < tc::fused::NGEMM; ++g) { p.wimg[g] = h->d_wimg[4 + g]; p.bias[g] = h->d_b[4 + g]; }
   p.wscale_inv = h->d_wscale_inv; p.w1frag = h->d_w1frag;
   p.w_head[0] = h->d_w[11]; p.w_head[1] = h->d_w[12]; p.b_head[0] = h->d_b[11]; p.b_head[1] = h->d_b[12];
-  p.geo = geo; p.topo = topo; p.M = M; p.error_flag = h->d_error; p.dev_flags = h->dev_flags;
+  p.geo = geo; p.topo = topo; p.M = M; p.error_flag = h->d_error;
   p.noise = nz.on; p.mu = nz.mu; p.theta = nz.theta; p.sigma = nz.sigma; p.seed = nz.seed; p.call = nz.call; p.seed_call = nz.seed_call;
-  cudaError_t e = (h->n_real == 12) ? launch_pipe<16, 1, 2, 4, 12>(p, M, h->sms, st)      // the padded 12-node build
-                                    : launch_pipe_variant<NODES>(h->ncta, h->variant, p, M, h->sms, st);
+  cudaError_t e = (h->n_real == 12) ? launch_pipe<16, 12>(p, M, h->sms, st)      // the padded 12-node build
+                                    : launch_pipe<NODES>(p, M, h->sms, st);
   h->launches.fetch_add(2);
   return e != cudaSuccess ? e : cudaGetLastError();
 }
@@ -737,9 +698,6 @@ int tactor_create(const tactor_weights* w, int nodes, int max_batch, int device,
   tactor_handle_s* h = new (std::nothrow) tactor_handle_s();
   if (!h) return afail(TFEM_ERR_ARG, "out of host memory");
   h->device = device; h->nodes = nodes; h->n_real = n_real; h->max_batch = max_batch;
-  if (const char* v = getenv("TACTOR_NCTA")) h->ncta = (atoi(v) == 2) ? 2 : 1;     // development switches (A/B timing)
-  if (const char* v = getenv("TACTOR_VARIANT")) h->variant = atoi(v);
-  if (const char* v = getenv("TACTOR_FLAGS")) h->dev_flags = atoi(v);
   Guard g(device);
   for (int l = 0; l < TACTOR_NLAYERS; ++l)
     if (!w->kernel[l] || !w->bias[l]) { tactor_destroy(h); return afail(TFEM_ERR_ARG, "missing layer weights"); }
@@ -748,8 +706,8 @@ int tactor_create(const tactor_weights* w, int nodes, int max_batch, int device,
   if (const char* v = getenv("TACTOR_NO_SPLIT")) { if (v[0] == '1') h->sms = 0; }
   if (e == cudaSuccess) e = cudaMalloc(&h->d_error, 65536);
   if (e == cudaSuccess) e = cudaMemset(h->d_error, 0, 65536);
-  if (e == cudaSuccess) e = (nodes == 16) ? set_pipe_smem_variant<16>(h->ncta, h->variant) : set_pipe_smem_variant<32>(h->ncta, h->variant);
-  if (e == cudaSuccess && n_real == 12) e = set_pipe_smem<16, 1, 2, 4, 12>();
+  if (e == cudaSuccess) e = (nodes == 16) ? set_pipe_smem<16>() : set_pipe_smem<32>();
+  if (e == cudaSuccess && n_real == 12) e = set_pipe_smem<16, 12>();
   if (e == cudaSuccess)
     e = (nodes == 16) ? cudaFuncSetAttribute(tactor::pareto_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, tactor::PARETO_SMEM)
                       : cudaFuncSetAttribute(tactor::pareto_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, tactor::PARETO_SMEM);
@@ -790,7 +748,7 @@ int tactor_set_weights_device(tactor_handle_t h, const tactor_weights* w, void* 
     a.d_w[l] = h->d_w[l]; a.d_b[l] = h->d_b[l];
     a.d_wimg[l] = reinterpret_cast<__half*>(h->d_wimg[l]);
   }
-  a.w1frag = h->d_w1frag; a.wscale_inv = h->d_wscale_inv; a.wmax = h->d_wmax; a.ncta = h->ncta;
+  a.w1frag = h->d_w1frag; a.wscale_inv = h->d_wscale_inv; a.wmax = h->d_wmax;
   cudaStream_t st = (cudaStream_t)stream;
   tactor::pack_wmax_kernel<<<TACTOR_NLAYERS, 256, 0, st>>>(a);
   tactor::pack_plain_kernel<<<dim3(16, TACTOR_NLAYERS), 256, 0, st>>>(a);

@@ -1,6 +1,6 @@
 // Whole-network fused actor kernel, fully pipelined ("pipe") formulation.
 //
-// One CTA (or CTA pair, NCTA = 2) carries a 128-row tile (ENVS environments of NODES nodes) through all 13
+// One CTA carries a 128-row tile (ENVS environments of NODES nodes) through all 13
 // GCNConv layers of multimodes_actor.call (train/code/truss2D_RL.py:75-127).  The adjacency product is moved IN FRONT
 // of the dense contraction,
 //
@@ -26,10 +26,9 @@
 //                            running ahead across GEMM boundaries
 //   issuer      1 warp       tcgen05.mma kind::f16 (Yhi.Whi + Yhi.Wlo + Ylo.Whi), A from tensor memory, B from
 //                            shared memory, accumulator g&1 of two (TMEM columns [0,208) and [256,464))
-//   epilogue    NEPIW warps  tcgen05.ld the finished accumulator while the next GEMM is already running (NEPIW = 8: two
-//                            warps per 32-row group, half of the columns each): relu(D / S) -> H (+)= (g <= 4), or the
-//                            sigmoid heads gcn_l4_1/2 (g = 5, 6); the bias is row 200 of the W image (A's column 200 is
-//                            the constant 1)
+//   epilogue    NEPIW warps  tcgen05.ld the finished accumulator while the next GEMM is already running (one warp per
+//                            32-row group): relu(D / S) -> H (+)= (g <= 4), or the sigmoid heads gcn_l4_1/2 (g = 5, 6);
+//                            the bias is row 200 of the W image (A's column 200 is the constant 1)
 //
 // TMEM map (512 columns): [0,208) acc0 | [208,256) A stages hi (6 x 8 columns of packed pairs) | [256,464) acc1
 //                         | [464,512) A stages lo
@@ -56,14 +55,16 @@ constexpr int LDH = 204;                                    // padded row length
                                                             // loads of layer 3 -- 4 row pairs x 8 features -- hit 32 distinct banks)
 constexpr int NCH = (KH + KCH - 1) / KCH;                   // 13 chunks per GEMM
 constexpr int W1F_WORDS = 3 * NCH * 2 * 32 * 4;             // layer-1 fragment image: [3][13][hi | lo][32 lanes][4]
+// warp roles: 4 NPH generators, NEPIW epilogue warps, issuer, W producer.  Measured fastest for both node counts against
+// 1, 3 or 4 generator phases and 8 epilogue warps (profiles/README.md)
+constexpr int NPH = 2;                                      // generator phases: a generator warp owns every NPH-th chunk
+constexpr int NEPIW = 4;                                    // epilogue warps, one per 32-row group
+constexpr int PTHREADS = (4 * NPH + NEPIW + 2) * 32;
 
-template <int NPH, int NEPIW>
-__host__ __device__ constexpr int pipe_threads() { return (4 * NPH + NEPIW + 2) * 32; }
-
-template <int NODES, int NCTA>
+template <int NODES>
 __host__ __device__ constexpr int pipe_smem_bytes() {
-  return Cfg<NCTA>::WST * Cfg<NCTA>::STAGE_BYTES + TCM * LDH * 4 + W1F_WORDS * 4 + 2 * (TCM / NODES) * 208 * 4 + 2 * TCM * 13 * 4 +
-         2 * NODES * NODES * 4 + 2 * 201 * 4 * 4 + 4 * TCM * 4 * 4 + 384;
+  return WST * STAGE_BYTES + TCM * LDH * 4 + W1F_WORDS * 4 + 2 * (TCM / NODES) * 208 * 4 + 2 * TCM * 13 * 4 +
+         2 * NODES * NODES * 4 + 2 * 201 * 4 * 4 + 2 * TCM * 4 * 4 + 384;
 }
 
 __device__ __forceinline__ uint32_t h2_bits(const __half2& h) { return *reinterpret_cast<const uint32_t*>(&h); }
@@ -80,9 +81,6 @@ __device__ __forceinline__ void tmem_ld8_async(uint32_t taddr, uint32_t* r) {
                : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
                : "r"(taddr));
 }
-__device__ __forceinline__ void named_bar_sync(int id, int count) {
-  asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(count) : "memory");
-}
 
 // -DTACTOR_PROF: per-warp wait / work cycle counters of CTA 0 (development build only: python -m mop_truss_marl_b200.build
 // --prof, scripts/actor_prof.py); the counters land behind the error flag: [warp][8] long long at error_flag + 32 ints
@@ -92,7 +90,7 @@ __device__ __forceinline__ void named_bar_sync(int id, int count) {
 #define PROF_ADD(slot, v) prof_c[slot] += (v)
 #define PROF_NOW() clock64()
 // time line of item 1 of CTA 0 (raw SM clock, 32 bits): words [w][48 visits][4] per generator warp, then the issuer's
-// [91 chunks][4] at word 4096 and the epilogue warps' [8][7][2] at word 4608, all behind error_flag + 2048 ints
+// [91 chunks][4] at word 4096 and the epilogue warps' [4][7][2] at word 4608, all behind error_flag + 2048 ints
 #define PROF_TRACE(word, value_expr) do { if (blockIdx.x == 0 && lane == 0 && P.error_flag) \
     reinterpret_cast<uint32_t*>(P.error_flag + 2048)[word] = (uint32_t)(value_expr); } while (0)
 #define PROF_FLUSH() do { if (blockIdx.x == 0 && lane == 0 && P.error_flag) { prof_c[7] = clock64() - prof_start; \
@@ -108,16 +106,14 @@ __device__ __forceinline__ void named_bar_sync(int id, int count) {
 
 // NREAL: nodes of a real graph when the tensors are padded to NODES rows per environment (12 in 16: the train/code shapes),
 // else NODES -- a compile-time constant, so that the production instantiations keep their shifts in the pooled scramble
-template <int NODES, int NCTA, int NPH, int NEPIW, int NREAL = NODES>
-__global__ void __launch_bounds__(pipe_threads<NPH, NEPIW>(), 1)
+template <int NODES, int NREAL = NODES>
+__global__ void __launch_bounds__(PTHREADS, 1)
 actor_pipe_kernel(const __grid_constant__ Params P) {
-  constexpr int NGENW = 4 * NPH, W_ISSUER = NGENW + NEPIW, W_PRODUCER = W_ISSUER + 1, PTHREADS = pipe_threads<NPH, NEPIW>();
+  constexpr int NGENW = 4 * NPH, W_ISSUER = NGENW + NEPIW, W_PRODUCER = W_ISSUER + 1;
   constexpr int ENVS = TCM / NODES;
   constexpr int KB = NODES / 16;                             // 16-node column blocks of an environment's adjacency matrix
-  constexpr int WST = Cfg<NCTA>::WST, STAGE_BYTES = Cfg<NCTA>::STAGE_BYTES, B_LBO = Cfg<NCTA>::B_LBO;
-  static_assert(pipe_smem_bytes<NODES, NCTA>() <= 232448, "shared memory budget");
+  static_assert(pipe_smem_bytes<NODES>() <= 232448, "shared memory budget");
   static_assert(NODES == 16 || NODES == 32, "a generator warp's 32 rows are two 16-node environments or one of 32");
-  static_assert(NEPIW == 4 || NEPIW == 8, "one or two epilogue warps per 32-row group");
   static_assert(KCH == 16 && NCH * KCH >= KH + 1, "16-wide chunks; the tail chunk holds the bias column");
   extern __shared__ __align__(128) unsigned char smem[];
   float* H = reinterpret_cast<float*>(smem + WST * STAGE_BYTES);             // [128][LDH]
@@ -127,11 +123,11 @@ actor_pipe_kernel(const __grid_constant__ Params P) {
   float* AnT = Xr2 + 2 * TCM * 13;                                           // [N(j)][N(n)] shared A_n, transposed (heads)
   uint32_t* AnF = reinterpret_cast<uint32_t*>(AnT + NODES * NODES);         // [KB * KB blocks][hi | lo][32 lanes][4] mma A fragments of the shared A_n
   float* Wh = AnT + 2 * NODES * NODES;                                           // [2][201][4] head kernels, row 200 = bias
-  float* Us = Wh + 2 * 201 * 4;                                              // [2 heads][2 column halves][128][4] head pre-activations
-  uint64_t* bars = reinterpret_cast<uint64_t*>(Us + 4 * TCM * 4);
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 5 * MAXST + 8);
-  // h_prog[row group][epilogue warp of the group]: 32 * item + 8-column blocks of GEMM 4 (the last term of the five-way sum
-  // H) this warp has stored; the generators of layer 3 start on a column chunk as soon as their rows of it are there
+  float* Us = Wh + 2 * 201 * 4;                                              // [2 heads][128][4] head pre-activations
+  uint64_t* bars = reinterpret_cast<uint64_t*>(Us + 2 * TCM * 4);
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 4 * MAXST + 8);
+  // h_prog[row group]: 32 * item + 8-column blocks of GEMM 4 (the last term of the five-way sum H) the group's epilogue
+  // warp has stored; the generators of layer 3 start on a column chunk as soon as their rows of it are there
   volatile int* h_prog = reinterpret_cast<volatile int*>(tmem_slot + 2);
   constexpr int NCB = KH / 8;                                // 25 blocks of 8 accumulator columns
 
@@ -154,41 +150,32 @@ actor_pipe_kernel(const __grid_constant__ Params P) {
     }
   };
   const int M = P.M;
-  // W ring (s < WST):  w_full  this CTA's W half landed (TMA tx)       w_peer  the peer's half landed (leader's copy)
-  //                    w_empty stage consumed (tcgen05.commit, multicast to the pair)
-  // A ring (s < PAST): a_full  A stage written (leader's copy; one arrive per generator warp of the chunk, 4 per CTA)
+  // W ring (s < WST):  w_full  W chunk landed (TMA tx)    w_empty stage consumed (tcgen05.commit)
+  // A ring (s < PAST): a_full  A stage written (one arrive per generator warp of the chunk, 4)
   //                    a_empty stage consumed (commit)
-  // acc_full[b] accumulator b complete (commit)   acc_empty[b] drained by the epilogue warps (leader's copy)
+  // acc_full[b] accumulator b complete (commit)   acc_empty[b] drained by the epilogue warps
   static_assert(WST <= MAXST && PAST <= MAXST, "barrier slots");
-  const uint32_t w_full = smem_u32(&bars[0]), w_peer = smem_u32(&bars[MAXST]), w_empty = smem_u32(&bars[2 * MAXST]);
-  const uint32_t a_full = smem_u32(&bars[3 * MAXST]), a_empty = smem_u32(&bars[4 * MAXST]);
-  const uint32_t acc_full = smem_u32(&bars[5 * MAXST]), acc_empty = smem_u32(&bars[5 * MAXST + 2]);
-  const uint32_t x_full = smem_u32(&bars[5 * MAXST + 6]);      // [2] the item's x_n / pooled rows have landed (cp.async arrivals of all generator threads)
-  const uint32_t cta_rank = (NCTA == 1) ? 0u : cluster_ctarank();
-  const bool is_leader = (cta_rank == 0);
+  const uint32_t w_full = smem_u32(&bars[0]), w_empty = smem_u32(&bars[MAXST]);
+  const uint32_t a_full = smem_u32(&bars[2 * MAXST]), a_empty = smem_u32(&bars[3 * MAXST]);
+  const uint32_t acc_full = smem_u32(&bars[4 * MAXST]), acc_empty = smem_u32(&bars[4 * MAXST + 2]);
+  const uint32_t x_full = smem_u32(&bars[4 * MAXST + 6]);      // [2] the item's x_n / pooled rows have landed (cp.async arrivals of all generator threads)
 
   if (warp == 0) {
-    if constexpr (NCTA == 1) {
-      asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "n"(512) : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    } else {
-      asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "n"(512) : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-    }
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "n"(512) : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
   }
   if (tid == 32) {
     for (int s = 0; s < WST; ++s) {
       mbar_init(w_full + 8 * s, 1);
-      mbar_init(w_peer + 8 * s, 1);
       mbar_init(w_empty + 8 * s, 1);
     }
     for (int s = 0; s < PAST; ++s) {
-      mbar_init(a_full + 8 * s, 4 * NCTA);                  // the four row-group warps of the chunk's phase
+      mbar_init(a_full + 8 * s, 4);                         // the four row-group warps of the chunk's phase
       mbar_init(a_empty + 8 * s, 1);
     }
     for (int b = 0; b < 2; ++b) {
       mbar_init(acc_full + 8 * b, 1);
-      mbar_init(acc_empty + 8 * b, NEPIW * NCTA);
+      mbar_init(acc_empty + 8 * b, NEPIW);
     }
     mbar_init(x_full, NGENW * 32);
     mbar_init(x_full + 8, NGENW * 32);
@@ -196,7 +183,7 @@ actor_pipe_kernel(const __grid_constant__ Params P) {
   }
   // item-independent constants: A_n (both orientations), the head kernels and the layer-1 fragment image; the
   // generators stage the per-item data
-  if (tid < 8) h_prog[tid] = 0;
+  if (tid < 4) h_prog[tid] = 0;
   for (int idx = tid; idx < NODES * NODES; idx += PTHREADS) AnT[(idx % NODES) * NODES + idx / NODES] = P.A_n[idx];
   for (int idx = tid; idx < KB * KB * 32; idx += PTHREADS) {
     // fp16 hi/lo A fragments of the 16 x 16 blocks of A_n (block (mt, kb): rows 16 mt.., columns 16 kb..), computed once
@@ -224,7 +211,6 @@ actor_pipe_kernel(const __grid_constant__ Params P) {
     reinterpret_cast<uint4*>(W1f)[idx] = __ldg(reinterpret_cast<const uint4*>(P.w1frag) + idx);
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
   __syncthreads();
-  if constexpr (NCTA == 2) cluster_sync_all();
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
   const uint32_t tmem_base = *tmem_slot;
   bool ok = true;
@@ -304,10 +290,7 @@ actor_pipe_kernel(const __grid_constant__ Params P) {
           if ((int)(u % NPH) != ph) continue;
           if (u >= PAST) PROF_WAIT(3, ok = mbar_wait(a_empty + 8 * sa, ((u / PAST) - 1) & 1) && ok);
           __syncwarp();
-          if (lane == 0) {
-            if (is_leader) mbar_arrive(a_full + 8 * sa);
-            else mbar_arrive_remote(a_full + 8 * sa, 0);
-          }
+          if (lane == 0) mbar_arrive(a_full + 8 * sa);
         }
         continue;
       }
@@ -403,10 +386,7 @@ actor_pipe_kernel(const __grid_constant__ Params P) {
         PROF_WAIT(4, asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"));
         asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
         __syncwarp();
-        if (lane == 0) {
-          if (is_leader) mbar_arrive(a_full + 8 * pending);
-          else mbar_arrive_remote(a_full + 8 * pending, 0);
-        }
+        if (lane == 0) mbar_arrive(a_full + 8 * pending);
         pending = -1;
       };
       uint32_t afr[2][KB][2][4];                               // [mt][kb][hi | lo][a0..a3] of the GEMM's adjacency matrix
@@ -434,15 +414,14 @@ actor_pipe_kernel(const __grid_constant__ Params P) {
           const long long prof_t1 = PROF_NOW();
           const int prof_v = (g * NCH + c) / NPH;
           if (it == 1) PROF_TRACE((warp * 48 + prof_v) * 4 + 0, prof_t1);
-          // the five-way sum H is handed over row group by row group, 16 columns at a time: the two epilogue warps of this
-          // warp's rows publish how many of their 8-column blocks of GEMM 4 are stored (h_prog), so layer 3 starts on
+          // the five-way sum H is handed over row group by row group, 16 columns at a time: the epilogue warp of this
+          // warp's rows publishes how many of its 8-column blocks of GEMM 4 are stored (h_prog), so layer 3 starts on
           // column chunk c as soon as blocks 2c, 2c + 1 are there instead of after the whole drain
           if (g == 5) {
-            const int want0 = it * 32 + (NEPIW == 8 ? min(c + 1, (NCB + 1) / 2) : min(2 * c + 2, NCB));
-            const int want1 = it * 32 + (NEPIW == 8 ? min(c + 1, NCB / 2) : min(2 * c + 2, NCB));
+            const int want = it * 32 + min(2 * c + 2, NCB);
             const long long t0_ = PROF_NOW();
             uint32_t spin = 0;
-            while ((h_prog[q * 2] < want0 || h_prog[q * 2 + 1] < want1) && ++spin < SPIN_LIMIT) { }
+            while (h_prog[q] < want && ++spin < SPIN_LIMIT) { }
             ok = ok && spin < SPIN_LIMIT;
             __threadfence_block();
             PROF_ADD(1, PROF_NOW() - t0_);
@@ -540,15 +519,10 @@ actor_pipe_kernel(const __grid_constant__ Params P) {
     if (bad && P.error_flag) atomicOr(P.error_flag, 2);        // an input left the fp16 range (or NaN)
   } else if (warp < NGENW + NEPIW) {
     // =================================================== epilogue =============================================
-    const int ew = warp - NGENW, q = ew & 3, half = ew >> 2;
+    const int q = warp & 3;                                    // row group
     const int r = 32 * q + lane;
     const int n = r % NODES;
     const int lane_env0 = lane & ~(NODES - 1);
-    // the 25 blocks of 8 accumulator columns: with two warps per row group, warp `half` takes blocks half, half + 2, ... so
-    // that both advance through the columns together (the generators of layer 3 follow them chunk by chunk, see h_prog)
-    constexpr int CBS = (NEPIW == 8) ? 2 : 1;                  // block stride
-    const int cb0 = (NEPIW == 8) ? half : 0;
-    const int ncb = (NEPIW == 8) ? (half ? NCB / 2 : (NCB + 1) / 2) : NCB;
     float nonfinite = 0.f;                                     // stays 0 while every accumulator entry is finite (x * 0 is NaN otherwise)
     for (int item = blockIdx.x, it = 0; item < P.n_items; item += gridDim.x, ++it) {
       int row0, rows_here;
@@ -561,29 +535,26 @@ actor_pipe_kernel(const __grid_constant__ Params P) {
         PROF_WAIT(0, ok = mbar_wait(acc_full + 8 * b, (uint32_t)((G >> 1) & 1)) && ok);
         if (!live) {
           __syncwarp();
-          if (lane == 0) {
-            if (is_leader) mbar_arrive(acc_empty + 8 * b);
-            else mbar_arrive_remote(acc_empty + 8 * b, 0);
-          }
+          if (lane == 0) mbar_arrive(acc_empty + 8 * b);
           continue;
         }
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
         const long long prof_t1 = PROF_NOW();
-        if (it == 1) PROF_TRACE(4608 + (ew * 7 + g) * 2, prof_t1);
-        const uint32_t tacc = tmem_base + ((uint32_t)(32 * q) << 16) + (uint32_t)(b ? TM_ACC1 : 0) + (uint32_t)(8 * cb0);
+        if (it == 1) PROF_TRACE(4608 + (q * 7 + g) * 2, prof_t1);
+        const uint32_t tacc = tmem_base + ((uint32_t)(32 * q) << 16) + (uint32_t)(b ? TM_ACC1 : 0);
         const float wsi = __ldg(P.wscale_inv + g);             // undoes the power-of-two scale folded into W (exact)
-        float* hrow = H + r * LDH + 8 * cb0;
+        float* hrow = H + r * LDH;
         const float* wh = Wh + (g >= 5 ? g - 5 : 0) * 201 * 4; // only used for g >= 5
         float u0 = 0.f, u1 = 0.f, u2 = 0.f;
         uint32_t vr[2][8];
         tmem_ld8_async(tacc, vr[0]);
 #pragma unroll 2
-        for (int i = 0; i < ncb; ++i) {
+        for (int i = 0; i < NCB; ++i) {
           asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
           float v[8];
 #pragma unroll
           for (int t = 0; t < 8; ++t) v[t] = __uint_as_float(vr[i & 1][t]);
-          if (i + 1 < ncb) tmem_ld8_async(tacc + (uint32_t)(8 * CBS * (i + 1)), vr[(i + 1) & 1]);   // in flight while block i is processed
+          if (i + 1 < NCB) tmem_ld8_async(tacc + (uint32_t)(8 * (i + 1)), vr[(i + 1) & 1]);   // in flight while block i is processed
           // an operand that left the fp16 range (|A.X| > 65504 became inf in the split) or a NaN shows up as a non-finite
           // accumulator entry here, before the ReLU can hide it: one FFMA per entry instead of range tracking in the generators
 #pragma unroll
@@ -593,7 +564,7 @@ actor_pipe_kernel(const __grid_constant__ Params P) {
           if (g <= 4) {
 #pragma unroll
             for (int t = 0; t < 8; ++t) v[t] = fmaxf(v[t], 0.f);
-            float4* dst = reinterpret_cast<float4*>(hrow + 8 * CBS * i);
+            float4* dst = reinterpret_cast<float4*>(hrow + 8 * i);
             float4 o0 = make_float4(0.f, 0.f, 0.f, 0.f), o1 = o0;
             if (g > 0) { o0 = dst[0]; o1 = dst[1]; }
             dst[0] = make_float4(fmaf(v[0], wsi, o0.x), fmaf(v[1], wsi, o0.y), fmaf(v[2], wsi, o0.z), fmaf(v[3], wsi, o0.w));
@@ -601,17 +572,14 @@ actor_pipe_kernel(const __grid_constant__ Params P) {
             if (g == 4) {                                      // H is complete in these 8 columns of this warp's rows
               __threadfence_block();
               __syncwarp();
-              if (lane == 0) {
-                h_prog[q * 2 + half] = it * 32 + i + 1;
-                if (NEPIW == 4) h_prog[q * 2 + 1] = it * 32 + i + 1;
-              }
+              if (lane == 0) h_prog[q] = it * 32 + i + 1;
             }
           } else {
 #pragma unroll
             for (int t = 0; t < 8; ++t) v[t] = fmaxf(v[t] * wsi, 0.f);
 #pragma unroll
             for (int t = 0; t < 8; ++t) {
-              const float4 w = *reinterpret_cast<const float4*>(wh + (8 * (cb0 + CBS * i) + t) * 4);
+              const float4 w = *reinterpret_cast<const float4*>(wh + (8 * i + t) * 4);
               u0 = fmaf(v[t], w.x, u0); u1 = fmaf(v[t], w.y, u1); u2 = fmaf(v[t], w.z, u2);
             }
           }
@@ -619,23 +587,14 @@ actor_pipe_kernel(const __grid_constant__ Params P) {
         asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
         __syncwarp();
         PROF_ADD(1, PROF_NOW() - prof_t1);
-        if (it == 1) PROF_TRACE(4608 + (ew * 7 + g) * 2 + 1, PROF_NOW());
-        if (lane == 0) {
-          if (is_leader) mbar_arrive(acc_empty + 8 * b);
-          else mbar_arrive_remote(acc_empty + 8 * b, 0);
-        }
+        if (it == 1) PROF_TRACE(4608 + (q * 7 + g) * 2 + 1, PROF_NOW());
+        if (lane == 0) mbar_arrive(acc_empty + 8 * b);
         if (g >= 5) {
           // output heads (truss2D_RL.py:121-125): sigmoid(A_n (x3 W4) + b4); the 16/32 rows of an environment are
-          // lanes of this warp.  With two warps per row group the column halves meet in shared memory first.
+          // lanes of this warp, whose x3 W4 rows meet in shared memory
           const int hd = g - 5, nout = 2 + hd;
-          float* us = Us + hd * 2 * TCM * 4;                   // [column half][128][4]
-          *reinterpret_cast<float4*>(us + (half * TCM + r) * 4) = make_float4(u0, u1, u2, 0.f);
-          if (NEPIW == 8) {
-            named_bar_sync(1 + q, 64);
-            if (half) continue;                                // the first warp of the pair finishes the head
-            const float4 o = *reinterpret_cast<const float4*>(us + (TCM + r) * 4);
-            *reinterpret_cast<float4*>(us + r * 4) = make_float4(u0 + o.x, u1 + o.y, u2 + o.z, 0.f);
-          }
+          float* us = Us + hd * TCM * 4;                       // [128][4]
+          *reinterpret_cast<float4*>(us + r * 4) = make_float4(u0, u1, u2, 0.f);
           __syncwarp();
           float o[3] = {wh[KH * 4 + 0], wh[KH * 4 + 1], wh[KH * 4 + 2]};
           for (int j = 0; j < NODES; ++j) {
@@ -662,60 +621,49 @@ actor_pipe_kernel(const __grid_constant__ Params P) {
     }  // items
     if (!(nonfinite == 0.f) && P.error_flag) atomicOr(P.error_flag, 2);   // an activation left the fp16 range (or NaN)
   } else if (warp == W_ISSUER) {
-    // =================================================== MMA issuer / W forwarder =============================
+    // =================================================== MMA issuer ===========================================
     // The whole warp walks the chunk sequence converged (all lanes poll the barriers); ONE elected lane issues the three
     // MMAs and the commits of a chunk.  Stage indices and barrier parities are running counters (no division), and the
     // shared-memory descriptor of a W stage is the stage-0 descriptor plus a constant (its address field counts 16-byte
     // units), so a chunk costs the issuer a few dozen instructions: it is the one serial thread every chunk passes through
     // (the first form -- one lane inside `if (lane == 0)`, u % WST / u % PAST, a switch over per-stage descriptors -- made
     // ptxas wrap every tcgen05 instruction in an elect / branch sequence: ~140 instructions and ~760 cycles per chunk).
-    if (is_leader) {
-      const uint64_t d_hi0 = make_desc(smem_u32(smem), B_LBO);
-      constexpr uint64_t D_STAGE = (uint64_t)(STAGE_BYTES >> 4), D_LO = (uint64_t)((NKB * B_LBO) >> 4);
-      static_assert((WST * STAGE_BYTES >> 4) < 0x4000, "the W ring must stay inside the descriptor's 14-bit address field");
-      uint32_t sw = 0, pw = 0, sa = 0, pa = 0, G = 0;
-      for (int item = blockIdx.x; item < P.n_items; item += gridDim.x) {
-        const bool prof_tr = (G == (uint32_t)NGEMM);          // item 1 of this CTA
-        for (int g = 0; g < NGEMM; ++g, ++G) {
-          const uint32_t b = G & 1u;
-          const uint32_t dacc = tmem_base + (b ? (uint32_t)TM_ACC1 : 0u);
-          if (G >= 2) {                                        // the epilogue of GEMM G-2 has drained this accumulator
-            PROF_WAIT(2, ok = mbar_wait_cluster(acc_empty + 8 * b, ((G >> 1) - 1u) & 1u) && ok);
-          }
+    const uint64_t d_hi0 = make_desc(smem_u32(smem), B_LBO);
+    constexpr uint64_t D_STAGE = (uint64_t)(STAGE_BYTES >> 4), D_LO = (uint64_t)((NKB * B_LBO) >> 4);
+    static_assert((WST * STAGE_BYTES >> 4) < 0x4000, "the W ring must stay inside the descriptor's 14-bit address field");
+    uint32_t sw = 0, pw = 0, sa = 0, pa = 0, G = 0;
+    for (int item = blockIdx.x; item < P.n_items; item += gridDim.x) {
+      const bool prof_tr = (G == (uint32_t)NGEMM);            // item 1 of this CTA
+      for (int g = 0; g < NGEMM; ++g, ++G) {
+        const uint32_t b = G & 1u;
+        const uint32_t dacc = tmem_base + (b ? (uint32_t)TM_ACC1 : 0u);
+        if (G >= 2) {                                          // the epilogue of GEMM G-2 has drained this accumulator
+          PROF_WAIT(2, ok = mbar_wait_cluster(acc_empty + 8 * b, ((G >> 1) - 1u) & 1u) && ok);
+        }
 #pragma unroll 1
-          for (int c = 0; c < NCH; ++c) {
-            if constexpr (NCTA == 2) ok = mbar_wait_cluster(a_full + 8 * sa, pa) && ok;
-            else PROF_WAIT(0, ok = mbar_wait(a_full + 8 * sa, pa) && ok);
-            if (prof_tr) PROF_TRACE(4096 + (g * NCH + c) * 4 + 0, PROF_NOW());
-            PROF_WAIT(1, ok = mbar_wait(w_full + 8 * sw, pw) && ok);
-            if (prof_tr) PROF_TRACE(4096 + (g * NCH + c) * 4 + 1, PROF_NOW());
-            if constexpr (NCTA == 2) ok = mbar_wait_cluster(w_peer + 8 * sw, pw) && ok;
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-            if (elect_one()) {
-              const uint32_t a_hi = tmem_base + (uint32_t)TM_AHI + (uint32_t)ACOLS * sa, a_lo = tmem_base + (uint32_t)TM_ALO + (uint32_t)ACOLS * sa;
-              const uint64_t d_hi = d_hi0 + D_STAGE * sw, d_lo = d_hi + D_LO;
-              mma_split<NCTA>(dacc, a_hi, d_hi, c != 0);       // Yhi.Whi + Yhi.Wlo + Ylo.Whi (the tail chunk is zero-padded)
-              mma_split<NCTA>(dacc, a_hi, d_lo, 1);
-              mma_split<NCTA>(dacc, a_lo, d_hi, 1);
-              mma_commit<NCTA>(w_empty + 8 * sw);
-              mma_commit<NCTA>(a_empty + 8 * sa);
-              if (c + 1 == NCH) mma_commit<NCTA>(acc_full + 8 * b);
-            }
-            __syncwarp();
-            if (prof_tr) PROF_TRACE(4096 + (g * NCH + c) * 4 + 2, PROF_NOW());
-            if (++sw == (uint32_t)WST) { sw = 0; pw ^= 1u; }
-            if (++sa == (uint32_t)PAST) { sa = 0; pa ^= 1u; }
+        for (int c = 0; c < NCH; ++c) {
+          PROF_WAIT(0, ok = mbar_wait(a_full + 8 * sa, pa) && ok);
+          if (prof_tr) PROF_TRACE(4096 + (g * NCH + c) * 4 + 0, PROF_NOW());
+          PROF_WAIT(1, ok = mbar_wait(w_full + 8 * sw, pw) && ok);
+          if (prof_tr) PROF_TRACE(4096 + (g * NCH + c) * 4 + 1, PROF_NOW());
+          asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+          if (elect_one()) {
+            const uint32_t a_hi = tmem_base + (uint32_t)TM_AHI + (uint32_t)ACOLS * sa, a_lo = tmem_base + (uint32_t)TM_ALO + (uint32_t)ACOLS * sa;
+            const uint64_t d_hi = d_hi0 + D_STAGE * sw, d_lo = d_hi + D_LO;
+            mma_split(dacc, a_hi, d_hi, c != 0);               // Yhi.Whi + Yhi.Wlo + Ylo.Whi (the tail chunk is zero-padded)
+            mma_split(dacc, a_hi, d_lo, 1);
+            mma_split(dacc, a_lo, d_hi, 1);
+            mma_commit(w_empty + 8 * sw);
+            mma_commit(a_empty + 8 * sa);
+            if (c + 1 == NCH) mma_commit(acc_full + 8 * b);
           }
+          __syncwarp();
+          if (prof_tr) PROF_TRACE(4096 + (g * NCH + c) * 4 + 2, PROF_NOW());
+          if (++sw == (uint32_t)WST) { sw = 0; pw ^= 1u; }
+          if (++sa == (uint32_t)PAST) { sa = 0; pa ^= 1u; }
         }
-      }  // items
-    } else if (lane == 0) {
-      for (int item = blockIdx.x, it = 0; item < P.n_items; item += gridDim.x, ++it)
-        for (int uu = 0; uu < NGEMM * NCH; ++uu) {             // peer CTA: tell the leader that W chunk u has landed here
-          const uint32_t u = (uint32_t)it * (uint32_t)(NGEMM * NCH) + (uint32_t)uu, sw = u % WST;
-          ok = mbar_wait(w_full + 8 * sw, (u / WST) & 1) && ok;
-          mbar_arrive_remote(w_peer + 8 * sw, 0);
-        }
-    }
+      }
+    }  // items
     __syncwarp();
   } else {
     // =================================================== W producer ===========================================
@@ -725,9 +673,8 @@ actor_pipe_kernel(const __grid_constant__ Params P) {
           for (int c = 0; c < NCH; ++c) {
             const uint32_t u = (uint32_t)it * (uint32_t)(NGEMM * NCH) + (uint32_t)(g * NCH + c), s = u % WST;
             if (u >= WST) PROF_WAIT(0, ok = mbar_wait(w_empty + 8 * s, ((u / WST) - 1) & 1) && ok);       // chunk u-WST consumed
-            const uint32_t bytes = (uint32_t)STAGE_BYTES;                                    // this CTA's half: hi then lo
-            const unsigned char* src = reinterpret_cast<const unsigned char*>(P.wimg[g]) +
-                                       (size_t)c * Cfg<NCTA>::CHUNK_IMG_BYTES + (size_t)cta_rank * bytes;
+            const uint32_t bytes = (uint32_t)STAGE_BYTES;                                    // hi then lo
+            const unsigned char* src = reinterpret_cast<const unsigned char*>(P.wimg[g]) + (size_t)c * bytes;
             mbar_expect_tx(w_full + 8 * s, bytes);
             bulk_g2s(smem_u32(smem + s * STAGE_BYTES), src, bytes, w_full + 8 * s);
           }
@@ -739,13 +686,7 @@ actor_pipe_kernel(const __grid_constant__ Params P) {
   if (!ok && P.error_flag) atomicOr(P.error_flag, 1);
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
   __syncthreads();
-  if constexpr (NCTA == 2) cluster_sync_all();               // neither CTA leaves while the pair's TMEM / barriers are in use
-  if (warp == 0) {
-    if constexpr (NCTA == 1)
-      asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(512) : "memory");
-    else
-      asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(512) : "memory");
-  }
+  if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(512) : "memory");
 }
 
 }  // namespace pipe

@@ -22,34 +22,22 @@ namespace tc {
 // the operand bytes and twice the tensor rate (3xTF32 on kind::tf32 was the first formulation of this kernel: 0.388 ms
 // against 0.382 ms per forward with everything else equal).  What fp16 lacks is range: W is pre-scaled by a power of
 // two per layer (undone exactly in the epilogue) and |A.X| > 65504 is reported through tactor_status.
-constexpr bool F16 = true;
 constexpr int TCM = 128;             // rows per CTA
 constexpr int TCN = 208;             // padded output columns (UMMA N, multiple of 16)
-constexpr int KCH = 16;              // K elements per chunk (f16: one MMA k-step of 16; tf32: two of 8)
-constexpr int KPC = F16 ? 8 : 4;     // K elements per 16-byte core-matrix row
+constexpr int KCH = 16;              // K elements per chunk (one MMA k-step)
+constexpr int KPC = 8;               // K elements per 16-byte core-matrix row
 constexpr int NKB = KCH / KPC;       // 16-byte core-matrix columns per chunk
 constexpr int SBO = 128;             // bytes between 8-row groups
+constexpr int B_LBO = TCN * 16;      // bytes between core matrices adjacent in K (B operand)
+constexpr int B_BYTES = NKB * B_LBO; // one of {hi, lo} of a chunk
+constexpr int WST = 3;               // W stages in shared memory (K chunks in flight)
+constexpr int STAGE_BYTES = 2 * B_BYTES;   // Bhi, Blo of one K chunk
+// fp32 accumulate, A and B K-major and f16, M = 128, N = 208
+constexpr uint32_t IDESC = (1u << 4) | ((uint32_t)(TCN >> 3) << 17) | ((uint32_t)(TCM >> 4) << 24);
 constexpr float F16_MAX = 65504.f;
 constexpr uint32_t SPIN_LIMIT = 1u << 24;
-
-// NCTA = 1: one CTA per 128-row tile.  NCTA = 2: a CTA pair (cluster of 2, tcgen05 cta_group::2) works on two
-// tiles with ONE M = 256 instruction stream: each CTA generates the A operand of its own 128 rows and holds only
-// its half of the W columns, so the weight stream out of L2 and the tensor core's B reads per SM are halved.
-template <int NCTA> struct Cfg {
-  static constexpr int BN = TCN / NCTA;                     // W columns held by one CTA
-  static constexpr int B_LBO = BN * 16;                     // bytes between core matrices adjacent in K (B operand)
-  static constexpr int B_BYTES = NKB * B_LBO;               // one of {hi, lo} of a full chunk
-  static constexpr int WST = 3;                             // W stages in shared memory (K chunks in flight)
-  static constexpr int STAGE_BYTES = 2 * B_BYTES;           // Bhi, Blo of one K chunk
-  static constexpr int CHUNK_IMG_BYTES = NCTA * 2 * B_BYTES;      // one full chunk of the W image (all CTAs)
-  // fp32 accumulate, A and B K-major, M = 128 * NCTA, N = 208; operand format 0 = f16, 2 = tf32
-  static constexpr uint32_t FMT = F16 ? 0u : 2u;
-  static constexpr uint32_t IDESC =
-      (1u << 4) | (FMT << 7) | (FMT << 10) | ((uint32_t)(TCN >> 3) << 17) | ((uint32_t)((TCM * NCTA) >> 4) << 24);
-};
-// W operand image in global memory: per chunk, per CTA of the pair, [hi: kb][n (BN)][16 bytes = KPC elements] then [lo: ...];
-// f16: every chunk is a full K = 16 step (rows k >= 200 are zero); tf32: the tail chunk holds 8 rows
-__host__ __device__ constexpr int chunk_kw(int K, int c) { return (K - c * KCH) < KCH ? (K - c * KCH) : KCH; }
+// W operand image in global memory: per chunk [hi: kb][n][16 bytes = KPC elements] then [lo: ...], STAGE_BYTES in all;
+// every chunk is a full K = 16 step (the rows past the bias row k = 200 are zero)
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
@@ -57,23 +45,14 @@ __device__ __forceinline__ uint64_t make_desc(uint32_t saddr, uint32_t lbo_bytes
   return (uint64_t)((saddr >> 4) & 0x3FFFu) | ((uint64_t)((lbo_bytes >> 4) & 0x3FFFu) << 16) |
          ((uint64_t)((SBO >> 4) & 0x3FFFu) << 32) | (1ull << 46);        // version 1 (Blackwell), no swizzle
 }
-// D[tmem] (+)= A[tmem] . B[smem]: A is [128 lanes = rows][8 columns] of tensor memory (of each CTA of a pair): one k
-// per column for tf32 (K = 8), two packed fp16 per column, even k in the low half, for f16 (K = 16)
-#define TACTOR_MMA_KIND "kind::f16"
-template <int NCTA>
+// D[tmem] (+)= A[tmem] . B[smem]: A is [128 lanes = rows][8 columns] of tensor memory, two packed fp16 per column, even k
+// in the low half (K = 16)
 __device__ __forceinline__ void mma_split(uint32_t d_tmem, uint32_t a_tmem, uint64_t b_desc, uint32_t accumulate) {
-  if constexpr (NCTA == 1)
-    asm volatile(
-        "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1." TACTOR_MMA_KIND " [%0], [%1], %2, %3, p;\n\t}\n" ::"r"(d_tmem),
-        "r"(a_tmem), "l"(b_desc), "r"(Cfg<1>::IDESC), "r"(accumulate)
-        : "memory");
-  else
-    asm volatile(
-        "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::2." TACTOR_MMA_KIND " [%0], [%1], %2, %3, p;\n\t}\n" ::"r"(d_tmem),
-        "r"(a_tmem), "l"(b_desc), "r"(Cfg<2>::IDESC), "r"(accumulate)
-        : "memory");
+  asm volatile(
+      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}\n" ::"r"(d_tmem),
+      "r"(a_tmem), "l"(b_desc), "r"(IDESC), "r"(accumulate)
+      : "memory");
 }
 __device__ __forceinline__ void tmem_st8(uint32_t taddr, const float* v) {
   asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"r"(taddr),
@@ -81,15 +60,9 @@ __device__ __forceinline__ void tmem_st8(uint32_t taddr, const float* v) {
                "r"(__float_as_uint(v[4])), "r"(__float_as_uint(v[5])), "r"(__float_as_uint(v[6])), "r"(__float_as_uint(v[7]))
                : "memory");
 }
-// all MMAs issued so far by this thread have completed -> one arrival on the barrier (of every CTA of the pair)
-template <int NCTA>
+// all MMAs issued so far by this thread have completed -> one arrival on the barrier
 __device__ __forceinline__ void mma_commit(uint32_t bar) {
-  if constexpr (NCTA == 1)
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-  else
-    asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
-                 "h"((uint16_t)3)
-                 : "memory");
+  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
 }
 // one lane of the (converged) warp
 __device__ __forceinline__ bool elect_one() {
@@ -131,7 +104,7 @@ __device__ __forceinline__ bool mbar_wait_relaxed(uint32_t bar, uint32_t parity,
   }
   return false;
 }
-// the same for a barrier that peer-CTA threads arrive on
+// the same with acquire semantics at cluster scope
 __device__ __forceinline__ bool mbar_wait_cluster(uint32_t bar, uint32_t parity) {
   for (uint32_t spin = 0; spin < SPIN_LIMIT; ++spin) {
     uint32_t done;
@@ -146,20 +119,6 @@ __device__ __forceinline__ bool mbar_wait_cluster(uint32_t bar, uint32_t parity)
 }
 __device__ __forceinline__ void mbar_arrive(uint32_t bar) {
   asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-// arrive on the barrier at the same shared-memory offset in CTA `cta` of the cluster
-__device__ __forceinline__ void mbar_arrive_remote(uint32_t bar, uint32_t cta) {
-  uint32_t ra;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(ra) : "r"(bar), "r"(cta));
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(ra) : "memory");
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
 }
 __device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
   asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst),
@@ -182,11 +141,6 @@ __device__ __forceinline__ void tmem_ld8(uint32_t taddr, float* v) {
 //   B [16 x 8]  col-major: b0 (k 2t..2t+1, col g)  b1 (k 2t+8.., col g)
 //   C [16 x 8]           : c0 c1 (row g, cols 2t, 2t+1)  c2 c3 (row g+8, same cols)
 __device__ __forceinline__ void hmma16816(float* c, const uint32_t* a, uint32_t b0, uint32_t b1) {
-#ifdef TACTOR_ABLATE_HMMA   // timing experiment only (wrong results): the generators without their warp-level tensor-core products;
-  // the empty asm keeps the accumulators opaque to the optimiser and emits nothing
-  asm volatile("" : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3]) : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-  return;
-#endif
   asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.f16.f16.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, {%0, %1, %2, %3};"
                : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
                : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
@@ -260,7 +214,6 @@ struct Params {
   int split_from;         // first work item that is a piece of a tile (tiles of the last partial wave), n_items if none
   int split_f;            // pieces per split tile: 1, 2 or 4
   int* error_flag;
-  int dev_flags;          // development switches (TACTOR_FLAGS, A/B timing): bit 0 = publish an A stage right after its store
 };
 
 }  // namespace fused

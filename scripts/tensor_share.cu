@@ -29,10 +29,10 @@ __global__ void __launch_bounds__(544, 1) share_kernel(long long* out, int nutc,
   long long t1 = t0;
   if (warp == 0) {
     if (nutc > 0) {
-      const uint64_t d = make_desc(smem_u32(smem), Cfg<1>::B_LBO);
+      const uint64_t d = make_desc(smem_u32(smem), B_LBO);
       if (elect_one()) {
-        for (int i = 0; i < nutc; ++i) mma_split<1>(tmem, tmem + 448, d, i != 0);
-        mma_commit<1>(smem_u32(&bar));
+        for (int i = 0; i < nutc; ++i) mma_split(tmem, tmem + 448, d, i != 0);
+        mma_commit(smem_u32(&bar));
       }
       __syncwarp();
       mbar_wait(smem_u32(&bar), 0);
@@ -99,12 +99,12 @@ __global__ void __launch_bounds__(544, 1) burst_kernel(long long* out, int nburs
   const long long t0 = clock64();
   long long count = 0, busy = 0;
   if (warp == 0) {
-    const uint64_t d = make_desc(smem_u32(smem), Cfg<1>::B_LBO);
+    const uint64_t d = make_desc(smem_u32(smem), B_LBO);
     for (int b = 0; b < nburst; ++b) {
       const long long tb = clock64();
       if (elect_one()) {
-        for (int i = 0; i < burst; ++i) mma_split<1>(tmem, tmem + 448, d, 1);
-        mma_commit<1>(smem_u32(&bar));
+        for (int i = 0; i < burst; ++i) mma_split(tmem, tmem + 448, d, 1);
+        mma_commit(smem_u32(&bar));
       }
       __syncwarp();
       mbar_wait(smem_u32(&bar), b & 1);

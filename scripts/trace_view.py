@@ -2,10 +2,10 @@
 import sys
 import numpy as np
 w = np.load(sys.argv[1])
-nph = int(sys.argv[2]) if len(sys.argv) > 2 else 2
+nph = 2                              # generator phases of actor_pipe_kernel
 gen = w[:16 * 48 * 4].reshape(16, 48, 4).astype(np.int64)
 iss = w[4096:4096 + 91 * 4].reshape(91, 4).astype(np.int64)
-epi = w[4608:4608 + 8 * 7 * 2].reshape(8, 7, 2).astype(np.int64)
+epi = w[4608:4608 + 4 * 7 * 2].reshape(4, 7, 2).astype(np.int64)
 t0 = iss[0, 0]
 rows = []
 for ph in range(nph):
@@ -23,5 +23,5 @@ prev = 0
 for uu, wp, s, x, m, st in rows:
     print(uu, uu // 13, uu % 13, "| w", wp, s, x - s, m - x, st - m, "|", iss[uu, 0] - t0, iss[uu, 2] - t0, iss[uu, 2] - t0 - prev, "|", iss[uu, 0] - t0 - st)
     prev = iss[uu, 2] - t0
-for ew in (0, 4):
+for ew in range(4):
     print("epilogue warp", ew, [(int(epi[ew, g, 0] - t0), int(epi[ew, g, 1] - epi[ew, g, 0])) for g in range(7)])

@@ -174,28 +174,6 @@ def test_last_wave_split_is_bit_identical(nodes, B, monkeypatch):
     assert bool(torch.isfinite(outs[0][0]).all()) and 0.0 < float(outs[0][0].min()) and float(outs[0][0].max()) < 1.0
 
 
-@pytest.mark.parametrize("nodes,B", [(16, 64), (32, 40)])
-def test_cta_pair_build_matches_single_cta(nodes, B, monkeypatch):
-    """TACTOR_NCTA=2 selects the CTA-pair instantiation (tcgen05.mma.cta_group::2, W split over two SMs): kept as a
-    measured alternative, it must give the same outputs as the production single-CTA kernel"""
-    from mop_truss_marl_b200 import actor, tf_checkpoint
-    w = tf_checkpoint.random_actor_weights(seed=9)
-    g = torch.Generator(device="cuda").manual_seed(2)
-    r = lambda *s: torch.rand(*s, device="cuda", generator=g)   # noqa: E731
-    sc = 1.0 / nodes
-    inp = (r(B, nodes, 13), r(nodes, nodes) * sc, r(B, nodes, nodes) * sc, r(B, nodes, nodes) * sc, r(B, nodes, nodes) * sc,
-           r(B, 2, 4), r(B, 2, 2) * 0.3)
-    outs = []
-    for ncta in ("1", "2"):
-        monkeypatch.setenv("TACTOR_NCTA", ncta)
-        pol = actor.BatchedActor(w, nodes, B)
-        geo, topo = pol.forward(*inp)
-        torch.cuda.synchronize()
-        pol.check()
-        outs.append((geo.clone(), topo.clone()))
-    assert float((outs[0][0] - outs[1][0]).abs().max()) <= 1e-6 and float((outs[0][1] - outs[1][1]).abs().max()) <= 1e-6
-
-
 def test_fp16_range_overflow_is_reported():
     """the split tensor-core product carries activations as fp16 hi + lo: an activation beyond 65504 cannot be
     represented and must be reported (tactor_status -> TfemError), never silently returned"""
@@ -222,30 +200,6 @@ def test_tmem_store_layout_selftest():
     0 and 16): the layout the kernel assumes is checked on the device itself"""
     from mop_truss_marl_b200 import actor
     actor.selftest_tmem_layout(0)
-
-
-@pytest.mark.parametrize("variant", ["1", "2", "3", "4"])
-def test_generator_variants_match_production(variant, monkeypatch):
-    """TACTOR_VARIANT selects other (generator phases, epilogue warps) builds of the fused kernel, kept for A/B timing;
-    the hidden layers are the same arithmetic in all of them, only the head's 200-term sum is split differently between
-    one and two epilogue warps per row group"""
-    from mop_truss_marl_b200 import actor, tf_checkpoint
-    w = tf_checkpoint.random_actor_weights(seed=11)
-    g = torch.Generator(device="cuda").manual_seed(3)
-    r = lambda *s: torch.rand(*s, device="cuda", generator=g)   # noqa: E731
-    for nodes, B in ((16, 333), (32, 77)):
-        sc = 1.0 / nodes
-        inp = (r(B, nodes, 13), r(nodes, nodes) * sc, r(B, nodes, nodes) * sc, r(B, nodes, nodes) * sc, r(B, nodes, nodes) * sc,
-               r(B, 2, 4), r(B, 2, 2) * 0.3)
-        outs = []
-        for v in ("0", variant):
-            monkeypatch.setenv("TACTOR_VARIANT", v)
-            pol = actor.BatchedActor(w, nodes, B)
-            geo, topo = pol.forward(*inp)
-            torch.cuda.synchronize()
-            pol.check()
-            outs.append((geo.clone(), topo.clone()))
-        assert float((outs[0][0] - outs[1][0]).abs().max()) <= 1e-6 and float((outs[0][1] - outs[1][1]).abs().max()) <= 1e-6
 
 
 def trained_weights(agent):
