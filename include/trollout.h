@@ -19,6 +19,10 @@
  * and with TROLLOUT_ZEROCOPY=0 every array is a cudaMemcpyAsync on a copy engine).  Same bytes over the link, but none of
  * the per-copy cost of the 11 + 13 arrays of a piece, so the batch can be cut finer (trollout_set_pieces).
  * TROLLOUT_HOSTTIME=1 prints the host-side share of the replayed steps (checks, cudaGraphLaunch, wait) at destroy time.
+ *
+ * trollout_create_agents / trollout_step_agents_host run the driver's whole inner step -- up to three agents acting on
+ * the same parent -- in one call: the parent crosses the link once instead of once per agent, and one graph launch
+ * and one pipeline fill serve all agents.
  */
 #ifndef TROLLOUT_H_
 #define TROLLOUT_H_
@@ -66,10 +70,39 @@ typedef struct trollout_io {
   float* a_topo;           /* [B,N,3] */
 } trollout_io;
 
+/* Several agents on one parent (master_DDPG_truss2D_MO.py:249-260: for k = 0, 1, 2 agents[k].act(state) then
+ * _game_modify(...) on that same parent; the training driver's transition holds the parent and the three children,
+ * train/code/truss2D_RL.py:439-456).  One child block per agent; each _game_modify draws its own coin
+ * (truss2D_ENV.py:460). */
+#define TROLLOUT_MAX_AGENTS 3
+
+typedef struct trollout_child {
+  trollout_state out;      /* child state (written); must not alias the parent or another child */
+  const uint8_t* coin;     /* [B] symmetry coin, NULL = all 0 */
+  float* point;            /* [B,4]  */
+  int32_t* status;         /* [B]    */
+  float* a_geo;            /* [B,N,2] this agent's actions as _game_modify left them (clipped) */
+  float* a_topo;           /* [B,N,3] */
+} trollout_child;
+
+typedef struct trollout_agents_io {
+  trollout_state in;       /* parent state (read), uploaded once for all agents; compact columns as in trollout_io */
+  const float* x_p;        /* [B,P,4] Pareto-front graph */
+  const float* A_p;        /* [B,P,P] */
+  const int32_t* n_pf;     /* [B] valid Pareto rows, NULL = all P */
+  int32_t P;
+  trollout_child child[TROLLOUT_MAX_AGENTS];   /* entries 0 .. n_agents-1 are used */
+} trollout_agents_io;
+
 /* env and actor must live on the same device; max_batch bounds B of later calls (device buffers are allocated once);
  * pieces >= 1 (boundaries are rounded to 32 environments). */
 const char* trollout_last_error(void);
 int trollout_create(tfem_handle_t env, tactor_handle_t actor, int max_batch, int pieces, trollout_handle_t* out);
+/* The same for n_agents (1..TROLLOUT_MAX_AGENTS) distinct actor handles, stepped together by trollout_step_agents_host;
+ * n_agents = 1 is trollout_create.  Every actor must be of the env's node count and on its device (the actor ABI cannot
+ * tell; host_pipeline.HostRollout checks it). */
+int trollout_create_agents(tfem_handle_t env, const tactor_handle_t* actors, int n_agents, int max_batch, int pieces,
+                           trollout_handle_t* out);
 int trollout_destroy(trollout_handle_t h);
 
 /* Replaces the equal pieces of trollout_create by an explicit schedule: n sizes (environments), multiples of 32 except
@@ -78,12 +111,22 @@ int trollout_destroy(trollout_handle_t h);
  * to fill the GPU.  Drops the step graphs cached so far. */
 int trollout_set_pieces(trollout_handle_t h, const int32_t* sizes, int n);
 
-/* OU-noise parameters as in tactor_act.  Returns after the last piece has landed in the host buffers. */
+/* OU-noise parameters as in tactor_act.  Returns after the last piece has landed in the host buffers.  A handle of
+ * several agents returns TFEM_ERR_ARG (use trollout_step_agents_host). */
 int trollout_step_host(trollout_handle_t h, int B, const trollout_io* io, float mu, float theta, float sigma,
                        uint64_t seed);
 
+/* Every agent of the handle acts on the same parent and steps its own child: per piece the parent goes up once, then
+ * on the compute stream agent k acts on it and its env-step reads it, and child k's download starts as soon as child k
+ * is done.  mu, theta, sigma, seed: one entry per agent.  Child k is bit for bit what trollout_step_host on a handle of
+ * actor k alone gives on the same parent with coin k and agent k's noise parameters (state tuple, move range, point,
+ * status, clipped actions; OU noise included: every actor draws the call indices a single-agent step would). */
+int trollout_step_agents_host(trollout_handle_t h, int B, const trollout_agents_io* io, const float* mu,
+                              const float* theta, const float* sigma, const uint64_t* seed);
+
 /* bytes moved per environment and step: host->device, device->host (for P Pareto rows); compact_columns != 0: the
- * parent tables travel as node_y / element_section and the child state carries them too */
+ * parent tables travel as node_y / element_section and the child state carries them too.  A handle of several agents
+ * counts the parent once up and every child down. */
 int trollout_bytes_per_env(trollout_handle_t h, int P, int compact_columns, size_t* h2d, size_t* d2h);
 
 /* Drops the CUDA graphs cached for the host buffers seen so far.  A cached graph replays copies against the raw host

@@ -72,29 +72,33 @@ constexpr size_t MAX_GRAPHS = 4, MAX_SEEN = 8;
 
 struct trollout_handle_s {
   tfem_handle_t env = nullptr;
-  tactor_handle_t actor = nullptr;
+  int n_agents = 1;
+  tactor_handle_t actors[TROLLOUT_MAX_AGENTS] = {};
   int device = 0, max_batch = 0;
   std::vector<int> piece_len;                      // environments per piece (multiples of 32 but the last), sum >= max_batch
   tfem_dims dims{};
-  Dev d;
+  Dev d;                                           // the parent; the last agent's child is stepped over it in place
+  // the child buffers of agent k: kid[n_agents - 1] is `d`; the other children get their own state, move range, point,
+  // status, actions and coin, so that no child overwrites what a later act or env-step of the same piece still reads
+  Dev kid[TROLLOUT_MAX_AGENTS];
   cudaStream_t s_in = nullptr, s_run = nullptr, s_out = nullptr;
-  std::vector<cudaEvent_t> ev_in, ev_run;
+  std::vector<cudaEvent_t> ev_in, ev_run;          // ev_run: one per (piece, agent), index piece * n_agents + agent
   cudaEvent_t ev_join = nullptr;
   std::vector<void*> allocs;
   // CUDA graphs of one whole step (every copy and kernel of every piece), replayed while the caller keeps passing the
   // same pinned buffers (a driver that ping-pongs two state tuples alternates between two graphs); a buffer set is
-  // captured the second time it is seen.  The OU-noise seed / call index travel through h_ctr -> d_ctr.
+  // captured the second time it is seen.  The OU-noise seed / call index of every agent travel through h_ctr -> d_ctr.
   struct Graph {
     std::vector<uintptr_t> key;
     cudaGraphExec_t exec = nullptr;
-    int64_t env_launches = 0, actor_launches = 0;
+    int64_t env_launches = 0, actor_launches[TROLLOUT_MAX_AGENTS] = {};
     int pieces = 0;
     uint64_t last_use = 0;
   };
   std::vector<Graph> graphs;                       // at most MAX_GRAPHS, least recently used one is replaced
   std::vector<std::vector<uintptr_t>> seen_once;   // at most MAX_SEEN
   uint64_t tick = 0;
-  uint64_t* h_ctr = nullptr;      // pinned: [seed, first call index]
+  uint64_t* h_ctr = nullptr;      // pinned: [seed, first call index] per agent
   uint64_t* d_ctr = nullptr;
   bool use_graph = true;
   bool timeline = false;                           // TROLLOUT_TIMELINE=1: print per-piece event times (direct path)
@@ -119,15 +123,37 @@ cudaError_t dalloc(trollout_handle_s* h, T** p, size_t count) {
   if (e == cudaSuccess) h->allocs.push_back(*p);
   return e;
 }
-// one (upload done, kernels done) event pair per piece
+// the child buffers one agent writes (the parent-only inputs x_p, A_p, A_n, n_pf stay null)
+cudaError_t alloc_child(trollout_handle_s* h, Dev& c, size_t B) {
+  const size_t N = h->dims.N, E = h->dims.E;
+  cudaError_t e = dalloc(h, &c.x_n, B * N * 13);
+  if (e == cudaSuccess) e = dalloc(h, &c.A_s, B * N * N);
+  if (e == cudaSuccess) e = dalloc(h, &c.A_ts, B * N * N);
+  if (e == cudaSuccess) e = dalloc(h, &c.A_cs, B * N * N);
+  if (e == cudaSuccess) e = dalloc(h, &c.raw_n, B * N * 12);
+  if (e == cudaSuccess) e = dalloc(h, &c.raw_e, B * E * 21);
+  if (e == cudaSuccess) e = dalloc(h, &c.mr, B * N * 2);
+  if (e == cudaSuccess) e = dalloc(h, &c.node_y, B * N);
+  if (e == cudaSuccess) e = dalloc(h, &c.elem_sec, B * E);
+  if (e == cudaSuccess) e = dalloc(h, &c.point, B * 4);
+  if (e == cudaSuccess) e = dalloc(h, &c.a_geo, B * N * 2);
+  if (e == cudaSuccess) e = dalloc(h, &c.a_topo, B * N * 3);
+  if (e == cudaSuccess) e = dalloc(h, &c.status, B);
+  if (e == cudaSuccess) e = dalloc(h, &c.coin, B);
+  return e;
+}
+// an upload-done event per piece, a kernels-done event per piece and agent
 cudaError_t piece_events(trollout_handle_s* h, size_t n) {
   cudaError_t e = cudaSuccess;
-  while (h->ev_in.size() < n && e == cudaSuccess) {
-    cudaEvent_t a = nullptr, b = nullptr;
-    e = cudaEventCreateWithFlags(&a, cudaEventDisableTiming);
-    if (e == cudaSuccess) { h->ev_in.push_back(a); e = cudaEventCreateWithFlags(&b, cudaEventDisableTiming); }
-    if (e == cudaSuccess) h->ev_run.push_back(b);
-  }
+  auto grow = [&](std::vector<cudaEvent_t>& v, size_t count) {
+    while (v.size() < count && e == cudaSuccess) {
+      cudaEvent_t a = nullptr;
+      e = cudaEventCreateWithFlags(&a, cudaEventDisableTiming);
+      if (e == cudaSuccess) v.push_back(a);
+    }
+  };
+  grow(h->ev_in, n);
+  grow(h->ev_run, n * (size_t)h->n_agents);
   return e;
 }
 }  // namespace
@@ -137,12 +163,26 @@ extern "C" {
 const char* trollout_last_error(void) { return g_roll_err.c_str(); }
 
 int trollout_create(tfem_handle_t env, tactor_handle_t actor, int max_batch, int pieces, trollout_handle_t* out) {
-  if (!env || !actor || !out) return rfail(TFEM_ERR_ARG, "null argument");
+  return trollout_create_agents(env, &actor, 1, max_batch, pieces, out);
+}
+
+int trollout_create_agents(tfem_handle_t env, const tactor_handle_t* actors, int n_agents, int max_batch, int pieces,
+                           trollout_handle_t* out) {
+  if (!env || !actors || !out) return rfail(TFEM_ERR_ARG, "null argument");
   *out = nullptr;
+  if (n_agents < 1 || n_agents > TROLLOUT_MAX_AGENTS)
+    return rfail(TFEM_ERR_ARG, "n_agents must be in 1.." + std::to_string(TROLLOUT_MAX_AGENTS) + ", got " + std::to_string(n_agents));
+  for (int k = 0; k < n_agents; ++k) {
+    if (!actors[k]) return rfail(TFEM_ERR_ARG, "null argument");
+    // every actor draws its noise from its own call counter: one handle twice would interleave the two agents' calls
+    for (int j = 0; j < k; ++j)
+      if (actors[j] == actors[k]) return rfail(TFEM_ERR_ARG, "the agents must be distinct actor handles");
+  }
   if (max_batch <= 0 || pieces <= 0) return rfail(TFEM_ERR_ARG, "max_batch and pieces must be positive");
   trollout_handle_s* h = new (std::nothrow) trollout_handle_s();
   if (!h) return rfail(TFEM_ERR_ARG, "out of host memory");
-  h->env = env; h->actor = actor; h->max_batch = max_batch;
+  h->env = env; h->max_batch = max_batch; h->n_agents = n_agents;
+  for (int k = 0; k < n_agents; ++k) h->actors[k] = actors[k];
   if (tfem_get_dims(env, &h->dims) != TFEM_OK) { delete h; return rfail(TFEM_ERR_ARG, "bad env handle"); }
   if (tfem::handle_family_count(env) > 1) {       // the captured pipeline carries no per-environment family ids
     delete h;
@@ -156,32 +196,21 @@ int trollout_create(tfem_handle_t env, tactor_handle_t actor, int max_batch, int
   int prev_dev = -1;
   cudaGetDevice(&prev_dev);
   cudaError_t e = cudaSetDevice(h->device);
-  const size_t B = (size_t)max_batch, N = h->dims.N, E = h->dims.E;
-  if (e == cudaSuccess) e = dalloc(h, &h->d.x_n, B * N * 13);
-  if (e == cudaSuccess) e = dalloc(h, &h->d.A_s, B * N * N);
-  if (e == cudaSuccess) e = dalloc(h, &h->d.A_ts, B * N * N);
-  if (e == cudaSuccess) e = dalloc(h, &h->d.A_cs, B * N * N);
-  if (e == cudaSuccess) e = dalloc(h, &h->d.raw_n, B * N * 12);
-  if (e == cudaSuccess) e = dalloc(h, &h->d.raw_e, B * E * 21);
-  if (e == cudaSuccess) e = dalloc(h, &h->d.mr, B * N * 2);
-  if (e == cudaSuccess) e = dalloc(h, &h->d.node_y, B * N);
-  if (e == cudaSuccess) e = dalloc(h, &h->d.elem_sec, B * E);
-  if (e == cudaSuccess) e = dalloc(h, &h->d.point, B * 4);
-  if (e == cudaSuccess) e = dalloc(h, &h->d.a_geo, B * N * 2);
-  if (e == cudaSuccess) e = dalloc(h, &h->d.a_topo, B * N * 3);
+  const size_t B = (size_t)max_batch, N = h->dims.N;
+  if (e == cudaSuccess) e = alloc_child(h, h->d, B);
   if (e == cudaSuccess) e = dalloc(h, &h->d.x_p, B * PMAX * 4);
   if (e == cudaSuccess) e = dalloc(h, &h->d.A_p, B * PMAX * PMAX);
   if (e == cudaSuccess) e = dalloc(h, &h->d.A_n, N * N);
-  if (e == cudaSuccess) e = dalloc(h, &h->d.status, B);
   if (e == cudaSuccess) e = dalloc(h, &h->d.n_pf, B);
-  if (e == cudaSuccess) e = dalloc(h, &h->d.coin, B);
+  for (int k = 0; k + 1 < n_agents && e == cudaSuccess; ++k) e = alloc_child(h, h->kid[k], B);
+  h->kid[n_agents - 1] = h->d;
   if (e == cudaSuccess) {
     std::vector<float> an(N * N);
     if (tfem_get_table(env, TFEM_TAB_A_N, an.data(), an.size() * 4) != TFEM_OK) e = cudaErrorInvalidValue;
     else e = cudaMemcpy(h->d.A_n, an.data(), an.size() * 4, cudaMemcpyHostToDevice);
   }
-  if (e == cudaSuccess) e = dalloc(h, &h->d_ctr, 2);
-  if (e == cudaSuccess) e = cudaHostAlloc(reinterpret_cast<void**>(&h->h_ctr), 16, cudaHostAllocDefault);
+  if (e == cudaSuccess) e = dalloc(h, &h->d_ctr, 2 * TROLLOUT_MAX_AGENTS);
+  if (e == cudaSuccess) e = cudaHostAlloc(reinterpret_cast<void**>(&h->h_ctr), 16 * TROLLOUT_MAX_AGENTS, cudaHostAllocDefault);
   if (e == cudaSuccess) e = cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming);
   if (const char* v = getenv("TROLLOUT_NO_GRAPH")) h->use_graph = (v[0] == '0');
   if (const char* v = getenv("TROLLOUT_ZEROCOPY")) { h->zc_mode = atoi(v); h->zerocopy = h->zc_mode >= 1; }
@@ -225,8 +254,9 @@ int trollout_bytes_per_env(trollout_handle_t h, int P, int compact_columns, size
   if (!h) return rfail(TFEM_ERR_ARG, "null argument");
   const size_t N = h->dims.N, E = h->dims.E;
   const size_t graph = 4 * (N * 13 + 3 * N * N + N * 2), tables = 4 * (N * 12 + E * 21), cols = 4 * (N + E);
-  if (h2d) *h2d = graph + (compact_columns ? cols : tables) + 1 + 4 * ((size_t)P * 4 + (size_t)P * P);
-  if (d2h) *d2h = graph + tables + (compact_columns ? cols : 0) + 4 * 4 + 4 + 4 * (N * 2 + N * 3);
+  const size_t K = (size_t)h->n_agents;             // the parent goes up once with one coin per agent; every child comes down
+  if (h2d) *h2d = graph + (compact_columns ? cols : tables) + K + 4 * ((size_t)P * 4 + (size_t)P * P);
+  if (d2h) *d2h = K * (graph + tables + (compact_columns ? cols : 0) + 4 * 4 + 4 + 4 * (N * 2 + N * 3));
   return TFEM_OK;
 }
 
@@ -258,11 +288,13 @@ int trollout_forget_buffers(trollout_handle_t h) {
 }
 
 // Enqueues every copy and kernel of one step on the three streams.  ctr_dev == nullptr: the noise call index is taken
-// from the actor handle (tactor_act); otherwise from device memory (tactor_act_dev, graph capture).  join: make s_in
-// wait for the last download (needed to close a capture).
-static int enqueue_step(trollout_handle_s* h, int B, const trollout_io* io, float mu, float theta, float sigma,
-                        uint64_t seed, const uint64_t* ctr_dev, bool join, int* pieces_out) {
-  const trollout_state &si = io->in, &so = io->out;
+// from the actor handles (tactor_act); otherwise from device memory (tactor_act_dev, graph capture: [seed, first call
+// index] of agent k at ctr_dev[2k]).  join: make s_in wait for the last download (needed to close a capture).  Per
+// piece: the parent goes up once; then for every agent k in turn act, env-step and the download of child k.
+static int enqueue_step(trollout_handle_s* h, int B, const trollout_agents_io* io, const float* mu, const float* theta,
+                        const float* sigma, const uint64_t* seed, const uint64_t* ctr_dev, bool join, int* pieces_out) {
+  const trollout_state& si = io->in;
+  const int K = h->n_agents;
   const size_t N = h->dims.N, E = h->dims.E, P = (size_t)io->P;
   const Dev& d = h->d;
   const bool compact = si.node_y && si.element_section;
@@ -302,7 +334,7 @@ static int enqueue_step(trollout_handle_s* h, int B, const trollout_io* io, floa
     else e = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, h->s_out);
   };
   if (ctr_dev) {
-    up(h->d_ctr, h->h_ctr, 16);
+    up(h->d_ctr, h->h_ctr, 16 * (size_t)K);
     flush(ups, h->s_in);
   }
   if (h->timeline && !ctr_dev) {
@@ -310,6 +342,7 @@ static int enqueue_step(trollout_handle_s* h, int B, const trollout_io* io, floa
     while (h->tl.size() < need) { cudaEvent_t ev; cudaEventCreate(&ev); h->tl.push_back(ev); }
     cudaEventRecord(h->tl[0], h->s_in);
   }
+  // the timeline's run and download events of a piece are re-recorded for every agent: it reports the last child
   int piece_idx = 0;
   for (int lo = 0; lo < B && e == cudaSuccess; lo += h->piece_len[piece_idx], ++piece_idx) {
     const int len = h->piece_len[piece_idx];
@@ -329,53 +362,63 @@ static int enqueue_step(trollout_handle_s* h, int B, const trollout_io* io, floa
     up(d.mr + l * N * 2, si.move_range + l * N * 2, nb * N * 2 * 4);
     up(d.x_p + l * P * 4, io->x_p + l * P * 4, nb * P * 4 * 4);
     up(d.A_p + l * P * P, io->A_p + l * P * P, nb * P * P * 4);
-    if (io->coin) up(d.coin + l, io->coin + l, nb);
+    for (int k = 0; k < K; ++k)
+      if (io->child[k].coin) up(h->kid[k].coin + l, io->child[k].coin + l, nb);
     if (io->n_pf) up(d.n_pf + l, io->n_pf + l, nb * 4);
     flush(ups, h->s_in);
     if (e == cudaSuccess) e = cudaEventRecord(h->ev_in[piece_idx], h->s_in);
     if (h->timeline && !ctr_dev) cudaEventRecord(h->tl[1 + 4 * piece_idx + 0], h->s_in);
-    // ---- act + step ----
+    // ---- act + step, then download, agent by agent ----
     if (e == cudaSuccess) e = cudaStreamWaitEvent(h->s_run, h->ev_in[piece_idx], 0);
     if (e != cudaSuccess) break;
     tactor_inputs ai{};
     ai.x_n = d.x_n + l * N * 13; ai.A_n = d.A_n; ai.A_s = d.A_s + l * N * N; ai.A_n_ts = d.A_ts + l * N * N;
     ai.A_n_cs = d.A_cs + l * N * N; ai.x_p = d.x_p + l * P * 4; ai.A_p = d.A_p + l * P * P;
     ai.n_pf = io->n_pf ? d.n_pf + l : nullptr; ai.P = io->P;
-    int rc = ctr_dev ? tactor_act_dev(h->actor, (int)nb, &ai, d.a_geo + l * N * 2, d.a_topo + l * N * 3, mu, theta, sigma,
-                                      ctr_dev, (uint32_t)piece_idx, h->s_run)
-                     : tactor_act(h->actor, (int)nb, &ai, d.a_geo + l * N * 2, d.a_topo + l * N * 3, mu, theta, sigma, seed,
-                                  h->s_run);
-    if (rc != TFEM_OK) { if (!ctr_dev) drain(); return rfail(rc, std::string("rollout: ") + tactor_last_error()); }
-    tfem_step_in in{};
-    if (compact) { in.set_node_y = d.node_y + l * N; in.set_element_section = d.elem_sec + l * E; }
-    in.set_node = d.raw_n + l * N * 12; in.set_element = d.raw_e + l * E * 21; in.a_geo = d.a_geo + l * N * 2;
-    in.a_topo = d.a_topo + l * N * 3; in.coin = io->coin ? d.coin + l : nullptr; in.move_range = d.mr + l * N * 2;
-    tfem_step_out o{};
-    o.x_n = d.x_n + l * N * 13; o.A_s = d.A_s + l * N * N; o.A_n_ts = d.A_ts + l * N * N; o.A_n_cs = d.A_cs + l * N * N;
-    o.nN_x_n = d.raw_n + l * N * 12; o.nN_x_e = d.raw_e + l * E * 21; o.point = d.point + l * 4; o.status = d.status + l;
-    if (so.node_y) o.node_y = d.node_y + l * N;
-    if (so.element_section) o.element_section = d.elem_sec + l * E;
-    rc = tfem_step(h->env, (int)nb, &in, &o, h->s_run);
-    if (rc != TFEM_OK) { if (!ctr_dev) drain(); return rfail(rc, std::string("rollout: ") + tfem_last_error()); }
-    e = cudaEventRecord(h->ev_run[piece_idx], h->s_run);
-    if (h->timeline && !ctr_dev) cudaEventRecord(h->tl[1 + 4 * piece_idx + 1], h->s_run);
-    // ---- download ----
-    if (e == cudaSuccess) e = cudaStreamWaitEvent(h->s_out, h->ev_run[piece_idx], 0);
-    down(so.x_n ? so.x_n + l * N * 13 : nullptr, d.x_n + l * N * 13, nb * N * 13 * 4);
-    down(so.A_s ? so.A_s + l * N * N : nullptr, d.A_s + l * N * N, nb * N * N * 4);
-    down(so.A_n_ts ? so.A_n_ts + l * N * N : nullptr, d.A_ts + l * N * N, nb * N * N * 4);
-    down(so.A_n_cs ? so.A_n_cs + l * N * N : nullptr, d.A_cs + l * N * N, nb * N * N * 4);
-    down(so.nN_x_n ? so.nN_x_n + l * N * 12 : nullptr, d.raw_n + l * N * 12, nb * N * 12 * 4);
-    down(so.nN_x_e ? so.nN_x_e + l * E * 21 : nullptr, d.raw_e + l * E * 21, nb * E * 21 * 4);
-    down(so.move_range ? so.move_range + l * N * 2 : nullptr, d.mr + l * N * 2, nb * N * 2 * 4);
-    down(so.node_y ? so.node_y + l * N : nullptr, d.node_y + l * N, nb * N * 4);
-    down(so.element_section ? so.element_section + l * E : nullptr, d.elem_sec + l * E, nb * E * 4);
-    down(io->point ? io->point + l * 4 : nullptr, d.point + l * 4, nb * 4 * 4);
-    down(io->status ? io->status + l : nullptr, d.status + l, nb * 4);
-    down(io->a_geo ? io->a_geo + l * N * 2 : nullptr, d.a_geo + l * N * 2, nb * N * 2 * 4);
-    down(io->a_topo ? io->a_topo + l * N * 3 : nullptr, d.a_topo + l * N * 3, nb * N * 3 * 4);
-    flush(downs, h->s_out);
-    if (h->timeline && !ctr_dev) cudaEventRecord(h->tl[1 + 4 * piece_idx + 2], h->s_out);
+    for (int k = 0; k < K && e == cudaSuccess; ++k) {
+      const Dev& c = h->kid[k];                       // == d for the last agent: its child is written over the parent
+      const trollout_child& ch = io->child[k];
+      const trollout_state& so = ch.out;
+      int rc = ctr_dev ? tactor_act_dev(h->actors[k], (int)nb, &ai, c.a_geo + l * N * 2, c.a_topo + l * N * 3, mu[k], theta[k],
+                                        sigma[k], ctr_dev + 2 * k, (uint32_t)piece_idx, h->s_run)
+                       : tactor_act(h->actors[k], (int)nb, &ai, c.a_geo + l * N * 2, c.a_topo + l * N * 3, mu[k], theta[k],
+                                    sigma[k], seed[k], h->s_run);
+      if (rc != TFEM_OK) { if (!ctr_dev) drain(); return rfail(rc, std::string("rollout: ") + tactor_last_error()); }
+      if (c.mr != d.mr)                                // the env-step reads and writes the move range in place
+        e = cudaMemcpyAsync(c.mr + l * N * 2, d.mr + l * N * 2, nb * N * 2 * 4, cudaMemcpyDeviceToDevice, h->s_run);
+      if (e != cudaSuccess) break;
+      tfem_step_in in{};
+      if (compact) { in.set_node_y = d.node_y + l * N; in.set_element_section = d.elem_sec + l * E; }
+      in.set_node = d.raw_n + l * N * 12; in.set_element = d.raw_e + l * E * 21; in.a_geo = c.a_geo + l * N * 2;
+      in.a_topo = c.a_topo + l * N * 3; in.coin = ch.coin ? c.coin + l : nullptr; in.move_range = c.mr + l * N * 2;
+      tfem_step_out o{};
+      o.x_n = c.x_n + l * N * 13; o.A_s = c.A_s + l * N * N; o.A_n_ts = c.A_ts + l * N * N; o.A_n_cs = c.A_cs + l * N * N;
+      o.nN_x_n = c.raw_n + l * N * 12; o.nN_x_e = c.raw_e + l * E * 21; o.point = c.point + l * 4; o.status = c.status + l;
+      if (so.node_y) o.node_y = c.node_y + l * N;
+      if (so.element_section) o.element_section = c.elem_sec + l * E;
+      rc = tfem_step(h->env, (int)nb, &in, &o, h->s_run);
+      if (rc != TFEM_OK) { if (!ctr_dev) drain(); return rfail(rc, std::string("rollout: ") + tfem_last_error()); }
+      cudaEvent_t done = h->ev_run[(size_t)piece_idx * K + k];
+      e = cudaEventRecord(done, h->s_run);
+      if (h->timeline && !ctr_dev) cudaEventRecord(h->tl[1 + 4 * piece_idx + 1], h->s_run);
+      // ---- download of child k: one list per child (a transfer kernel takes at most COPY_MAX arrays) ----
+      if (e == cudaSuccess) e = cudaStreamWaitEvent(h->s_out, done, 0);
+      down(so.x_n ? so.x_n + l * N * 13 : nullptr, c.x_n + l * N * 13, nb * N * 13 * 4);
+      down(so.A_s ? so.A_s + l * N * N : nullptr, c.A_s + l * N * N, nb * N * N * 4);
+      down(so.A_n_ts ? so.A_n_ts + l * N * N : nullptr, c.A_ts + l * N * N, nb * N * N * 4);
+      down(so.A_n_cs ? so.A_n_cs + l * N * N : nullptr, c.A_cs + l * N * N, nb * N * N * 4);
+      down(so.nN_x_n ? so.nN_x_n + l * N * 12 : nullptr, c.raw_n + l * N * 12, nb * N * 12 * 4);
+      down(so.nN_x_e ? so.nN_x_e + l * E * 21 : nullptr, c.raw_e + l * E * 21, nb * E * 21 * 4);
+      down(so.move_range ? so.move_range + l * N * 2 : nullptr, c.mr + l * N * 2, nb * N * 2 * 4);
+      down(so.node_y ? so.node_y + l * N : nullptr, c.node_y + l * N, nb * N * 4);
+      down(so.element_section ? so.element_section + l * E : nullptr, c.elem_sec + l * E, nb * E * 4);
+      down(ch.point ? ch.point + l * 4 : nullptr, c.point + l * 4, nb * 4 * 4);
+      down(ch.status ? ch.status + l : nullptr, c.status + l, nb * 4);
+      down(ch.a_geo ? ch.a_geo + l * N * 2 : nullptr, c.a_geo + l * N * 2, nb * N * 2 * 4);
+      down(ch.a_topo ? ch.a_topo + l * N * 3 : nullptr, c.a_topo + l * N * 3, nb * N * 3 * 4);
+      flush(downs, h->s_out);
+      if (h->timeline && !ctr_dev) cudaEventRecord(h->tl[1 + 4 * piece_idx + 2], h->s_out);
+    }
   }
   if (join) {
     if (e == cudaSuccess) e = cudaEventRecord(h->ev_join, h->s_out);
@@ -397,12 +440,12 @@ static bool pinned(const void* p, bool* mapped = nullptr) {
   return a.type == cudaMemoryTypeHost;
 }
 
-int trollout_step_host(trollout_handle_t h, int B, const trollout_io* io, float mu, float theta, float sigma,
-                       uint64_t seed) {
-  if (!h || !io) return rfail(TFEM_ERR_ARG, "null argument");
+static int step_agents(trollout_handle_t h, int B, const trollout_agents_io* io, const float* mu, const float* theta,
+                       const float* sigma, const uint64_t* seed) {
   if (B < 0 || B > h->max_batch) return rfail(TFEM_ERR_ARG, "batch exceeds max_batch");
   if (B == 0) return TFEM_OK;
-  const trollout_state &si = io->in, &so = io->out;
+  const int K = h->n_agents;
+  const trollout_state& si = io->in;
   const bool compact_in = si.node_y && si.element_section;
   if (!si.x_n || !si.A_s || !si.A_n_ts || !si.A_n_cs || (!compact_in && (!si.nN_x_n || !si.nN_x_e)) || !si.move_range ||
       !io->x_p || !io->A_p)
@@ -415,19 +458,25 @@ int trollout_step_host(trollout_handle_t h, int B, const trollout_io* io, float 
   if (e != cudaSuccess) return rfail(TFEM_ERR_CUDA, std::string("rollout step: ") + cudaGetErrorString(e));
 
   // ---- graph path: same pinned buffers as the captured step -> one cudaGraphLaunch instead of ~30 API calls a piece ----
-  const void* ptrs[] = {si.x_n, si.A_s, si.A_n_ts, si.A_n_cs, compact_in ? nullptr : si.nN_x_n, compact_in ? nullptr : si.nN_x_e,
-                        si.move_range, si.node_y, si.element_section, io->coin, io->x_p, io->A_p,
-                        io->n_pf, so.x_n, so.A_s, so.A_n_ts, so.A_n_cs, so.nN_x_n, so.nN_x_e, so.move_range, so.node_y,
-                        so.element_section, io->point, io->status, io->a_geo, io->a_topo};
-  const bool noise = !(sigma == 0.f && theta == 0.f);
+  std::vector<const void*> ptrs = {si.x_n, si.A_s, si.A_n_ts, si.A_n_cs, compact_in ? nullptr : si.nN_x_n,
+                                   compact_in ? nullptr : si.nN_x_e, si.move_range, si.node_y, si.element_section,
+                                   io->x_p, io->A_p, io->n_pf};
+  for (int k = 0; k < K; ++k) {
+    const trollout_child& c = io->child[k];
+    const trollout_state& so = c.out;
+    ptrs.insert(ptrs.end(), {c.coin, so.x_n, so.A_s, so.A_n_ts, so.A_n_cs, so.nN_x_n, so.nN_x_e, so.move_range, so.node_y,
+                             so.element_section, c.point, c.status, c.a_geo, c.a_topo});
+  }
   const auto t_begin = std::chrono::steady_clock::now();
   if (h->use_graph) {
     std::vector<uintptr_t> key;
     for (const void* p : ptrs) key.push_back(reinterpret_cast<uintptr_t>(p));
-    uint32_t fb[3];
-    memcpy(&fb[0], &mu, 4); memcpy(&fb[1], &theta, 4); memcpy(&fb[2], &sigma, 4);
     key.push_back((uintptr_t)B); key.push_back((uintptr_t)io->P);
-    key.push_back(fb[0]); key.push_back(fb[1]); key.push_back(fb[2]);
+    for (int k = 0; k < K; ++k) {
+      uint32_t fb[3];
+      memcpy(&fb[0], &mu[k], 4); memcpy(&fb[1], &theta[k], 4); memcpy(&fb[2], &sigma[k], 4);
+      key.push_back(fb[0]); key.push_back(fb[1]); key.push_back(fb[2]);
+    }
     trollout_handle_s::Graph* hit = nullptr;
     for (auto& g : h->graphs) if (g.key == key) hit = &g;
     if (!hit) {
@@ -443,7 +492,9 @@ int trollout_step_host(trollout_handle_t h, int B, const trollout_io* io, float 
         if (all_pinned) {
           h->zc_capture = all_mapped;
           trollout_handle_s::Graph ng;
-          const int64_t env0 = tfem_launch_count(h->env), act0 = tactor_launch_count(h->actor);
+          int64_t act0[TROLLOUT_MAX_AGENTS];
+          const int64_t env0 = tfem_launch_count(h->env);
+          for (int k = 0; k < K; ++k) act0[k] = tactor_launch_count(h->actors[k]);
           e = cudaStreamBeginCapture(h->s_in, cudaStreamCaptureModeRelaxed);
           if (e != cudaSuccess) return rfail(TFEM_ERR_CUDA, std::string("rollout capture: ") + cudaGetErrorString(e));
           const int rc = enqueue_step(h, B, io, mu, theta, sigma, seed, h->d_ctr, true, &ng.pieces);
@@ -451,9 +502,11 @@ int trollout_step_host(trollout_handle_t h, int B, const trollout_io* io, float 
           e = cudaStreamEndCapture(h->s_in, &g);
           // the kernels were recorded, not run: take their bookings back (every replay books them)
           ng.env_launches = tfem_launch_count(h->env) - env0;
-          ng.actor_launches = tactor_launch_count(h->actor) - act0;
           tfem_book_launches(h->env, -ng.env_launches);
-          tactor_reserve_calls(h->actor, 0, -ng.actor_launches);
+          for (int k = 0; k < K; ++k) {
+            ng.actor_launches[k] = tactor_launch_count(h->actors[k]) - act0[k];
+            tactor_reserve_calls(h->actors[k], 0, -ng.actor_launches[k]);
+          }
           if (rc != TFEM_OK) { if (g) cudaGraphDestroy(g); cudaGetLastError(); return rc; }
           if (e == cudaSuccess) e = cudaGraphInstantiate(&ng.exec, g, 0);
           if (g) cudaGraphDestroy(g);
@@ -484,8 +537,11 @@ int trollout_step_host(trollout_handle_t h, int B, const trollout_io* io, float 
     }
     if (hit) {
       hit->last_use = ++h->tick;
-      h->h_ctr[0] = seed;
-      h->h_ctr[1] = tactor_reserve_calls(h->actor, noise ? (uint32_t)hit->pieces : 0u, hit->actor_launches);
+      for (int k = 0; k < K; ++k) {                  // the call indices the direct path would have drawn
+        const bool noise = !(sigma[k] == 0.f && theta[k] == 0.f);
+        h->h_ctr[2 * k] = seed[k];
+        h->h_ctr[2 * k + 1] = tactor_reserve_calls(h->actors[k], noise ? (uint32_t)hit->pieces : 0u, hit->actor_launches[k]);
+      }
       tfem_book_launches(h->env, hit->env_launches);
       const auto t_launch = std::chrono::steady_clock::now();
       e = cudaGraphLaunch(hit->exec, h->s_in);
@@ -524,6 +580,25 @@ int trollout_step_host(trollout_handle_t h, int B, const trollout_io* io, float 
   }
   if (e != cudaSuccess) return rfail(TFEM_ERR_CUDA, std::string("rollout step: ") + cudaGetErrorString(e));
   return TFEM_OK;
+}
+
+int trollout_step_host(trollout_handle_t h, int B, const trollout_io* io, float mu, float theta, float sigma,
+                       uint64_t seed) {
+  if (!h || !io) return rfail(TFEM_ERR_ARG, "null argument");
+  if (h->n_agents != 1)
+    return rfail(TFEM_ERR_ARG, "the rollout handle runs " + std::to_string(h->n_agents) +
+                                   " agents (trollout_create_agents): step it with trollout_step_agents_host");
+  trollout_agents_io a{};
+  a.in = io->in; a.x_p = io->x_p; a.A_p = io->A_p; a.n_pf = io->n_pf; a.P = io->P;
+  a.child[0].out = io->out; a.child[0].coin = io->coin; a.child[0].point = io->point; a.child[0].status = io->status;
+  a.child[0].a_geo = io->a_geo; a.child[0].a_topo = io->a_topo;
+  return step_agents(h, B, &a, &mu, &theta, &sigma, &seed);
+}
+
+int trollout_step_agents_host(trollout_handle_t h, int B, const trollout_agents_io* io, const float* mu,
+                              const float* theta, const float* sigma, const uint64_t* seed) {
+  if (!h || !io || !mu || !theta || !sigma || !seed) return rfail(TFEM_ERR_ARG, "null argument");
+  return step_agents(h, B, io, mu, theta, sigma, seed);
 }
 
 }  // extern "C"
