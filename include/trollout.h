@@ -23,6 +23,11 @@
  * trollout_create_agents / trollout_step_agents_host run the driver's whole inner step -- up to three agents acting on
  * the same parent -- in one call: the parent crosses the link once instead of once per agent, and one graph launch
  * and one pipeline fill serve all agents.
+ *
+ * trollout_step_host_mixed / trollout_step_agents_host_mixed step a rollout whose env handle was made by
+ * tfem_create_mixed: the batch of the training driver, where every episode has its own shape and truss type
+ * (train/code/master_DDPG_truss2D_MO.py:787-815).  The parent's family ids go up with the parent, one tfem_step_mixed
+ * launch per piece and agent steps environments of every family, and every child keeps its parent's ids.
  */
 #ifndef TROLLOUT_H_
 #define TROLLOUT_H_
@@ -95,7 +100,8 @@ typedef struct trollout_agents_io {
 } trollout_agents_io;
 
 /* env and actor must live on the same device; max_batch bounds B of later calls (device buffers are allocated once);
- * pieces >= 1 (boundaries are rounded to 32 environments). */
+ * pieces >= 1 (boundaries are rounded to 32 environments).  env may be a handle of several families (tfem_create_mixed):
+ * such a rollout steps with the _mixed calls below. */
 const char* trollout_last_error(void);
 int trollout_create(tfem_handle_t env, tactor_handle_t actor, int max_batch, int pieces, trollout_handle_t* out);
 /* The same for n_agents (1..TROLLOUT_MAX_AGENTS) distinct actor handles, stepped together by trollout_step_agents_host;
@@ -112,7 +118,8 @@ int trollout_destroy(trollout_handle_t h);
 int trollout_set_pieces(trollout_handle_t h, const int32_t* sizes, int n);
 
 /* OU-noise parameters as in tactor_act.  Returns after the last piece has landed in the host buffers.  A handle of
- * several agents returns TFEM_ERR_ARG (use trollout_step_agents_host). */
+ * several agents returns TFEM_ERR_ARG (use trollout_step_agents_host), and so does an env handle of several families
+ * (use trollout_step_host_mixed). */
 int trollout_step_host(trollout_handle_t h, int B, const trollout_io* io, float mu, float theta, float sigma,
                        uint64_t seed);
 
@@ -124,9 +131,24 @@ int trollout_step_host(trollout_handle_t h, int B, const trollout_io* io, float 
 int trollout_step_agents_host(trollout_handle_t h, int B, const trollout_agents_io* io, const float* mu,
                               const float* theta, const float* sigma, const uint64_t* seed);
 
+/* The two steps above over a mixed-family batch (tfem_step_mixed): family is a HOST array [B] of uint8 indices into
+ * the env handle's families, 16-byte aligned (TFEM_ERR_ALIGN otherwise; pinned for overlap and for the graph).  It goes
+ * up with the parent; nothing about it comes down, because every child has its parent's families.  Environment b of
+ * every child is bit for bit what the plain call gives on a rollout over a handle of family family[b] alone, with the
+ * same pieces.  A captured step reads the ids when it is replayed, so the caller may rewrite them in the same buffer
+ * between steps.  An id >= the handle's family count sets TFEM_STATUS_BAD_FAMILY in that environment's status; the
+ * child's other host outputs for that environment are then unspecified (they carry whatever the rollout's device
+ * buffers held), and every other environment is unaffected.  An env handle made by tfem_create returns TFEM_ERR_ARG.
+ * A handle of one family made by tfem_create_mixed may be stepped by both kinds of call. */
+int trollout_step_host_mixed(trollout_handle_t h, int B, const uint8_t* family, const trollout_io* io, float mu,
+                             float theta, float sigma, uint64_t seed);
+int trollout_step_agents_host_mixed(trollout_handle_t h, int B, const uint8_t* family, const trollout_agents_io* io,
+                                    const float* mu, const float* theta, const float* sigma, const uint64_t* seed);
+
 /* bytes moved per environment and step: host->device, device->host (for P Pareto rows); compact_columns != 0: the
  * parent tables travel as node_y / element_section and the child state carries them too.  A handle of several agents
- * counts the parent once up and every child down. */
+ * counts the parent once up and every child down; an env handle of several families adds the parent's family id (1 byte)
+ * up. */
 int trollout_bytes_per_env(trollout_handle_t h, int P, int compact_columns, size_t* h2d, size_t* d2h);
 
 /* Drops the CUDA graphs cached for the host buffers seen so far.  A cached graph replays copies against the raw host

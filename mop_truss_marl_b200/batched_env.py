@@ -206,7 +206,8 @@ class MixedTrussEnv(BatchedTrussEnv):
     ``reset(family_ids)`` takes a uint8 CUDA tensor [B] of indices into ``families`` and keeps a copy as
     ``self.family_ids``; ``step`` has the signature of ``BatchedTrussEnv.step`` (``parent=`` children copy the parent's
     family ids).  ``int_obj`` is [F, 2].  The single-family calls (``solve_only``, ``solve_dense_dmma``) and
-    ``host_pipeline.HostRollout`` refuse a batch of more than one family."""
+    ``host_pipeline.HostRollout`` refuse a batch of more than one family; ``host_pipeline.MixedHostRollout`` steps it
+    from host-resident state."""
 
     def __init__(self, families, batch: int, device="cuda:0", fp64_outputs: bool = True):
         self.specs = tuple(FAMILIES[f] if isinstance(f, str) else f for f in families)

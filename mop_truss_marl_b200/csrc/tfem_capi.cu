@@ -52,7 +52,7 @@ int single_family(tfem_handle_t h, const char* call, const char* instead) {
 
 // the mixed entry points need the mixed kernel configured (tfem_create_mixed); a tables-only handle fails at launch
 int mixed_family(tfem_handle_t h, const char* call) {
-  if (h->device < 0 || h->launch.smem_mixed > 0) return 0;
+  if (h->device < 0 || tfem::handle_is_mixed(h)) return 0;
   return fail(TFEM_ERR_ARG, std::string(call) + ": the handle was made by tfem_create; use tfem_create_mixed");
 }
 
@@ -441,3 +441,4 @@ void tfem_book_launches(tfem_handle_t h, int64_t n) { if (h) h->launches.fetch_a
 }  // extern "C"
 
 int tfem::handle_family_count(tfem_handle_t h) { return h ? h->n_families : 0; }
+bool tfem::handle_is_mixed(tfem_handle_t h) { return h && h->launch.smem_mixed > 0; }

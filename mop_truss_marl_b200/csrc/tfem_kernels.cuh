@@ -41,6 +41,8 @@ int step_kernel_launch(int nx, const StepArgs& args, const LaunchInfo& info, cud
 
 // families staged by a handle (tfem_create_mixed); internal to the library, not part of the C ABI
 __attribute__((visibility("hidden"))) int handle_family_count(tfem_handle_t h);
+// the handle has the mixed-family kernel configured (made by tfem_create_mixed on a device): tfem_step_mixed serves it
+__attribute__((visibility("hidden"))) bool handle_is_mixed(tfem_handle_t h);
 
 // dense blocked Cholesky with DMMA trailing updates (tfem_dense.cu); returns cudaError_t as int
 int dense_solve_launch(const FamilyTables* d_tables, int B, const double* y, const int32_t* section, double* d,

@@ -20,6 +20,7 @@ struct Dev {
   float *node_y = nullptr, *elem_sec = nullptr;     // compact live columns of the raw tables
   int32_t *status = nullptr, *n_pf = nullptr;
   uint8_t* coin = nullptr;
+  uint8_t* family = nullptr;                        // the parent's family ids (an env handle made by tfem_create_mixed)
 };
 constexpr int PMAX = 50;
 
@@ -184,10 +185,6 @@ int trollout_create_agents(tfem_handle_t env, const tactor_handle_t* actors, int
   h->env = env; h->max_batch = max_batch; h->n_agents = n_agents;
   for (int k = 0; k < n_agents; ++k) h->actors[k] = actors[k];
   if (tfem_get_dims(env, &h->dims) != TFEM_OK) { delete h; return rfail(TFEM_ERR_ARG, "bad env handle"); }
-  if (tfem::handle_family_count(env) > 1) {       // the captured pipeline carries no per-environment family ids
-    delete h;
-    return rfail(TFEM_ERR_UNSUPPORTED, "the env handle holds several families (tfem_create_mixed): the rollout steps one family");
-  }
   int piece = (max_batch + pieces - 1) / pieces;
   piece = (piece + 31) / 32 * 32;                  // piece boundaries on 32 environments: every sub-array stays 16-byte aligned
   for (int lo = 0; lo < max_batch; lo += piece) h->piece_len.push_back(piece);
@@ -202,6 +199,7 @@ int trollout_create_agents(tfem_handle_t env, const tactor_handle_t* actors, int
   if (e == cudaSuccess) e = dalloc(h, &h->d.A_p, B * PMAX * PMAX);
   if (e == cudaSuccess) e = dalloc(h, &h->d.A_n, N * N);
   if (e == cudaSuccess) e = dalloc(h, &h->d.n_pf, B);
+  if (e == cudaSuccess && tfem::handle_is_mixed(env)) e = dalloc(h, &h->d.family, B);
   for (int k = 0; k + 1 < n_agents && e == cudaSuccess; ++k) e = alloc_child(h, h->kid[k], B);
   h->kid[n_agents - 1] = h->d;
   if (e == cudaSuccess) {
@@ -255,7 +253,8 @@ int trollout_bytes_per_env(trollout_handle_t h, int P, int compact_columns, size
   const size_t N = h->dims.N, E = h->dims.E;
   const size_t graph = 4 * (N * 13 + 3 * N * N + N * 2), tables = 4 * (N * 12 + E * 21), cols = 4 * (N + E);
   const size_t K = (size_t)h->n_agents;             // the parent goes up once with one coin per agent; every child comes down
-  if (h2d) *h2d = graph + (compact_columns ? cols : tables) + K + 4 * ((size_t)P * 4 + (size_t)P * P);
+  const size_t family = tfem::handle_family_count(h->env) > 1 ? 1 : 0;   // the parent's family id
+  if (h2d) *h2d = graph + (compact_columns ? cols : tables) + K + family + 4 * ((size_t)P * 4 + (size_t)P * P);
   if (d2h) *d2h = K * (graph + tables + (compact_columns ? cols : 0) + 4 * 4 + 4 + 4 * (N * 2 + N * 3));
   return TFEM_OK;
 }
@@ -291,8 +290,10 @@ int trollout_forget_buffers(trollout_handle_t h) {
 // from the actor handles (tactor_act); otherwise from device memory (tactor_act_dev, graph capture: [seed, first call
 // index] of agent k at ctr_dev[2k]).  join: make s_in wait for the last download (needed to close a capture).  Per
 // piece: the parent goes up once; then for every agent k in turn act, env-step and the download of child k.
-static int enqueue_step(trollout_handle_s* h, int B, const trollout_agents_io* io, const float* mu, const float* theta,
-                        const float* sigma, const uint64_t* seed, const uint64_t* ctr_dev, bool join, int* pieces_out) {
+// family != nullptr (host [B]): the ids go up with the parent and the env-steps are tfem_step_mixed.
+static int enqueue_step(trollout_handle_s* h, int B, const uint8_t* family, const trollout_agents_io* io, const float* mu,
+                        const float* theta, const float* sigma, const uint64_t* seed, const uint64_t* ctr_dev, bool join,
+                        int* pieces_out) {
   const trollout_state& si = io->in;
   const int K = h->n_agents;
   const size_t N = h->dims.N, E = h->dims.E, P = (size_t)io->P;
@@ -365,6 +366,7 @@ static int enqueue_step(trollout_handle_s* h, int B, const trollout_agents_io* i
     for (int k = 0; k < K; ++k)
       if (io->child[k].coin) up(h->kid[k].coin + l, io->child[k].coin + l, nb);
     if (io->n_pf) up(d.n_pf + l, io->n_pf + l, nb * 4);
+    if (family) up(d.family + l, family + l, nb);
     flush(ups, h->s_in);
     if (e == cudaSuccess) e = cudaEventRecord(h->ev_in[piece_idx], h->s_in);
     if (h->timeline && !ctr_dev) cudaEventRecord(h->tl[1 + 4 * piece_idx + 0], h->s_in);
@@ -396,7 +398,8 @@ static int enqueue_step(trollout_handle_s* h, int B, const trollout_agents_io* i
       o.nN_x_n = c.raw_n + l * N * 12; o.nN_x_e = c.raw_e + l * E * 21; o.point = c.point + l * 4; o.status = c.status + l;
       if (so.node_y) o.node_y = c.node_y + l * N;
       if (so.element_section) o.element_section = c.elem_sec + l * E;
-      rc = tfem_step(h->env, (int)nb, &in, &o, h->s_run);
+      rc = family ? tfem_step_mixed(h->env, (int)nb, d.family + l, &in, &o, h->s_run)
+                  : tfem_step(h->env, (int)nb, &in, &o, h->s_run);
       if (rc != TFEM_OK) { if (!ctr_dev) drain(); return rfail(rc, std::string("rollout: ") + tfem_last_error()); }
       cudaEvent_t done = h->ev_run[(size_t)piece_idx * K + k];
       e = cudaEventRecord(done, h->s_run);
@@ -440,8 +443,8 @@ static bool pinned(const void* p, bool* mapped = nullptr) {
   return a.type == cudaMemoryTypeHost;
 }
 
-static int step_agents(trollout_handle_t h, int B, const trollout_agents_io* io, const float* mu, const float* theta,
-                       const float* sigma, const uint64_t* seed) {
+static int step_agents(trollout_handle_t h, int B, const uint8_t* family, const trollout_agents_io* io, const float* mu,
+                       const float* theta, const float* sigma, const uint64_t* seed) {
   if (B < 0 || B > h->max_batch) return rfail(TFEM_ERR_ARG, "batch exceeds max_batch");
   if (B == 0) return TFEM_OK;
   const int K = h->n_agents;
@@ -460,7 +463,7 @@ static int step_agents(trollout_handle_t h, int B, const trollout_agents_io* io,
   // ---- graph path: same pinned buffers as the captured step -> one cudaGraphLaunch instead of ~30 API calls a piece ----
   std::vector<const void*> ptrs = {si.x_n, si.A_s, si.A_n_ts, si.A_n_cs, compact_in ? nullptr : si.nN_x_n,
                                    compact_in ? nullptr : si.nN_x_e, si.move_range, si.node_y, si.element_section,
-                                   io->x_p, io->A_p, io->n_pf};
+                                   io->x_p, io->A_p, io->n_pf, family};
   for (int k = 0; k < K; ++k) {
     const trollout_child& c = io->child[k];
     const trollout_state& so = c.out;
@@ -471,7 +474,7 @@ static int step_agents(trollout_handle_t h, int B, const trollout_agents_io* io,
   if (h->use_graph) {
     std::vector<uintptr_t> key;
     for (const void* p : ptrs) key.push_back(reinterpret_cast<uintptr_t>(p));
-    key.push_back((uintptr_t)B); key.push_back((uintptr_t)io->P);
+    key.push_back((uintptr_t)B); key.push_back((uintptr_t)io->P); key.push_back(family != nullptr);
     for (int k = 0; k < K; ++k) {
       uint32_t fb[3];
       memcpy(&fb[0], &mu[k], 4); memcpy(&fb[1], &theta[k], 4); memcpy(&fb[2], &sigma[k], 4);
@@ -497,7 +500,7 @@ static int step_agents(trollout_handle_t h, int B, const trollout_agents_io* io,
           for (int k = 0; k < K; ++k) act0[k] = tactor_launch_count(h->actors[k]);
           e = cudaStreamBeginCapture(h->s_in, cudaStreamCaptureModeRelaxed);
           if (e != cudaSuccess) return rfail(TFEM_ERR_CUDA, std::string("rollout capture: ") + cudaGetErrorString(e));
-          const int rc = enqueue_step(h, B, io, mu, theta, sigma, seed, h->d_ctr, true, &ng.pieces);
+          const int rc = enqueue_step(h, B, family, io, mu, theta, sigma, seed, h->d_ctr, true, &ng.pieces);
           cudaGraph_t g = nullptr;
           e = cudaStreamEndCapture(h->s_in, &g);
           // the kernels were recorded, not run: take their bookings back (every replay books them)
@@ -560,7 +563,7 @@ static int step_agents(trollout_handle_t h, int B, const trollout_agents_io* io,
   }
   // ---- direct path (pageable buffers, or TROLLOUT_NO_GRAPH=1) ----
   int np_done = 0;
-  if (int rc = enqueue_step(h, B, io, mu, theta, sigma, seed, nullptr, false, &np_done)) {
+  if (int rc = enqueue_step(h, B, family, io, mu, theta, sigma, seed, nullptr, false, &np_done)) {
     // a piece failed mid-step: copies of earlier pieces may still be reading / writing the caller's host buffers
     cudaStreamSynchronize(h->s_in); cudaStreamSynchronize(h->s_run); cudaStreamSynchronize(h->s_out);
     return rc;
@@ -582,23 +585,66 @@ static int step_agents(trollout_handle_t h, int B, const trollout_agents_io* io,
   return TFEM_OK;
 }
 
+// the plain steps serve an env handle of one family (as tfem_step does)
+static int single_family(trollout_handle_t h, const char* call, const char* instead) {
+  const int F = tfem::handle_family_count(h->env);
+  if (F == 1) return TFEM_OK;
+  return rfail(TFEM_ERR_ARG, std::string(call) + ": the env handle holds " + std::to_string(F) + " families; use " + instead);
+}
+
+// the _mixed steps need the mixed env-step (tfem_create_mixed) and ids the transfer kernel can read in 16-byte units
+static int mixed_family(trollout_handle_t h, const uint8_t* family, const char* call) {
+  if (!tfem::handle_is_mixed(h->env))
+    return rfail(TFEM_ERR_ARG, std::string(call) + ": the env handle was made by tfem_create; make it with tfem_create_mixed");
+  if (!family) return rfail(TFEM_ERR_ARG, std::string(call) + ": the family ids are required");
+  if (reinterpret_cast<uintptr_t>(family) & 15)
+    return rfail(TFEM_ERR_ALIGN, std::string(call) + ": the family ids must be 16-byte aligned");
+  return TFEM_OK;
+}
+
+// the one-agent call as a trollout_agents_io of one child
+static trollout_agents_io one_child(const trollout_io* io) {
+  trollout_agents_io a{};
+  a.in = io->in; a.x_p = io->x_p; a.A_p = io->A_p; a.n_pf = io->n_pf; a.P = io->P;
+  a.child[0].out = io->out; a.child[0].coin = io->coin; a.child[0].point = io->point; a.child[0].status = io->status;
+  a.child[0].a_geo = io->a_geo; a.child[0].a_topo = io->a_topo;
+  return a;
+}
+
 int trollout_step_host(trollout_handle_t h, int B, const trollout_io* io, float mu, float theta, float sigma,
                        uint64_t seed) {
   if (!h || !io) return rfail(TFEM_ERR_ARG, "null argument");
   if (h->n_agents != 1)
     return rfail(TFEM_ERR_ARG, "the rollout handle runs " + std::to_string(h->n_agents) +
                                    " agents (trollout_create_agents): step it with trollout_step_agents_host");
-  trollout_agents_io a{};
-  a.in = io->in; a.x_p = io->x_p; a.A_p = io->A_p; a.n_pf = io->n_pf; a.P = io->P;
-  a.child[0].out = io->out; a.child[0].coin = io->coin; a.child[0].point = io->point; a.child[0].status = io->status;
-  a.child[0].a_geo = io->a_geo; a.child[0].a_topo = io->a_topo;
-  return step_agents(h, B, &a, &mu, &theta, &sigma, &seed);
+  if (int rc = single_family(h, "trollout_step_host", "trollout_step_host_mixed")) return rc;
+  const trollout_agents_io a = one_child(io);
+  return step_agents(h, B, nullptr, &a, &mu, &theta, &sigma, &seed);
 }
 
 int trollout_step_agents_host(trollout_handle_t h, int B, const trollout_agents_io* io, const float* mu,
                               const float* theta, const float* sigma, const uint64_t* seed) {
   if (!h || !io || !mu || !theta || !sigma || !seed) return rfail(TFEM_ERR_ARG, "null argument");
-  return step_agents(h, B, io, mu, theta, sigma, seed);
+  if (int rc = single_family(h, "trollout_step_agents_host", "trollout_step_agents_host_mixed")) return rc;
+  return step_agents(h, B, nullptr, io, mu, theta, sigma, seed);
+}
+
+int trollout_step_host_mixed(trollout_handle_t h, int B, const uint8_t* family, const trollout_io* io, float mu,
+                             float theta, float sigma, uint64_t seed) {
+  if (!h || !io) return rfail(TFEM_ERR_ARG, "null argument");
+  if (h->n_agents != 1)
+    return rfail(TFEM_ERR_ARG, "the rollout handle runs " + std::to_string(h->n_agents) +
+                                   " agents (trollout_create_agents): step it with trollout_step_agents_host_mixed");
+  if (int rc = mixed_family(h, family, "trollout_step_host_mixed")) return rc;
+  const trollout_agents_io a = one_child(io);
+  return step_agents(h, B, family, &a, &mu, &theta, &sigma, &seed);
+}
+
+int trollout_step_agents_host_mixed(trollout_handle_t h, int B, const uint8_t* family, const trollout_agents_io* io,
+                                    const float* mu, const float* theta, const float* sigma, const uint64_t* seed) {
+  if (!h || !io || !mu || !theta || !sigma || !seed) return rfail(TFEM_ERR_ARG, "null argument");
+  if (int rc = mixed_family(h, family, "trollout_step_agents_host_mixed")) return rc;
+  return step_agents(h, B, family, io, mu, theta, sigma, seed);
 }
 
 }  // extern "C"

@@ -10,6 +10,10 @@ and piece i-1 downloads (PCIe is full duplex).  PyTorch only provides the pinned
 ``HostRollout(env, [actor0, actor1, actor2])`` runs the driver's whole inner step in one call
 (``trollout_step_agents_host``): every agent acts on the same parent and steps its own child
 (``master_DDPG_truss2D_MO.py:249-260``), and the parent crosses the link once instead of once per agent.
+
+``MixedHostRollout(mix_env, actors)`` does the same over a ``batched_env.MixedTrussEnv``, the training driver's batch
+of episodes of different shapes and truss types (``trollout_step_host_mixed`` / ``trollout_step_agents_host_mixed``):
+the state tuple carries each environment's family id as ``"family"``.
 """
 from __future__ import annotations
 
@@ -27,7 +31,7 @@ STATE_OUT = ("x_n", "A_s", "A_n_ts", "A_n_cs", "nN_x_n", "nN_x_e", "move_range",
 COMPACT = ("node_y", "element_section")
 ROLLOUT_EXPORTS = ("trollout_last_error", "trollout_create", "trollout_destroy", "trollout_step_host",
                    "trollout_bytes_per_env", "trollout_forget_buffers", "trollout_set_pieces", "trollout_create_agents",
-                   "trollout_step_agents_host")
+                   "trollout_step_agents_host", "trollout_step_host_mixed", "trollout_step_agents_host_mixed")
 MAX_AGENTS = 3                                   # TROLLOUT_MAX_AGENTS
 
 
@@ -59,6 +63,11 @@ _lib.trollout_create_agents.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.c_i
 _lib.trollout_step_host.argtypes = [C.c_void_p, C.c_int, C.POINTER(_IO), C.c_float, C.c_float, C.c_float, C.c_uint64]
 _lib.trollout_step_agents_host.argtypes = [C.c_void_p, C.c_int, C.POINTER(_AgentsIO), C.POINTER(C.c_float),
                                            C.POINTER(C.c_float), C.POINTER(C.c_float), C.POINTER(C.c_uint64)]
+_lib.trollout_step_host_mixed.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.POINTER(_IO), C.c_float, C.c_float,
+                                          C.c_float, C.c_uint64]
+_lib.trollout_step_agents_host_mixed.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.POINTER(_AgentsIO),
+                                                 C.POINTER(C.c_float), C.POINTER(C.c_float), C.POINTER(C.c_float),
+                                                 C.POINTER(C.c_uint64)]
 _lib.trollout_bytes_per_env.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_size_t), C.POINTER(C.c_size_t)]
 _lib.trollout_forget_buffers.argtypes = [C.c_void_p]
 _lib.trollout_set_pieces.argtypes = [C.c_void_p, C.POINTER(C.c_int32), C.c_int]
@@ -84,10 +93,15 @@ class HostRollout:
     copy engines, whose per-copy cost makes more pieces a loss.  With several agents "auto" counts the download of one
     child, which is what one transfer of a piece carries: the pieces are those of a one-agent rollout."""
 
+    _mixed = False                             # steps through the _mixed calls (MixedHostRollout)
+
     def __init__(self, env, actor, pieces="auto"):
         self.env, self.actor = env, actor
         self.actors = list(actor) if isinstance(actor, (list, tuple)) else [actor]
         self._h = C.c_void_p()
+        if len(getattr(env, "specs", ())) > 1 and not self._mixed:
+            raise capi.TfemError("the env batch holds several families (%d): step it with MixedHostRollout"
+                                 % len(env.specs))
         for a in self.actors:                  # the actor ABI cannot tell its node count or device: checked here
             if getattr(a, "nodes", None) != env.N or getattr(a, "device", None) != env.device:
                 raise ValueError("every actor must be a BatchedActor of the env's %d nodes on %s (got %s nodes on %s)"
@@ -235,12 +249,11 @@ class HostRollout:
         :meth:`step_agents`."""
         if len(self.actors) > 1:
             raise ValueError("this rollout runs %d actors: step it with step_agents" % len(self.actors))
-        env, act = self.env, self.actors[0]
+        act = self.actors[0]
         io = _IO()
         self._parent(io, state_host, x_p_host, A_p_host, n_pf_host)
         self._child(io, out_host, coin_host)
-        with torch.cuda.device(env.device):
-            _check(_lib.trollout_step_host(self._h, env.B, C.byref(io), act.mu, act.theta, act.sigma, act.seed))
+        self._step_call(state_host, io, act.mu, act.theta, act.sigma, act.seed)
         act.update_num += 1
         return out_host
 
@@ -263,8 +276,71 @@ class HostRollout:
         theta = (C.c_float * K)(*[a.theta for a in acts])
         sigma = (C.c_float * K)(*[a.sigma for a in acts])
         seed = (C.c_uint64 * K)(*[a.seed for a in acts])
-        with torch.cuda.device(self.env.device):
-            _check(_lib.trollout_step_agents_host(self._h, self.env.B, C.byref(io), mu, theta, sigma, seed))
+        self._step_call(state_host, io, mu, theta, sigma, seed)
         for a in acts:
             a.update_num += 1
         return outs_host
+
+    def _step_call(self, state_host, io, *noise):
+        """the C call of one step: an ``_IO`` goes to trollout_step_host, an ``_AgentsIO`` to trollout_step_agents_host"""
+        fn = _lib.trollout_step_agents_host if isinstance(io, _AgentsIO) else _lib.trollout_step_host
+        with torch.cuda.device(self.env.device):
+            _check(fn(self._h, self.env.B, C.byref(io), *noise))
+
+
+class MixedHostRollout(HostRollout):
+    """:class:`HostRollout` over a ``batched_env.MixedTrussEnv``: every environment has its own family (the training
+    driver draws a shape and a truss type per episode, ``train/code/master_DDPG_truss2D_MO.py:787-815``), and one call
+    steps them all -- one env-step launch per piece and agent over every family.  The host state tuple carries the
+    family ids as ``state_host["family"]`` (uint8 [B], indices into ``env.specs``), which :meth:`alloc_host` adds.
+    ``step`` / ``step_agents`` copy the parent's ids into every output set that has a ``"family"`` tensor of its own,
+    so a child can be fed back as the next parent.  Environment b of a child is bit for bit what a ``HostRollout``
+    over a batch of family ``env.specs[family[b]]`` gives with the same pieces.  The ids are read when a captured step
+    is replayed: they may be rewritten in the same buffer between steps.  An id out of range sets
+    ``capi.STATUS_BAD_FAMILY`` in that environment's ``status``; its other outputs are then unspecified."""
+
+    _mixed = True
+
+    def __init__(self, env, actor, pieces="auto"):
+        from .batched_env import MixedTrussEnv
+        if not isinstance(env, MixedTrussEnv):
+            raise ValueError("MixedHostRollout steps a batched_env.MixedTrussEnv (got %s): use HostRollout"
+                             % type(env).__name__)
+        super().__init__(env, actor, pieces)
+
+    def alloc_host(self, compact: bool = True, raw_tables: bool = True):
+        """:meth:`HostRollout.alloc_host` plus ``"family"``: pinned uint8 [B]"""
+        h = super().alloc_host(compact, raw_tables)
+        h["family"] = torch.empty(self.env.B, dtype=torch.uint8).pin_memory()
+        return h
+
+    def step(self, state_host: dict, coin_host, x_p_host: torch.Tensor, A_p_host: torch.Tensor, out_host: dict,
+             n_pf_host=None):
+        """:meth:`HostRollout.step`; ``state_host["family"]`` is required"""
+        super().step(state_host, coin_host, x_p_host, A_p_host, out_host, n_pf_host)
+        self._pass_family(state_host, [out_host])
+        return out_host
+
+    def step_agents(self, state_host: dict, coins_host, x_p_host: torch.Tensor, A_p_host: torch.Tensor, outs_host,
+                    n_pf_host=None):
+        """:meth:`HostRollout.step_agents`; ``state_host["family"]`` is required"""
+        super().step_agents(state_host, coins_host, x_p_host, A_p_host, outs_host, n_pf_host)
+        self._pass_family(state_host, outs_host)
+        return outs_host
+
+    def _step_call(self, state_host, io, *noise):
+        fam = state_host.get("family")
+        if fam is None:
+            raise ValueError("state_host lacks 'family': the uint8 [B] family ids (MixedHostRollout.alloc_host)")
+        fam = self._chk(fam, (self.env.B,), torch.uint8)
+        fn = _lib.trollout_step_agents_host_mixed if isinstance(io, _AgentsIO) else _lib.trollout_step_host_mixed
+        with torch.cuda.device(self.env.device):
+            _check(fn(self._h, self.env.B, fam, C.byref(io), *noise))
+
+    @staticmethod
+    def _pass_family(state_host, outs_host):
+        """every child has its parent's families"""
+        fam = state_host["family"]
+        for o in outs_host:
+            if "family" in o and o["family"].data_ptr() != fam.data_ptr():
+                o["family"].copy_(fam)
