@@ -99,8 +99,9 @@ pareto_kernel(const float* __restrict__ x_p, const float* __restrict__ A_p, cons
   }
   __syncthreads();
   // the reference's stack-and-reshape scramble (x14b[b,n,h] = pooled[b,(n*200+h)/N]) is applied by the fused
-  // kernel's operand generator, so only the pooled embedding is materialised
-  if (tid < LD) pooled_out[(size_t)b * LD + tid] = (tid < HID) ? ((red[tid] + red[LD + tid]) + (red[2 * LD + tid] + red[3 * LD + tid])) : 0.f;
+  // kernel's operand generator, so only the pooled embedding is materialised -- times XPRE, like every mix operand
+  // (tactor_tc.cuh)
+  if (tid < LD) pooled_out[(size_t)b * LD + tid] = (tid < HID) ? ((red[tid] + red[LD + tid]) + (red[2 * LD + tid] + red[3 * LD + tid])) * tc::XPRE : 0.f;
 }
 // Small fronts (P <= PSMALL; the reset-time graph has P = 1): one thread per feature column, everything recomputed in
 // registers -- no barrier-separated stages, a few registers, many CTAs per SM (the tiled kernel above needs 3 barriers and
@@ -145,7 +146,7 @@ pareto_small_kernel(const float* __restrict__ x_p, const float* __restrict__ A_p
       }
     }
   }
-  if (tid < LD) pooled_out[(size_t)b * LD + tid] = (tid < HID) ? sum : 0.f;
+  if (tid < LD) pooled_out[(size_t)b * LD + tid] = (tid < HID) ? sum * tc::XPRE : 0.f;
 }
 
 // P == 1 (the reset-time graph, truss2D_ENV.py:348-351): pooled[h] = relu(A_p x_p W14[:,h] + b[h]) is five FMAs per
@@ -169,7 +170,7 @@ pareto_p1_kernel(const float* __restrict__ x_p, const float* __restrict__ A_p, c
     const float t0 = fmaf(x.w, w3, fmaf(x.z, w2, fmaf(x.y, w1, x.x * w0)));   // same operation order as the general kernels
     float sum = 0.f;
     if (valid > 0) sum = fmaxf(fmaf(a, t0, 0.f) + bias, 0.f);
-    pooled_out[(size_t)b * LD + tid] = (tid < HID) ? sum : 0.f;
+    pooled_out[(size_t)b * LD + tid] = (tid < HID) ? sum * tc::XPRE : 0.f;
   }
 }
 
@@ -289,7 +290,7 @@ pareto_tri_kernel(const float* __restrict__ x_p, const float* __restrict__ A_p, 
 #pragma unroll
   for (int k = 0; k < NC; ++k) {
     const int h = lane + 32 * k;
-    if (h < LD) pooled_out[(size_t)b * LD + h] = (h < HID) ? ((sum[0][k] + sum[1][k]) + (sum[2][k] + sum[3][k])) : 0.f;
+    if (h < LD) pooled_out[(size_t)b * LD + h] = (h < HID) ? ((sum[0][k] + sum[1][k]) + (sum[2][k] + sum[3][k])) * tc::XPRE : 0.f;
   }
 }
 
@@ -360,8 +361,8 @@ __global__ void __launch_bounds__(256) pack_wmax_kernel(PackArgs a) {
     for (int w = 1; w < 8; ++w) m = fmaxf(m, red[w]);
     a.wmax[l] = m;
     const float inv = 1.f / pow2_scale_dev(m);
-    if (l >= 4 && l <= 10) a.wscale_inv[l - 4] = inv;
-    if (l < 3) a.wscale_inv[tc::fused::NGEMM + l] = inv;
+    if (l >= 4 && l <= 10) a.wscale_inv[l - 4] = (l >= 9) ? inv / tc::HPRE : inv * (tc::HPRE / tc::XPRE);   // like upload_weights
+    if (l < 3) a.wscale_inv[tactor::tc::fused::NGEMM + l] = inv * tc::XPRE;
   }
 }
 
@@ -618,6 +619,13 @@ cudaError_t upload_weights(tactor_handle_s* h, const tactor_weights* w) {
         pack(we(2 * t + 8, f0 + 8), we(2 * t + 9, f0 + 8), hi[3], lo[3]);
       }
   }
+  // the mix operands are carried times a power of two (tactor_tc.cuh): layer 1 puts XPRE in (its outputs are X of the
+  // first four mixes; the pooled Pareto embedding, X of the fifth, carries it from the Pareto kernels), the layer-2
+  // epilogues turn it into HPRE on the five-way sum H, and the epilogues of the two layer-3 GEMMs, whose X is H, take it out
+  for (int l = 0; l < 3; ++l) wscale_inv[tactor::tc::fused::NGEMM + l] *= tactor::tc::XPRE;
+  for (int g = 0; g < 5; ++g) wscale_inv[g] *= tactor::tc::HPRE / tactor::tc::XPRE;
+  wscale_inv[5] /= tactor::tc::HPRE;
+  wscale_inv[6] /= tactor::tc::HPRE;
   if (e == cudaSuccess && !h->d_w1frag) e = cudaMalloc(&h->d_w1frag, frag.size() * 4);
   if (e == cudaSuccess) e = cudaMemcpy(h->d_w1frag, frag.data(), frag.size() * 4, cudaMemcpyHostToDevice);
   // the scales live in device memory: a CUDA graph that captured a forward of this handle (trollout_step_host) reads the

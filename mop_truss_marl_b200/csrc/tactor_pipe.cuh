@@ -28,7 +28,7 @@
 //                            shared memory, accumulator g&1 of two (TMEM columns [0,208) and [256,464))
 //   epilogue    NEPIW warps  tcgen05.ld the finished accumulator while the next GEMM is already running (one warp per
 //                            32-row group): relu(D / S) -> H (+)= (g <= 4), or the sigmoid heads gcn_l4_1/2 (g = 5, 6);
-//                            the bias is row 200 of the W image (A's column 200 is the constant 1)
+//                            the bias is row 200 of the W image (A's column 200 is the constant XPRE or HPRE, tactor_tc.cuh)
 //
 // TMEM map (512 columns): [0,208) acc0 | [208,256) A stages hi (6 x 8 columns of packed pairs) | [256,464) acc1
 //                         | [464,512) A stages lo
@@ -429,7 +429,7 @@ actor_pipe_kernel(const __grid_constant__ Params P) {
           // X fragments of the chunk: xb[16-row block][8-feature half][hi | lo][rows 2t.. | rows 8 + 2t..]
           uint32_t xb[2][2][2][2];
           if (g <= 3) {
-            // layer 1 on the tensor core: X^T [16 features x 8 rows] = relu([W1k ; b1k]^T . [Z, 1]^T / S) for the four
+            // layer 1 on the tensor core: X^T [16 features x 8 rows] = relu([W1k ; b1k]^T . [Z, 1]^T) XPRE / S for the four
             // 8-row blocks; accumulator element (feature g8 (+8), rows 2t, 2t+1) is exactly what the mix needs as B fragment
             const uint4 wh = *reinterpret_cast<const uint4*>(w1f + ((c * 2 + 0) * 32 + lane) * 4);
             const uint4 wl = *reinterpret_cast<const uint4*>(w1f + ((c * 2 + 1) * 32 + lane) * 4);
@@ -484,9 +484,9 @@ actor_pipe_kernel(const __grid_constant__ Params P) {
                 const int kr = kr_of(mt, kb);
                 hmma_split(y, afr[mt][kb][0], afr[mt][kb][1], xb[kr][nt][0], xb[kr][nt][1]);
               }
-              // column 200 of A is the constant 1 that multiplies the bias row of the W image (columns 201..207 are zero
-              // because X is)
-              if (k0 + 8 * nt == KH && t4 == 0) { y[0] = 1.f; y[2] = 1.f; }
+              // column 200 of A is the constant that multiplies the bias row of the W image: the factor every entry of
+              // Y carries, XPRE in layer 2, HPRE in layer 3 (columns 201..207 are zero because X is)
+              if (k0 + 8 * nt == KH && t4 == 0) { y[0] = (g <= 4) ? XPRE : HPRE; y[2] = y[0]; }
               split2(y[0], y[1], oh[mt][2 * nt], ol[mt][2 * nt]);              // lane g8,     column 4 nt + t4
               split2(y[2], y[3], oh[mt][2 * nt + 1], ol[mt][2 * nt + 1]);      // lane g8 + 8, column 4 nt + t4
             }
@@ -542,7 +542,7 @@ actor_pipe_kernel(const __grid_constant__ Params P) {
         const long long prof_t1 = PROF_NOW();
         if (it == 1) PROF_TRACE(4608 + (q * 7 + g) * 2, prof_t1);
         const uint32_t tacc = tmem_base + ((uint32_t)(32 * q) << 16) + (uint32_t)(b ? TM_ACC1 : 0);
-        const float wsi = __ldg(P.wscale_inv + g);             // undoes the power-of-two scale folded into W (exact)
+        const float wsi = __ldg(P.wscale_inv + g);             // undoes the power-of-two scale folded into W and the operand factors (exact)
         float* hrow = H + r * LDH;
         const float* wh = Wh + (g >= 5 ? g - 5 : 0) * 201 * 4; // only used for g >= 5
         float u0 = 0.f, u1 = 0.f, u2 = 0.f;

@@ -2,7 +2,7 @@
 //
 //   * a CTA owns 128 rows (8 environments of 16 nodes / 4 of 32) and all 208 (padded) output columns
 //   * X.W on the 5th-gen tensor cores: tcgen05.mma kind::f16, M=128 N=208 K=16 per instruction, fp32 accumulators in TMEM
-//   * float32-equivalent accuracy by the fp16 hi/lo split (three MMAs per k-step into the same accumulator)
+//   * float32-like accuracy inside the fp16 window by the hi/lo split (three MMAs per k-step into the same accumulator)
 //   * the B operand (W) sits in shared memory in the canonical no-swizzle K-major layout (8-row x 16-byte core
 //     matrices): W is pre-scaled, pre-split and pre-laid-out on the host so a K-chunk is ONE cp.async.bulk (TMA 1-D
 //     bulk copy, completion on an mbarrier)
@@ -18,10 +18,20 @@ namespace tc {
 
 // Operand precision of the split product: x = hi + lo with hi = fp16(x), lo = fp16(x - hi), X.W ~= Xhi.Whi + Xhi.Wlo +
 // Xlo.Whi on tcgen05.mma kind::f16 (K = 16 per instruction).  fp16 carries the same 11-bit significand as tf32, so the
-// result is float32-equivalent like 3xTF32 (measured <= 6e-6 on the sigmoid outputs against the float64 oracle) at half
+// result is float32-like as 3xTF32 is (measured <= 6e-6 on the sigmoid outputs against the float64 oracle) at half
 // the operand bytes and twice the tensor rate (3xTF32 on kind::tf32 was the first formulation of this kernel: 0.388 ms
 // against 0.382 ms per forward with everything else equal).  What fp16 lacks is range: W is pre-scaled by a power of
-// two per layer (undone exactly in the epilogue) and |A.X| > 65504 is reported through tactor_status.
+// two per layer (undone exactly in the epilogue) and an operand beyond 65504 is reported through tactor_status.  The
+// split is float32-like only while the operand is at least 2^-3: below that lo = fp16(x - hi) is an fp16 subnormal, so
+// the operand keeps an absolute error of 2^-25 instead of a relative one of 2^-22.  The activations are not scaled by
+// the weights' power of two, and a trained actor has most of its mix operands below 2^-3 (DESIGN.md section 3.3): so
+// the mix operands X and Y = A.X are carried times a power of two -- XPRE in the five mixes of layer 2 (layer 1's 1/S and
+// the pooled Pareto embedding put the factor in), HPRE in the two of layer 3, whose X is the five-way sum H (the layer-2
+// epilogues write H times HPRE); the constant bias column of Y carries the factor of its GEMM and the epilogue's 1/S
+// takes it out, all exact.  The window of the true activations is [2^-9, 65504 / 64] in layer 2 and [2^-6, 65504 / 8]
+// for H, which is larger (a sum of five terms).
+constexpr float XPRE = 64.f;
+constexpr float HPRE = 8.f;
 constexpr int TCM = 128;             // rows per CTA
 constexpr int TCN = 208;             // padded output columns (UMMA N, multiple of 16)
 constexpr int KCH = 16;              // K elements per chunk (one MMA k-step)
