@@ -11,6 +11,7 @@ import os
 import numpy as np
 import pytest
 
+from mop_truss_marl_b200.families import SYM_NONE, TRAIN_FAMILIES
 from util import FAMILY_NAMES, F32_FIELDS, FP64_TOL, assert_f32_close, load_golden, nrm
 
 pytestmark = pytest.mark.gpu
@@ -108,10 +109,10 @@ def test_transitions_vs_golden(envmod, name):
                     tag="%s tr[%d] mode %d" % (name, i, g["tr_mode"][i]))
 
 
-@pytest.mark.parametrize("name", FAMILY_NAMES + ("train0_roof", "train1_bridge", "train4_roof"))
+@pytest.mark.parametrize("name", FAMILY_NAMES + TRAIN_FAMILIES)
 def test_random_walk_vs_oracle(envmod, name):
-    """every environment feeds its own state back; the oracle follows each one (the four test/ families and three of the
-    6 x 2 train/code shapes: 12 nodes, mixed spans, no symmetry step)"""
+    """every environment feeds its own state back; the oracle follows each one (the four test/ families and the ten
+    6 x 2 train/code families: 12 nodes, mixed spans, no symmetry step)"""
     from oracle.truss_oracle import TrussOracle
     o = TrussOracle(name)
     B = 48 if o.mesh.N <= 16 else 16
@@ -139,7 +140,7 @@ def test_random_walk_vs_oracle(envmod, name):
             assert nrm(cpu(env.point64[i]), want["point64"]) <= FP64_TOL
 
 
-@pytest.mark.parametrize("name", FAMILY_NAMES)
+@pytest.mark.parametrize("name", FAMILY_NAMES + TRAIN_FAMILIES)
 def test_adversarial_transition_vs_oracle(envmod, name):
     """ties, exact 0/1, out-of-range, inf / NaN geometry actions and absurd stale move ranges: the
     post-transition heights (float64 bits + weak flags), sections, clipped actions and new move range must be
@@ -209,7 +210,7 @@ def test_step_host_equals_step(envmod, name):
     assert np.array_equal(mr, cpu(env.move_range)) and np.array_equal(hg, cpu(a_geo)) and np.array_equal(ht, cpu(a_topo))
 
 
-@pytest.mark.parametrize("name", ["small_roof", "large_bridge"])
+@pytest.mark.parametrize("name", ("small_roof", "large_bridge") + TRAIN_FAMILIES)
 def test_solve_only_vs_oracle(envmod, name):
     from oracle.truss_oracle import TrussOracle
     o = TrussOracle(name)
@@ -272,7 +273,8 @@ def test_degenerate_geometry_sets_status(envmod):
         o.solve_only(y[1], sec[1])
 
 
-@pytest.mark.parametrize("name,B", [("small_bridge", 4096), ("small_roof", 16384), ("large_bridge", 8192)])
+@pytest.mark.parametrize("name,B", [("small_bridge", 4096), ("small_roof", 16384), ("large_bridge", 8192),
+                                    ("train0_roof", 16384), ("train3_bridge", 16384)])
 def test_full_size_properties(envmod, name, B):
     """BASELINE.json batch sizes: size-independent properties of the solved batch"""
     env = make_env(envmod, name, B)
@@ -297,12 +299,14 @@ def test_full_size_properties(envmod, name, B):
     rx = sum(env.reactions[:, tnsc[i, a] - 1 - ndof] for i, a in res_ids if a == 0)
     assert float(((ry + P.sum()).abs() / P.sum().abs()).max()) <= 1e-9
     assert float((rx.abs() / P.sum().abs()).max()) <= 1e-9
-    # (3) the symmetry pass leaves mirror-symmetric geometry and sections -> mirror-symmetric deflections
+    # (3) the symmetry pass leaves mirror-symmetric geometry and sections -> mirror-symmetric deflections (the training
+    # shapes have mixed spans and no symmetry pass)
     nx = N // 2
     y = env.nN_x_n[:, :, 1]
-    assert torch.equal(y[:, nx:], y[:, nx:].flip(1)) and torch.equal(y[:, :nx], y[:, :nx].flip(1))
-    dy = env.nN_x_n[:, :, 10].double()
-    assert float(((dy[:, :nx] - dy[:, :nx].flip(1)).abs().max() / dy.abs().max())) <= 1e-6
+    if env.spec.symmetry != SYM_NONE:
+        assert torch.equal(y[:, nx:], y[:, nx:].flip(1)) and torch.equal(y[:, :nx], y[:, :nx].flip(1))
+        dy = env.nN_x_n[:, :, 10].double()
+        assert float(((dy[:, :nx] - dy[:, :nx].flip(1)).abs().max() / dy.abs().max())) <= 1e-6
     # (4) re-solving the emitted geometry reproduces d bit-exactly (idempotence of the FEM stage)
     sec = env.nN_x_e[:, :, 0].to(torch.int32).contiguous()
     again = env.solve_only(y.double().contiguous(), sec)
