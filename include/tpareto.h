@@ -22,13 +22,20 @@ extern "C" {
 const char* tpareto_last_error(void);
 
 /* points    [B,P,4] float32 device: obj1, obj2, con1, con2 per point (the `point` tensors of tfem_step)
- * counts    [B] int32 device, valid points per environment (NULL = all P)
+ * counts    [B] int32 device, valid points per environment, clamped to 0..P (0 or below: no point, as if none were
+ *           feasible; NULL = all P)
  * ref_point host double[2] (NULL = {1, 1})
  * front_idx [B,P] int32: indices of the front members in the reference's order (obj1 ascending), -1 padded
  * front_len [B]   int32: 0 when no point is feasible (the reference raises IndexError there)
  * stats     [B,5] double: max_distance, dis_distance, p_norm_inv_cd, sum_distance, std_cd (simple_cull's tuple)
  * hv        [B]   double: union_rectangles_fastest(front, ref_point)
- * Any output may be NULL.  Runs on the current device, on `stream`. */
+ * Any output may be NULL; the others are written as without it.  Runs on the current device, on `stream`.
+ * Non-finite points follow the reference's comparisons: a NaN constraint is feasible (NaN > 1 is false), a NaN objective
+ * is never dominated and dominates nothing, NaN tuples are never duplicates.  The list puts a NaN after every number (NumPy's
+ * sort convention) in obj1 and, within equal obj1, in the obj2-descending key, then orders by index; the reference's own
+ * order there is whatever Python's sort makes of inconsistent comparisons.  Statistics and hypervolume propagate NaN like
+ * NumPy (max_distance of a list holding a NaN objective is NaN, not the largest number).
+ * Refused (nothing written): P outside 1..TPARETO_MAX_POINTS (TFEM_ERR_ARG), points not 16-byte aligned (TFEM_ERR_ALIGN). */
 int tpareto_front_hv(int B, int P, const float* points, const int32_t* counts, const double* ref_point,
                      int32_t* front_idx, int32_t* front_len, double* stats, double* hv, void* stream);
 
@@ -37,8 +44,11 @@ int tpareto_front_hv(int B, int P, const float* points, const int32_t* counts, c
  * and keep the order of the draw; statistics and hypervolume are those of the thinned list.  The reference draws with
  * random.sample; here the draw is an input, so the result is deterministic:
  * thin_pick [B, max_front - 2] int32 device = what random.sample(range(F - 2), max_front - 2) returned for that environment
- * (positions in the crowd-sorted list; rows of environments whose front has <= max_front members are not read).
- * tpareto_front_hv (no draw) leaves larger fronts unthinned.  3 <= max_front <= 64. */
+ * (positions in the crowd-sorted list, clamped to 0..F - 3; rows of environments whose front has <= max_front members are
+ * not read and may hold anything).  A NaN crowd distance sorts after every number.  The crowd distances round each product
+ * as NumPy does, so exact ties (the mirrored gaps of a front symmetric in obj1 <-> obj2) stay ties and the stable order holds.
+ * tpareto_front_hv (no draw) leaves larger fronts unthinned.  3 <= max_front <= 64 (the training driver's MAX_FRONT is 20,
+ * the test runs' 50); outside it, or with thin_pick NULL, the call returns TFEM_ERR_ARG and writes nothing. */
 int tpareto_front_hv_thin(int B, int P, const float* points, const int32_t* counts, const double* ref_point,
                           const int32_t* thin_pick, int max_front, int32_t* front_idx, int32_t* front_len, double* stats,
                           double* hv, void* stream);

@@ -21,13 +21,35 @@ __device__ __forceinline__ double warp_sum(double v) {
   for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
   return v;
 }
+// min / max that propagate NaN like np.minimum / np.maximum / ndarray.max (fmin / fmax drop it); equal to fmin / fmax on
+// numbers up to the sign of a zero result, which no output of the kernel depends on
+__device__ __forceinline__ double nan_min(double a, double b) { return (a < b || a != a) ? a : b; }
+__device__ __forceinline__ double nan_max(double a, double b) { return (a > b || a != a) ? a : b; }
 __device__ __forceinline__ double warp_max(double v) {
-  for (int o = 16; o; o >>= 1) v = fmax(v, __shfl_xor_sync(0xffffffffu, v, o));
+  for (int o = 16; o; o >>= 1) v = nan_max(v, __shfl_xor_sync(0xffffffffu, v, o));
   return v;
 }
 __device__ __forceinline__ double warp_min(double v) {
-  for (int o = 16; o; o >>= 1) v = fmin(v, __shfl_xor_sync(0xffffffffu, v, o));
+  for (int o = 16; o; o >>= 1) v = nan_min(v, __shfl_xor_sync(0xffffffffu, v, o));
   return v;
+}
+// Sort keys with NumPy's NaN convention: a NaN comes after every number, NaNs tie with each other.  Each returns whether
+// key a (at index j) goes before key b (at index k), ties by index, so ranks by counting are a permutation for any input;
+// a comparison that is not a total order would give two members one rank and leave a slot unwritten.
+__device__ __forceinline__ bool key_tie(bool an, bool bn, double a, double b) { return an == bn && (an || a == b); }
+__device__ __forceinline__ bool asc_before(double a, int j, double b, int k) {
+  const bool an = a != a, bn = b != b;
+  return key_tie(an, bn, a, b) ? j < k : (an != bn ? bn : a < b);
+}
+__device__ __forceinline__ bool desc_before(double a, int j, double b, int k) {
+  const bool an = a != a, bn = b != b;
+  return key_tie(an, bn, a, b) ? j < k : (an != bn ? bn : a > b);
+}
+// the front's list order (utils.py:57): obj1 ascending, then obj2 descending, then index
+__device__ __forceinline__ bool list_before(float4 q, int j, float4 p, int i) {
+  const bool qn = q.x != q.x, pn = p.x != p.x;
+  if (!key_tie(qn, pn, q.x, p.x)) return qn != pn ? pn : q.x < p.x;
+  return desc_before(q.y, j, p.y, i);
 }
 __device__ __forceinline__ int warp_isum(int v) {
   for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
@@ -78,7 +100,7 @@ pareto_front_hv_kernel(int B, int P, const float* __restrict__ points, const int
       for (int j = 0; j < n; ++j) {
         if (!member[warp][j] || j == i) continue;
         const float4 q = pt[j];
-        if (q.x < p.x || (q.x == p.x && (q.y > p.y || (q.y == p.y && j < i)))) ++rank;
+        if (list_before(q, j, p, i)) ++rank;
       }
       order[warp][rank] = i;
       fx[warp][rank] = (double)p.x;
@@ -93,8 +115,10 @@ pareto_front_hv_kernel(int B, int P, const float* __restrict__ points, const int
       int* sorted = reinterpret_cast<int*>(scratch[warp] + MAXP * 8);        // [MAXP] interior members by crowd distance
       for (int k = lane; k < F; k += 32) {
         auto dist = [&](int a) {
+          // each product rounded like NumPy's: a contracted fma(ax, ax, ay * ay) can split a tie the stable sort below
+          // must keep, e.g. the mirrored gaps of a front symmetric in obj1 <-> obj2
           const double ax = fx[warp][a] - fx[warp][a + 1], ay = fy[warp][a] - fy[warp][a + 1];
-          return sqrt(ax * ax + ay * ay);
+          return sqrt(__dadd_rn(__dmul_rn(ax, ax), __dmul_rn(ay, ay)));
         };
         crowd[k] = (k == 0) ? dist(0) : (k == F - 1) ? dist(F - 2) : dist(k - 1) + dist(k);
       }
@@ -102,7 +126,7 @@ pareto_front_hv_kernel(int B, int P, const float* __restrict__ points, const int
       for (int k = 1 + lane; k < F - 1; k += 32) {
         int r = 0;
         const double ck = crowd[k];
-        for (int j = 1; j < F - 1; ++j) r += (crowd[j] > ck || (crowd[j] == ck && j < k)) ? 1 : 0;
+        for (int j = 1; j < F - 1; ++j) r += desc_before(crowd[j], j, ck, k) ? 1 : 0;
         sorted[r] = k;
       }
       __syncwarp();
@@ -146,7 +170,7 @@ pareto_front_hv_kernel(int B, int P, const float* __restrict__ points, const int
         const double ax = fx[warp][k] - fx[warp][k + 1], ay = fy[warp][k] - fy[warp][k + 1];
         d[s] = sqrt(ax * ax + ay * ay);
         dsum += d[s];
-        dmax = fmax(dmax, d[s]);
+        dmax = nan_max(dmax, d[s]);
       }
     }
     dsum = warp_sum(dsum);
@@ -171,7 +195,7 @@ pareto_front_hv_kernel(int B, int P, const float* __restrict__ points, const int
         if (k + 2 < F) {
           c[s] = fabs(fx[warp][k] - fx[warp][k + 2]) + fabs(fy[warp][k] - fy[warp][k + 2]);
           csum += c[s];
-          cmax = fmax(cmax, c[s]);
+          cmax = nan_max(cmax, c[s]);
         }
       }
       csum = warp_sum(csum);
@@ -207,7 +231,7 @@ pareto_front_hv_kernel(int B, int P, const float* __restrict__ points, const int
         for (int k = lane; k < F; k += 32) {
           int r = 0;
           const double xk = fx[warp][k];
-          for (int j = 0; j < F; ++j) r += (fx[warp][j] < xk || (fx[warp][j] == xk && j < k)) ? 1 : 0;
+          for (int j = 0; j < F; ++j) r += asc_before(fx[warp][j], j, xk, k) ? 1 : 0;
           tx[r] = xk; ty[r] = fy[warp][k];
         }
         __syncwarp();
@@ -216,11 +240,11 @@ pareto_front_hv_kernel(int B, int P, const float* __restrict__ points, const int
       double area = 0.0, minx = INFINITY, miny = INFINITY;
       for (int k = lane; k < F; k += 32) {
         double h = 0.0;
-        for (int j = 0; j <= k; ++j) h = fmax(h, 1.0 - fmin(sy[j], 1.0));
-        const double x0 = fmin(sx[k], 1.0), x1 = (k + 1 < F) ? fmin(sx[k + 1], 1.0) : 1.0;
+        for (int j = 0; j <= k; ++j) h = nan_max(h, 1.0 - nan_min(sy[j], 1.0));
+        const double x0 = nan_min(sx[k], 1.0), x1 = (k + 1 < F) ? nan_min(sx[k + 1], 1.0) : 1.0;
         area += (x1 - x0) * h;
-        minx = fmin(minx, sx[k]);
-        miny = fmin(miny, sy[k]);
+        minx = nan_min(minx, sx[k]);
+        miny = nan_min(miny, sy[k]);
       }
       area = warp_sum(area);
       minx = warp_min(minx);

@@ -15,8 +15,8 @@ Parity status: **pinned** -- ``tests/test_pareto_oracle.py`` runs both functions
 ``utils.py`` on random point sets (float64 inputs, so both sides compute in float64) and against
 ``tests/golden/pareto.npz`` recorded from the reference by ``tests/golden/make_golden_pareto.py``.  (With the driver's
 ``np.float32`` points the reference's scalar arithmetic runs in float32; the statistics then agree to ~1e-6.)
-The reference samples the front down with ``random.sample`` when it holds more than MAX_FRONT = 50 points (:120-142): the
-first and the last member stay, 48 of the others are drawn from the list sorted by crowd distance (descending, stable)
+The reference samples the front down with ``random.sample`` when it holds more than MAX_FRONT points (:120-142; 50 in the
+test runs, 20 in ``train/code``): the first and the last member stay, MAX_FRONT - 2 of the others are drawn from the list sorted by crowd distance (descending, stable)
 and keep the ORDER of the draw.  ``front_stats(points, thin_pick=...)`` reproduces it for an explicit draw: ``thin_pick`` is
 what ``random.sample(range(F - 2), MAX_FRONT - 2)`` returned (positions in that sorted list); the pinning test feeds the same
 positions to the reference by patching ``utils.random.sample``.
@@ -26,6 +26,13 @@ from __future__ import annotations
 import numpy as np
 
 MAX_FRONT = 50
+
+
+def nan_last(v):
+    """sort key of a number with NumPy's NaN convention: after every number, NaNs tied.  The reference sorts with Python's
+    comparisons, which are not an order once a NaN is present, so its result there depends on the input order: a known
+    divergence (DESIGN.md section 4)."""
+    return (1, 0.0) if v != v else (0, v)
 
 
 def front_indices(points):
@@ -42,7 +49,7 @@ def front_indices(points):
             continue
         seen.add(pts[i])
         front.append(i)
-    front.sort(key=lambda i: (pts[i][0], -pts[i][1], i))                           # sorted by obj1 (:57); ties: see tests
+    front.sort(key=lambda i: (nan_last(pts[i][0]), nan_last(-pts[i][1]), i))       # sorted by obj1 (:57); ties: see tests
     return front
 
 
@@ -53,7 +60,7 @@ def thin_order(f, thin_pick, max_front=MAX_FRONT):
     crowd = np.empty(F)
     crowd[0], crowd[-1] = d[0], d[-1]
     crowd[1:-1] = d[:-1] + d[1:]
-    interior = sorted(range(1, F - 1), key=lambda i: crowd[i], reverse=True)      # stable: ties keep the obj1 order
+    interior = sorted(range(1, F - 1), key=lambda i: nan_last(-crowd[i]))         # descending, stable: ties keep the obj1 order
     pick = [int(k) for k in thin_pick]
     if len(pick) != max_front - 2 or len(set(pick)) != len(pick) or min(pick) < 0 or max(pick) >= F - 2:
         raise ValueError("thin_pick must hold %d distinct positions below %d" % (max_front - 2, F - 2))
