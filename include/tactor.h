@@ -46,8 +46,10 @@ typedef struct tactor_inputs {
 
 const char* tactor_last_error(void);
 
-/* nodes = N: 16 or 32 (the test/ families), or 12 (the 6 x 2 shapes of train/code: every tensor keeps its [B,12,...] shape,
- * the graphs are padded to 16 nodes internally); max_batch = largest B of any later call (workspace is allocated once). */
+/* nodes = N = 2 num_x: any even count 6..32 (num_x 3..16).  16 and 32 (the test/ families) run natively; a smaller count
+ * (12: the 6 x 2 shapes of train/code) keeps its [B,N,...] tensors, which are padded internally to the 16-node build
+ * (N <= 16) or the 32-node build (N > 16).  Other counts return TFEM_ERR_UNSUPPORTED before any device call.
+ * max_batch = largest B of any later call (workspace is allocated once). */
 int tactor_create(const tactor_weights* w, int nodes, int max_batch, int device, tactor_handle_t* out);
 int tactor_destroy(tactor_handle_t h);
 

@@ -140,7 +140,11 @@ const char* tfem_last_error(void);
 
 /* gen_model(...) + Game_research04(...): builds the mesh, supports, loads, DOF map, symmetry tables
  * and the initial objectives for one family on CUDA device `device`.  device < 0 gives a tables-only
- * handle (tfem_get_dims / tfem_get_table work, every compute entry point returns TFEM_ERR_CUDA). */
+ * handle (tfem_get_dims / tfem_get_table work, every compute entry point returns TFEM_ERR_CUDA).
+ * Families: 3 <= num_x <= TFEM_MAX_NX (one kernel lane per node; num_x = 2 leaves no free bottom node to carry
+ * a load) with TFEM_SYM_NONE, the ENV of train/code; the small and large symmetry conventions only for
+ * num_x 6, 8 and 16, the chord lengths whose truss2D_ENV.py carries their index lists.  Anything else
+ * returns TFEM_ERR_UNSUPPORTED, and tfem_last_error names the limit. */
 int tfem_create(const tfem_family_desc* desc, int device, tfem_handle_t* out);
 int tfem_destroy(tfem_handle_t h);
 int tfem_get_dims(tfem_handle_t h, tfem_dims* out);

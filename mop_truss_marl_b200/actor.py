@@ -58,7 +58,8 @@ def selftest_tmem_layout(device: int = 0) -> None:
 
 
 class BatchedActor:
-    """One agent's actor for up to ``max_batch`` environments of ``nodes`` nodes (12, 16 or 32) on ``device``.
+    """One agent's actor for up to ``max_batch`` environments of ``nodes`` nodes (2 num_x: any even count
+    from 6 to 32) on ``device``.
 
     ``weights``: ``{layer name: (kernel [in,out], bias [out])}`` as returned by
     :func:`mop_truss_marl_b200.tf_checkpoint.load_actor_weights`."""

@@ -12,9 +12,11 @@
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
+#include <array>
 #include <atomic>
 #include <new>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "../../include/tactor.h"
@@ -424,14 +426,14 @@ __global__ void __launch_bounds__(32) pack_w1frag_kernel(PackArgs a) {
   pack(we(2 * t + 8, f0 + 8), we(2 * t + 9, f0 + 8), hi[3], lo[3]);
 }
 
-// 12-node graphs (the 6 x 2 shapes of train/code) run on the 16-node build: every environment is padded to 16 rows with zero
-// features and zero adjacency rows / columns (a padded node neither sends nor receives), the kernel divides the pooled
-// scramble by the real node count and writes only the real rows.
+// Graphs of fewer nodes than their build (12 nodes: the 6 x 2 shapes of train/code; any 2 num_x below 16 or 32) run on the
+// NP-node build: every environment is padded to NP rows with zero features and zero adjacency rows / columns (a padded node
+// neither sends nor receives), the kernel divides the pooled scramble by the real node count and writes only the real rows.
+template <int NP>
 __global__ void __launch_bounds__(256)
 pad_nodes_kernel(int B, int n, const float* __restrict__ x_n, const float* __restrict__ A_n, const float* __restrict__ A_s,
                  const float* __restrict__ A_ts, const float* __restrict__ A_cs, float* __restrict__ x_o, float* __restrict__ An_o,
                  float* __restrict__ As_o, float* __restrict__ Ats_o, float* __restrict__ Acs_o) {
-  constexpr int NP = 16;
   const int per_env = NP * 13 + 3 * NP * NP;
   const long long total = (long long)B * per_env;
   for (long long idx = (long long)blockIdx.x * 256 + threadIdx.x; idx < total; idx += (long long)gridDim.x * 256) {
@@ -464,8 +466,8 @@ thread_local std::string g_actor_err;
 }
 struct tactor_handle_s {
   int device = 0, nodes = 0, max_batch = 0;
-  int n_real = 0;                      // nodes of the caller's graphs (12: padded to 16 internally; else = nodes)
-  float* pad[5] = {};                  // padded x_n, A_n, A_s, A_n_ts, A_n_cs of a 12-node handle
+  int n_real = 0;                      // nodes of the caller's graphs (< nodes: padded to the build's width internally)
+  float* pad[5] = {};                  // padded x_n, A_n, A_s, A_n_ts, A_n_cs of a handle with n_real < nodes
   float* d_w[TACTOR_NLAYERS] = {};     // packed [Kpad, 208]
   float* d_b[TACTOR_NLAYERS] = {};     // [208]
   float* pooled = nullptr;             // [max_batch, 208] Pareto embedding
@@ -529,6 +531,26 @@ cudaError_t set_pipe_smem() {
   return cudaFuncSetAttribute(tactor::tc::pipe::actor_pipe_kernel<NODES, NREAL>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                               tactor::tc::pipe::pipe_smem_bytes<NODES>());
 }
+
+// One actor_pipe_kernel instantiation per real node count 2 num_x, num_x = 3..16: counts up to 16 run on the 16-node build,
+// larger ones on the 32-node build.  The real count stays a template parameter, so that the pooled scramble and the output
+// rows use constant arithmetic.
+constexpr int ACTOR_MIN_NODES = 6, ACTOR_MAX_NODES = 32;
+constexpr int build_nodes(int n_real) { return n_real <= 16 ? 16 : 32; }
+
+struct PipeEntry {
+  cudaError_t (*launch)(tactor::tc::fused::Params&, int, int, cudaStream_t);
+  cudaError_t (*set_smem)();
+};
+template <int... I>
+constexpr std::array<PipeEntry, sizeof...(I)> pipe_table(std::integer_sequence<int, I...>) {
+  return {{{launch_pipe<build_nodes(ACTOR_MIN_NODES + 2 * I), ACTOR_MIN_NODES + 2 * I>,
+            set_pipe_smem<build_nodes(ACTOR_MIN_NODES + 2 * I), ACTOR_MIN_NODES + 2 * I>}...}};
+}
+constexpr auto kPipes = pipe_table(std::make_integer_sequence<int, (ACTOR_MAX_NODES - ACTOR_MIN_NODES) / 2 + 1>{});
+
+bool actor_nodes_supported(int n) { return n >= ACTOR_MIN_NODES && n <= ACTOR_MAX_NODES && n % 2 == 0; }
+const PipeEntry& pipe_for(int n_real) { return kPipes[(n_real - ACTOR_MIN_NODES) / 2]; }
 
 // (re)builds the device copies of the weights: packed [Kpad,208] kernels / [208] biases and the tcgen05 operand
 // images of the seven [200,200] layers.  Buffers are allocated on first use and overwritten afterwards.
@@ -682,8 +704,7 @@ cudaError_t run_forward(tactor_handle_s* h, int B, const tactor_inputs* in, floa
   p.w_head[0] = h->d_w[11]; p.w_head[1] = h->d_w[12]; p.b_head[0] = h->d_b[11]; p.b_head[1] = h->d_b[12];
   p.geo = geo; p.topo = topo; p.M = M; p.error_flag = h->d_error;
   p.noise = nz.on; p.mu = nz.mu; p.theta = nz.theta; p.sigma = nz.sigma; p.seed = nz.seed; p.call = nz.call; p.seed_call = nz.seed_call;
-  cudaError_t e = (h->n_real == 12) ? launch_pipe<16, 12>(p, M, h->sms, st)      // the padded 12-node build
-                                    : launch_pipe<NODES>(p, M, h->sms, st);
+  cudaError_t e = pipe_for(h->n_real).launch(p, M, h->sms, st);
   h->launches.fetch_add(2);
   return e != cudaSuccess ? e : cudaGetLastError();
 }
@@ -696,9 +717,10 @@ const char* tactor_last_error(void) { return g_actor_err.c_str(); }
 int tactor_create(const tactor_weights* w, int nodes, int max_batch, int device, tactor_handle_t* out) {
   if (!w || !out) return afail(TFEM_ERR_ARG, "null argument");
   *out = nullptr;
-  if (nodes != 12 && nodes != 16 && nodes != 32) return afail(TFEM_ERR_UNSUPPORTED, "nodes must be 12, 16 or 32");
+  if (!actor_nodes_supported(nodes))
+    return afail(TFEM_ERR_UNSUPPORTED, "nodes must be even and in 6..32 (2 num_x for num_x 3..16), got " + std::to_string(nodes));
   const int n_real = nodes;
-  if (nodes == 12) nodes = 16;          // 12-node graphs (train/code) are padded to the 16-node build, see pad_nodes_kernel
+  nodes = build_nodes(n_real);          // smaller graphs are padded to the 16- or 32-node build, see pad_nodes_kernel
   if (max_batch <= 0) return afail(TFEM_ERR_ARG, "max_batch must be positive");
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return afail(TFEM_ERR_CUDA, "no CUDA device: no CPU path");
@@ -714,15 +736,15 @@ int tactor_create(const tactor_weights* w, int nodes, int max_batch, int device,
   if (const char* v = getenv("TACTOR_NO_SPLIT")) { if (v[0] == '1') h->sms = 0; }
   if (e == cudaSuccess) e = cudaMalloc(&h->d_error, 65536);
   if (e == cudaSuccess) e = cudaMemset(h->d_error, 0, 65536);
-  if (e == cudaSuccess) e = (nodes == 16) ? set_pipe_smem<16>() : set_pipe_smem<32>();
-  if (e == cudaSuccess && n_real == 12) e = set_pipe_smem<16, 12>();
+  if (e == cudaSuccess) e = pipe_for(n_real).set_smem();
   if (e == cudaSuccess)
     e = (nodes == 16) ? cudaFuncSetAttribute(tactor::pareto_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, tactor::PARETO_SMEM)
                       : cudaFuncSetAttribute(tactor::pareto_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, tactor::PARETO_SMEM);
   if (e == cudaSuccess) e = cudaMalloc(&h->pooled, (size_t)max_batch * tactor::LD * 4);
   if (e == cudaSuccess) e = cudaMalloc(&h->pareto_flag, (size_t)max_batch * sizeof(int));
   if (n_real != nodes) {
-    const size_t sz[5] = {(size_t)max_batch * 16 * 13, 16 * 16, (size_t)max_batch * 256, (size_t)max_batch * 256, (size_t)max_batch * 256};
+    const size_t np = (size_t)nodes;
+    const size_t sz[5] = {max_batch * np * 13, np * np, max_batch * np * np, max_batch * np * np, max_batch * np * np};
     for (int k = 0; k < 5 && e == cudaSuccess; ++k) e = cudaMalloc(&h->pad[k], sz[k] * sizeof(float));
   }
   if (const char* v = getenv("TACTOR_PARETO_DENSE")) h->pareto_dense = (v[0] == '1');
@@ -803,11 +825,12 @@ static int forward_impl(tactor_handle_t h, int B, const tactor_inputs* in, float
   if (B == 0) return TFEM_OK;
   Guard g(h->device);
   tactor_inputs padded;
-  if (h->n_real != h->nodes) {          // 12 -> 16 nodes: zero-padded copies of the graph tensors in handle-owned buffers
-    const long long total = (long long)B * (16 * 13 + 3 * 256);
+  if (h->n_real != h->nodes) {          // n_real -> 16 or 32 nodes: zero-padded copies of the graph tensors in handle-owned buffers
+    const long long np = h->nodes, total = (long long)B * (np * 13 + 3 * np * np);
     const int grid = (int)((total + 255) / 256 < 148 * 8 ? (total + 255) / 256 : 148 * 8);
-    tactor::pad_nodes_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(B, h->n_real, in->x_n, in->A_n, in->A_s, in->A_n_ts, in->A_n_cs,
-                                                                      h->pad[0], h->pad[1], h->pad[2], h->pad[3], h->pad[4]);
+    auto pad = (h->nodes == 16) ? tactor::pad_nodes_kernel<16> : tactor::pad_nodes_kernel<32>;
+    pad<<<grid, 256, 0, (cudaStream_t)stream>>>(B, h->n_real, in->x_n, in->A_n, in->A_s, in->A_n_ts, in->A_n_cs, h->pad[0], h->pad[1],
+                                                h->pad[2], h->pad[3], h->pad[4]);
     h->launches.fetch_add(1);
     padded = *in;
     padded.x_n = h->pad[0]; padded.A_n = h->pad[1]; padded.A_s = h->pad[2]; padded.A_n_ts = h->pad[3]; padded.A_n_cs = h->pad[4];

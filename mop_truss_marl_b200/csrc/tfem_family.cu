@@ -38,8 +38,9 @@ static float norm_col(float v, float mn, float mx) {
 bool build_family(const tfem_family_desc& d, Family& f) {
   f.desc = d;
   const int nx = d.num_x;
-  if (nx != 6 && nx != 8 && nx != 16) {
-    f.error = "num_x must be 6 (train/code), 8 or 16 (test/00..03): the compiled kernel shapes; got " + std::to_string(nx);
+  if (nx < 3 || nx > TFEM_MAX_NX) {
+    f.error = "num_x must be 3.." + std::to_string(TFEM_MAX_NX) + " (one kernel lane per node, at most 32 nodes; num_x = 2 leaves "
+              "no free bottom node to carry a load); got " + std::to_string(nx);
     return false;
   }
   if (d.truss_type != TFEM_BRIDGE && d.truss_type != TFEM_ROOF) {
@@ -48,6 +49,13 @@ bool build_family(const tfem_family_desc& d, Family& f) {
   }
   if (d.symmetry < TFEM_SYM_NONE || d.symmetry > TFEM_SYM_LARGE) {
     f.error = "bad symmetry convention";
+    return false;
+  }
+  if (d.symmetry != TFEM_SYM_NONE && nx != 6 && nx != 8 && nx != 16) {
+    // the reference's symmetry index lists exist only in the 8- and 16-column truss2D_ENV.py files
+    f.error = std::string("the ") + (d.symmetry == TFEM_SYM_SMALL ? "small" : "large") +
+              " symmetry convention is defined for num_x 6, 8 and 16 only; num_x = " + std::to_string(nx) +
+              " takes TFEM_SYM_NONE (train/code's ENV, which has no symmetry step)";
     return false;
   }
   const int N = 2 * nx, E = 5 * nx - 4;
@@ -227,11 +235,14 @@ bool build_family(const tfem_family_desc& d, Family& f) {
   }
   auto& mp = f.maps;
   mp.clear();
+  // every section starts on a multiple of 4 entries: the kernel reads a section's map with 64- or 128-bit loads (only an
+  // odd num_x, whose x_n map has 26 num_x entries, needs the padding)
+  auto section = [&mp](int32_t* off) { while (mp.size() % 4) mp.push_back(0); *off = (int)mp.size(); };
   static const int xn_const_col[13] = {0, -1, 1, 2, 3, 4, 5, -1, -1, -1, -1, -1, -1};
   static const int xn_dyn_col[13] = {-1, 0, -1, -1, -1, -1, -1, 1, 2, 3, 4, 5, 6};
   static const int raw_const_col[12] = {0, -1, 1, 2, 3, 4, 5, -1, -1, -1, -1, -1};
   static const int raw_dyn_col[12] = {-1, 0, -1, -1, -1, -1, -1, 1, 2, 3, 4, 5};
-  t.map_xn = (int)mp.size();
+  section(&t.map_xn);
   for (int i = 0; i < N; ++i)
     for (int k = 0; k < 13; ++k)
       mp.push_back((uint16_t)(xn_const_col[k] >= 0 ? pl.xn_const(xn_const_col[k]) + i : pl.xn_dyn(xn_dyn_col[k]) + i));
@@ -243,14 +254,14 @@ bool build_family(const tfem_family_desc& d, Family& f) {
   const int adj_cols[3] = {EL_AS, EL_TS, EL_CS};
   int32_t* adj_off[3] = {&t.map_as, &t.map_ts, &t.map_cs};
   for (int m = 0; m < 3; ++m) {
-    *adj_off[m] = (int)mp.size();
+    section(adj_off[m]);
     for (int i = 0; i < N * N; ++i) mp.push_back((uint16_t)(pair_el[i] >= 0 ? pl.el(adj_cols[m]) + pair_el[i] : 0));
   }
-  t.map_rawn = (int)mp.size();
+  section(&t.map_rawn);
   for (int i = 0; i < N; ++i)
     for (int k = 0; k < 12; ++k)
       mp.push_back((uint16_t)(raw_const_col[k] >= 0 ? pl.raw_const(raw_const_col[k]) + i : pl.raw_dyn(raw_dyn_col[k]) + i));
-  t.map_rawe = (int)mp.size();
+  section(&t.map_rawe);
   for (int el = 0; el < E; ++el) {
     for (int k = 0; k < 7; ++k) mp.push_back((uint16_t)(pl.el(k) + el));
     for (int s = 0; s < 2; ++s) {

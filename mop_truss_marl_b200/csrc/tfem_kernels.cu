@@ -23,6 +23,9 @@
 
 #include <math_constants.h>
 
+#include <array>
+#include <utility>
+
 namespace tfem {
 
 namespace {
@@ -86,6 +89,11 @@ __device__ __forceinline__ float round2(float v) { return __fdiv_rn(rintf(__fmul
 
 // numpy float32 pairwise sum (n <= 128): executed by the whole warp, the array lives in shared memory
 __device__ __forceinline__ float pairwise_sum_warp(const float* a, int n, int lane) {
+  if (n < 8) {                             // numpy adds fewer than 8 values in order (N = 6 nodes: num_x = 3)
+    float res = 0.f;
+    for (int i = 0; i < n; ++i) res = __fadd_rn(res, a[i]);
+    return res;
+  }
   const int k = lane & 7;
   float r = a[k];
   const int nfull = n - (n % 8);
@@ -680,18 +688,26 @@ tfem_step_kernel(const StepArgs args) {
           const uint2 mm = m[q];
           o[q] = make_float4(pool[mm.x & 0xffffu], pool[mm.x >> 16], pool[mm.y & 0xffffu], pool[mm.y >> 16]);
         }
-      } else {
-        // an environment's slice of this tensor is not a multiple of 16 bytes (nN_x_e of the 6 x 2 shapes: 26 x 21 floats),
-        // so neither are the slice addresses: 64-bit stores (every per-environment count is even)
+      } else if (count % 2 == 0) {
+        // an environment's slice of this tensor is not a multiple of 16 bytes (nN_x_e of the 6 x 2 shapes: 26 x 21 floats,
+        // x_n of an odd num_x: 26 num_x floats), so neither are the slice addresses: 64-bit stores
         float2* o2 = reinterpret_cast<float2*>(dst + (size_t)b * count);
         const uint32_t* m1 = reinterpret_cast<const uint32_t*>(maps + map_off);
         for (int q = lane; q < count / 2; q += 32) {
           const uint32_t mm = m1[q];
           o2[q] = make_float2(pool[mm & 0xffffu], pool[mm >> 16]);
         }
+      } else {
+        // nN_x_e of an odd num_x (21 E floats, E = 5 num_x - 4 odd): 32-bit stores
+        float* o1 = dst + (size_t)b * count;
+        for (int q = lane; q < count; q += 32) o1[q] = pool[maps[map_off + q]];
       }
     };
-    static_assert((N * 13) % 4 == 0 && (N * N) % 4 == 0 && (N * 12) % 4 == 0 && (E * 21) % 2 == 0, "vector width of the output streams");
+    // The path is chosen from the per-environment count, a compile-time constant: 128-bit stores need a count = 0 mod 4,
+    // 64-bit stores a count = 0 mod 2, and both need the map section to start on as many entries (build_family starts
+    // every section on a multiple of 4).  The adjacency tensors and nN_x_n always take the 128-bit path; x_n (13 N) takes
+    // the 64-bit one for odd num_x, nN_x_e (21 E) the 32-bit one.
+    static_assert((N * N) % 4 == 0 && (N * 12) % 4 == 0 && (N * 13) % 2 == 0, "vector width of the output streams");
     emit(args.out.x_n, fam->map_xn, N * 13);
     emit(args.out.A_s, fam->map_as, N * N);
     emit(args.out.A_n_ts, fam->map_ts, N * N);
@@ -707,63 +723,66 @@ int smem_bytes_for(int map_entries, int n_tables = 1) {
   return align16(n_tables * (int)sizeof(FamilyTables)) + align16(((map_entries + 7) & ~7) * 2) + WARPS_PER_CTA * Dims<NX>::WARP_BYTES;
 }
 
-}  // namespace
+// The chord lengths the env-step kernel is built for: one lane per node, so N = 2 NX <= 32; NX = 2 leaves no free bottom node
+// to carry a bridge's load.  Every NX has the env-step / reset / solve-only, the gene-vector and the mixed-family kernel.
+constexpr int NX_MIN = 3, NX_MAX = TFEM_MAX_NX;
 
-namespace {
-template <int NX, bool GM, bool MF>
-cudaError_t configure_one(int smem, int* ctas) {
-  cudaError_t err = cudaFuncSetAttribute(tfem_step_kernel<NX, GM, MF>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+using StepKernel = void (*)(const StepArgs);
+struct NxKernels {
+  StepKernel step, genes, mixed;
+  int (*smem)(int map_entries, int n_tables);
+};
+
+template <int... I>
+constexpr std::array<NxKernels, sizeof...(I)> nx_table(std::integer_sequence<int, I...>) {
+  return {{{tfem_step_kernel<NX_MIN + I, false, false>, tfem_step_kernel<NX_MIN + I, true, false>,
+            tfem_step_kernel<NX_MIN + I, false, true>, smem_bytes_for<NX_MIN + I>}...}};
+}
+constexpr auto kNxKernels = nx_table(std::make_integer_sequence<int, NX_MAX - NX_MIN + 1>{});
+
+const NxKernels* kernels_for(int nx) { return (nx >= NX_MIN && nx <= NX_MAX) ? &kNxKernels[nx - NX_MIN] : nullptr; }
+
+cudaError_t configure_one(StepKernel k, int smem, int* ctas) {
+  cudaError_t err = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
   if (err != cudaSuccess) return err;
-  err = cudaFuncSetAttribute(tfem_step_kernel<NX, GM, MF>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+  err = cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
   if (err != cudaSuccess) return err;
-  return cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas, tfem_step_kernel<NX, GM, MF>, WARPS_PER_CTA * 32, smem);
+  return cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas, k, WARPS_PER_CTA * 32, smem);
 }
 
 // The opt-in size is an attribute of the function, shared by every live handle of this NX.  It is set to what the
 // largest family count needs (capped by the device's per-block limit), never to what one handle needs, so creating a
 // handle of few families cannot break a live handle of more.
-template <int NX>
-cudaError_t configure_mixed_nx(int map_entries, int single_ctas, int n_families, int* smem, int* max_families) {
+cudaError_t configure_mixed_nx(const NxKernels& k, int map_entries, int single_ctas, int n_families, int* smem,
+                               int* max_families) {
   int dev = 0, optin = 0;
   cudaError_t err = cudaGetDevice(&dev);
   if (err == cudaSuccess) err = cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
   if (err != cudaSuccess) return err;
   int top = TFEM_MAX_FAMILIES;
-  while (top > 1 && smem_bytes_for<NX>(map_entries, top) > optin) --top;
+  while (top > 1 && k.smem(map_entries, top) > optin) --top;
   int ctas = 0;
-  err = configure_one<NX, false, true>(smem_bytes_for<NX>(map_entries, top), &ctas);
+  err = configure_one(k.mixed, k.smem(map_entries, top), &ctas);
   if (err != cudaSuccess) return err;
   *max_families = 0;
   for (int f = 1; f <= top; ++f) {
-    err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas, tfem_step_kernel<NX, false, true>, WARPS_PER_CTA * 32,
-                                                        smem_bytes_for<NX>(map_entries, f));
+    err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas, k.mixed, WARPS_PER_CTA * 32, k.smem(map_entries, f));
     if (err != cudaSuccess) return err;
     if (ctas < single_ctas) break;
     *max_families = f;
   }
-  *smem = (n_families <= *max_families) ? smem_bytes_for<NX>(map_entries, n_families) : 0;
+  *smem = (n_families <= *max_families) ? k.smem(map_entries, n_families) : 0;
   return cudaSuccess;
 }
 }  // namespace
 
 int step_kernel_configure(int nx, int device, int map_entries, LaunchInfo* info) {
-  cudaError_t err;
-  int smem = 0, ctas = 0, ctas_g = 0, sms = 0;
-  if (nx == 6) {                   // the 6 x 2 shapes of train/code/master_DDPG_truss2D_MO.py:787-795
-    smem = smem_bytes_for<6>(map_entries);
-    err = configure_one<6, false, false>(smem, &ctas);
-    if (err == cudaSuccess) err = configure_one<6, true, false>(smem, &ctas_g);
-  } else if (nx == 8) {
-    smem = smem_bytes_for<8>(map_entries);
-    err = configure_one<8, false, false>(smem, &ctas);
-    if (err == cudaSuccess) err = configure_one<8, true, false>(smem, &ctas_g);
-  } else if (nx == 16) {
-    smem = smem_bytes_for<16>(map_entries);
-    err = configure_one<16, false, false>(smem, &ctas);
-    if (err == cudaSuccess) err = configure_one<16, true, false>(smem, &ctas_g);
-  } else {
-    return (int)cudaErrorInvalidValue;
-  }
+  const NxKernels* k = kernels_for(nx);
+  if (!k) return (int)cudaErrorInvalidValue;
+  int ctas = 0, ctas_g = 0, sms = 0;
+  const int smem = k->smem(map_entries, 1);
+  cudaError_t err = configure_one(k->step, smem, &ctas);
+  if (err == cudaSuccess) err = configure_one(k->genes, smem, &ctas_g);
   if (err != cudaSuccess) return (int)err;
   err = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
   if (err != cudaSuccess) return (int)err;
@@ -779,16 +798,15 @@ int step_kernel_configure(int nx, int device, int map_entries, LaunchInfo* info)
 }
 
 int step_kernel_configure_mixed(int nx, int map_entries, int n_families, LaunchInfo* info, int* max_families) {
-  cudaError_t err;
-  if (nx == 6) err = configure_mixed_nx<6>(map_entries, info->ctas_per_sm, n_families, &info->smem_mixed, max_families);
-  else if (nx == 8) err = configure_mixed_nx<8>(map_entries, info->ctas_per_sm, n_families, &info->smem_mixed, max_families);
-  else if (nx == 16) err = configure_mixed_nx<16>(map_entries, info->ctas_per_sm, n_families, &info->smem_mixed, max_families);
-  else return (int)cudaErrorInvalidValue;
-  return (int)err;
+  const NxKernels* k = kernels_for(nx);
+  if (!k) return (int)cudaErrorInvalidValue;
+  return (int)configure_mixed_nx(*k, map_entries, info->ctas_per_sm, n_families, &info->smem_mixed, max_families);
 }
 
 int step_kernel_launch(int nx, const StepArgs& args, const LaunchInfo& info, cudaStream_t stream) {
   if (args.B <= 0) return 0;
+  const NxKernels* k = kernels_for(nx);
+  if (!k) return (int)cudaErrorInvalidValue;
   const bool gm = args.mode == MODE_GENES, mf = args.family != nullptr;
   if (mf && (gm || info.smem_mixed <= 0)) return (int)cudaErrorInvalidValue;
   const int needed = (args.B + WARPS_PER_CTA - 1) / WARPS_PER_CTA;
@@ -801,17 +819,7 @@ int step_kernel_launch(int nx, const StepArgs& args, const LaunchInfo& info, cud
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;     // see griddepcontrol.wait in the kernel
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr; cfg.numAttrs = 1;
-  cudaError_t e;
-  if (nx == 6 && mf) e = cudaLaunchKernelEx(&cfg, tfem_step_kernel<6, false, true>, args);
-  else if (nx == 6 && !gm) e = cudaLaunchKernelEx(&cfg, tfem_step_kernel<6, false, false>, args);
-  else if (nx == 6) e = cudaLaunchKernelEx(&cfg, tfem_step_kernel<6, true, false>, args);
-  else if (nx == 8 && mf) e = cudaLaunchKernelEx(&cfg, tfem_step_kernel<8, false, true>, args);
-  else if (nx == 8 && !gm) e = cudaLaunchKernelEx(&cfg, tfem_step_kernel<8, false, false>, args);
-  else if (nx == 8) e = cudaLaunchKernelEx(&cfg, tfem_step_kernel<8, true, false>, args);
-  else if (nx == 16 && mf) e = cudaLaunchKernelEx(&cfg, tfem_step_kernel<16, false, true>, args);
-  else if (nx == 16 && !gm) e = cudaLaunchKernelEx(&cfg, tfem_step_kernel<16, false, false>, args);
-  else if (nx == 16) e = cudaLaunchKernelEx(&cfg, tfem_step_kernel<16, true, false>, args);
-  else return (int)cudaErrorInvalidValue;
+  const cudaError_t e = cudaLaunchKernelEx(&cfg, mf ? k->mixed : gm ? k->genes : k->step, args);
   return (int)(e != cudaSuccess ? e : cudaGetLastError());
 }
 
